@@ -9,6 +9,7 @@ K7 Adam -> K2 priority write-back -> target copy) over one batch per rank.
 
   python bench.py [--gpus N --steps K --warmup W]          our arm (one rank per GPU under torchrun)
   python bench.py --impl reference [...]                  the reference's CPU path (oracle port), host cores
+  python bench.py --dump-outputs DIR [...]                also write what the last timed update computed, DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what each key means.
 """
@@ -396,6 +397,43 @@ def time_stage(fn, iters, torch):
   return e0.elapsed_time(e1) / iters * 1e-3
 
 
+DUMP_BUDGET = 64_000_000
+DUMP_SAMPLE = 1 << 20
+
+
+def dump_outputs(out_dir, arrays):
+  """Writes each array as `out_dir/<name>.npy` for output-by-output comparison of two builds.  Floating-point arrays
+  are stored as float32, integer arrays (indices, keys) as float64, which holds them exactly below 2**53."""
+  arrays = {k: np.asarray(v) for k, v in arrays.items()}
+  arrays = {k: v.astype(np.float64 if v.dtype.kind in 'iub' else np.float32) for k, v in arrays.items()}
+  total = sum(v.nbytes for v in arrays.values())
+  if total > DUMP_BUDGET:
+    raise ValueError(f'--dump-outputs: {total} bytes exceed the {DUMP_BUDGET} byte budget')
+  os.makedirs(out_dir, exist_ok=True)
+  for name, v in arrays.items():
+    np.save(os.path.join(out_dir, f'{name}.npy'), v)
+
+
+def dqn_outputs(learner, ds, net, tgt):
+  """What the last DQN update handed its caller: loss, TD errors, importance weights, the priorities written back,
+  the sampled items and q(o_tm1), plus the updated state (online parameters in full; target parameters and Adam
+  moments as a fixed, seeded sample of DUMP_SAMPLE positions, which keeps the dump inside DUMP_BUDGET; the update
+  count)."""
+  import torch
+  torch.cuda.synchronize()
+  pick = torch.as_tensor(np.sort(np.random.default_rng(0).choice(net.params.size, DUMP_SAMPLE, replace=False)),
+                         device=net.params.flat.device)
+  host = lambda t: t.detach().cpu().numpy()
+  return {
+      'loss': host(learner.loss), 'td_error': host(learner.td), 'importance_weight': host(learner.weight),
+      'priority': host(learner.priority), 'q_tm1': host(learner.q_values()[0]),
+      'sample_index': host(ds.idx), 'sample_key': host(ds.keys.view(torch.int64)), 'sample_prob': host(ds.prob),
+      'online_params': host(net.params.flat), 'target_params_sample': host(tgt.params.flat[pick]),
+      'adam_m_sample': host(learner._m[pick]), 'adam_v_sample': host(learner._v[pick]),
+      'num_steps': host(learner._num_steps),
+  }
+
+
 def run_ours(args):
   import torch
   import torch.distributed as dist
@@ -466,6 +504,8 @@ def run_ours(args):
     dev_s = float(tt)
   ms_per_step = dev_s / args.steps * 1e3
   value = world * args.steps / dev_s
+  if args.dump_outputs and rank == 0:     # before the end-to-end leg below moves the learner on
+    dump_outputs(args.dump_outputs, dqn_outputs(learner, ds, net, tgt))
 
   if args.profile:
     if rank == 0:
@@ -494,7 +534,7 @@ def run_ours(args):
     e2e_step(i)
   barrier()
   t0 = time.perf_counter()
-  e2e_steps = max(args.steps, 200)       # at least as long as the value leg; short driver runs still time 200 updates (~70 ms)
+  e2e_steps = args.steps
   for i in range(e2e_steps):
     e2e_step(i + 3)
   learner.flush()
@@ -731,7 +771,7 @@ def run_d4pg(args):
     e2e_step(i)
   barrier()
   t0 = time.perf_counter()
-  e2e_steps = max(args.steps, 200)
+  e2e_steps = args.steps
   for i in range(e2e_steps):
     e2e_step(i + 3)
   last = learner.drain()
@@ -870,7 +910,7 @@ def run_sumtree(args):
   hk, hp = torch.empty(B, dtype=torch.int64).pin_memory(), torch.empty(B).pin_memory()
   barrier()
   t0 = time.perf_counter()
-  e2e_steps = max(args.steps // 2, 5)
+  e2e_steps = args.steps
   for _ in range(e2e_steps):
     u.copy_(hu, non_blocking=True)
     step()
@@ -933,8 +973,9 @@ def run_sumtree(args):
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--gpus', type=int, default=1)
-  ap.add_argument('--steps', type=int, default=2000)
-  ap.add_argument('--warmup', type=int, default=50)
+  ap.add_argument('--steps', type=int, default=None,
+                  help='timed steps of every timed leg (default 2000; sumtree 100; reference arm 10, sumtree 3)')
+  ap.add_argument('--warmup', type=int, default=None, help='default 50; sumtree 5; reference arm 2, sumtree 1')
   ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
   ap.add_argument('--precision', default=os.environ.get('B200RL_PRECISION', 'bf16'), choices=['fp32', 'tf32', 'tc', 'bf16'],
                   help="'bf16' (default): bf16 dataflow on tcgen05 (kind::f16); 'tf32' ('tc'): fp32 tensors with tf32 operands; "
@@ -948,14 +989,24 @@ def main():
   ap.add_argument('--no-graph', action='store_true')
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--profile', action='store_true', help='only warm-up + timed steps (for ncu captures)')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='dqn workload of our arm: after the timed steps, write what the last one computed as DIR/<name>.npy '
+                       '(float32 / float64, at most 64 MB; the inputs are seeded, so two builds can be compared)')
   args = ap.parse_args()
   if args.items is None:
     args.items = 100_000_000 if args.workload == 'sumtree' else 1_000_000
-  if args.workload == 'sumtree' and args.steps == 2000 and args.warmup == 50:
-    args.steps, args.warmup = 100, 5          # a step is 2^20 draws + updates: keep the default run short
+  # a sumtree step is 2^20 draws + updates, and the reference arm runs on the host: shorter default runs
   if args.impl == 'reference':
-    if args.steps >= 100:                     # defaults sized for the GPU arm; bound the CPU run
-      args.steps, args.warmup = (10, 2) if args.workload != 'sumtree' else (3, 1)
+    steps, warmup = (10, 2) if args.workload != 'sumtree' else (3, 1)
+  else:
+    steps, warmup = (2000, 50) if args.workload != 'sumtree' else (100, 5)
+  args.steps = steps if args.steps is None else args.steps
+  args.warmup = warmup if args.warmup is None else args.warmup
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and (args.impl != 'ours' or args.workload != 'dqn'):
+    ap.error('--dump-outputs is implemented for the dqn workload of our arm')
+  if args.impl == 'reference':
     (run_reference if args.workload == 'dqn' else run_reference_other)(args)
   elif args.workload == 'd4pg':
     run_d4pg(args)

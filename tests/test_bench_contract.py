@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -53,3 +55,49 @@ def test_parity_record_states_the_tested_tolerance():
   finally:
     bench.ROOT = old_root
   assert rec['mode'] == 'bf16' and rec['tol'] is None and rec['max_rel_err_td'] is None
+
+
+def test_dump_outputs_writes_float_arrays_within_the_budget(tmp_path):
+  """`--dump-outputs` stores float32 / float64 only (integers exactly, as float64) and refuses a dump over its budget."""
+  import numpy as np
+  sys.path.insert(0, ROOT)
+  import bench
+  idx = np.array([0, 3, (1 << 40) + 7], np.int64)
+  bench.dump_outputs(str(tmp_path / 'd'), {'idx': idx, 'td': np.arange(4, dtype=np.float32), 'w': np.ones(2, np.float64)})
+  got = {p.stem: np.load(p) for p in (tmp_path / 'd').glob('*.npy')}
+  assert got['idx'].dtype == np.float64 and np.array_equal(got['idx'].astype(np.int64), idx)
+  assert got['td'].dtype == np.float32 and got['w'].dtype == np.float32
+  with pytest.raises(ValueError):
+    bench.dump_outputs(str(tmp_path / 'big'), {'x': np.zeros(bench.DUMP_BUDGET // 4 + 1, np.float32)})
+  assert not (tmp_path / 'big').exists()
+  out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--dump-outputs', str(tmp_path)],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+  assert out.returncode != 0 and '--dump-outputs' in out.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_last_timed_update(tmp_path):
+  """Our arm, small table: `--steps` is the number of timed updates (the dumped update count is warm-up + steps), and
+  the same arguments give the same inputs, so two runs sample the same items and compute the same update."""
+  import numpy as np
+  steps, warmup = 4, 3
+  runs = []
+  for i in range(2):
+    d = tmp_path / f'run{i}'
+    out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', str(steps), '--warmup', str(warmup),
+                          '--items', '8192', '--no-cpu-baseline', '--dump-outputs', str(d)],
+                         capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line['steps'] == steps and line['e2e']['steps'] == steps
+    files = sorted(d.glob('*.npy'))
+    assert sum(f.stat().st_size for f in files) <= 64_000_000
+    runs.append({f.stem: np.load(f) for f in files})
+  a, b = runs
+  assert a.keys() == b.keys() and {'loss', 'td_error', 'priority', 'online_params', 'sample_index'} <= a.keys()
+  assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+  assert a['num_steps'].tolist() == [warmup + steps]
+  assert a['td_error'].shape == a['priority'].shape == a['sample_index'].shape == (256,)
+  np.testing.assert_array_equal(a['sample_index'], b['sample_index'])
+  for k in a:
+    np.testing.assert_allclose(a[k], b[k], rtol=1e-5, atol=1e-6 * float(np.abs(a[k]).max()), err_msg=k)

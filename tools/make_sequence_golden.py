@@ -1,7 +1,7 @@
 """Writes tests/golden/sequence_cases.json from the reference's own SequenceAdder test vectors
 (`acme/adders/reverb/sequence_test.py:25-181`, TEST_CASES).  The reference module cannot be imported here (it needs
 reverb / tensorflow), so the TEST_CASES literal is cut out of the file and evaluated with this repo's dm_env shim, which
-builds the same TimeSteps.  Run in the build container (needs /root/reference):  python tools/make_sequence_golden.py"""
+builds the same TimeSteps.  Needs a checkout of the reference:  python tools/make_sequence_golden.py <reference checkout>"""
 import json
 import os
 import sys
@@ -10,11 +10,11 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from acme_b200 import dm_env  # noqa: E402
 
-SRC = '/root/reference/acme/adders/reverb/sequence_test.py'
+SRC = os.path.join('acme', 'adders', 'reverb', 'sequence_test.py')
 
 
-def main():
-  text = open(SRC).read()
+def main(reference_root):
+  text = open(os.path.join(reference_root, SRC)).read()
   a = text.index('TEST_CASES = [')
   b = text.index('\n]\n', a) + 3
   ns = {'dm_env': dm_env}
@@ -35,4 +35,4 @@ def main():
 
 
 if __name__ == '__main__':
-  main()
+  main(sys.argv[1])
