@@ -262,7 +262,8 @@ __device__ __forceinline__ void store_staged_rows(const Epilogue& e, const float
       const long long row = dst_row(r);
       if (row < 0 || col >= N) continue;
       const float4 a = staged_chunk<BN>(slab, r, c);
-      if (obf || mbf || e.scale != 0.f) {
+      // a split-K partial is stored raw (finish4); finish() would apply the epilogue and write `out` instead
+      if (!e.partial && (obf || mbf || e.scale != 0.f)) {
         const float v[4] = {a.x, a.y, a.z, a.w};
 #pragma unroll
         for (int j = 0; j < 4; ++j) if (col + j < N) finish(e, (int)row, col + j, v[j]);

@@ -1,12 +1,45 @@
-"""bf16 dataflow kernels (gemm_bf16.cu) through the C ABI against PyTorch-CPU fp32 on the SAME bf16-rounded operands: the
-only differences left are the fp32 summation order and the rounding of a bf16 output (2^-9 relative), so the bounds are
-tight.  Shapes: the DQN-Atari layers at small batch plus the benchmarked batch for the dense layer."""
+"""bf16 dataflow kernels (gemm_bf16.cu) through the C ABI against an fp64 reference on the SAME bf16-rounded operands.
+
+Every output element is held to its own bound (`_check`):
+
+    |got - ref| <= C_ACC * (|A|.|B|)_ij + c_out * |ref_ij|
+
+where |A|.|B| is the same product (or convolution) on absolute values, bias magnitude included, and c_out = 2^-8 for a
+bf16 output (one round-to-nearest to 8 significant bits: < 2^-8 relative) and 0 for an fp32 one.  Every row with a
+reduction of 1024 or more also proves that the bound REJECTS the reference recomputed without one 64-wide k-block, without
+the last (possibly ragged) k-block and, for split-K rows, without one whole split (`_assert_rejects`).
+
+C_ACC = 2^-16.  Measured on a B200 (1000 W power limit), max over the rows below of |err| / (|A|.|B|) on fp32 outputs
+and split-K partials:
+    linear_fwd_bf16 7.8e-07    linear_dgrad_bf16 3.9e-07    linear_wgrad_bf16 2.5e-07    colsum_bf16 1.1e-08
+    conv2d_fwd_bf16 3.3e-07    conv2d_wgrad_bf16 4.4e-07 (row image: 4.4e-07)          conv2d_dgrad_bf16 2.6e-07
+i.e. <= 2^-20, 20x below C_ACC.  The estimate it was first set from, 2^-12, left the rejection of a conv1 weight
+gradient without its last 25-pixel k-block at only 2x; at 2^-16 the smallest rejection margin is 32x.  (Run with `-s`:
+each check prints its ratio, and each rejection its margin, as `bf16-bound ...`.)
+
+Each variant-table row names the launch signature the dispatcher (`launch_h`, gemm_bf16.cu) must produce: the kernels
+seen by torch.profiler (template arguments KE, A mode, B mode, BN included), the change of b200rl_launch_count(), and
+for split-K the number of [M][N] fp32 partial slabs written into a sentinel-filled workspace -- each slab is checked
+against the fp64 partial sum of its own k-range, which pins the split boundaries.  A dispatcher change that moves a row
+to another variant fails here and the row is updated on purpose.  Every output sits inside a sentinel-filled buffer
+(lead bytes, ld padding, extra rows): a store outside the logical region fails the row."""
+import ctypes
+import re
+
 import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
 
 _KEEP = []
+C_ACC = 2.0 ** -16
+C_OUT_BF16 = 2.0 ** -8
+WS_BYTES = 64 << 20
+SENT = 0xFF                 # sentinel byte: 0xFFFF / 0xFFFFFFFF are NaNs no kernel computes
+LEAD = 256                  # guard bytes before an output (keeps the output 256-byte aligned)
+EINVAL = -1
+NONE, RELU, ELU, TANH = 0, 1, 2, 3
+SMS = 148
 
 
 def dev(x, dtype=None):
@@ -27,148 +60,657 @@ def _release():
 
 
 def bf(x):
-  """fp32 array rounded to bf16 (as fp32)."""
+  """array rounded to bf16 (returned as float64, exact)."""
   import torch
-  return torch.as_tensor(np.ascontiguousarray(x, np.float32)).to(torch.bfloat16).float().numpy()
+  return torch.as_tensor(np.ascontiguousarray(x, np.float32)).to(torch.bfloat16).double().numpy()
 
 
-def close(got, want, tol, name=''):
-  got, want = np.asarray(got, np.float64), np.asarray(want, np.float64)
-  scale = max(float(np.abs(want).max()), 1e-30)
-  err = float(np.abs(got - want).max()) / scale
-  assert err <= tol, f'{name}: max error {err:.3e} of scale exceeds {tol:.1e}'
-
-
-def ws():
+def mat_dev(a, ld=None, bf16=True):
+  """[rows][cols] device matrix with row stride ld; the padding columns hold NaN (a kernel that reads them poisons its
+  sums)."""
   import torch
-  t = torch.empty(64 << 20, dtype=torch.uint8, device='cuda')
+  rows, cols = a.shape
+  ld = ld or cols
+  t = torch.full((rows, ld), float('nan'), dtype=torch.bfloat16 if bf16 else torch.float32, device='cuda')
+  t[:, :cols] = torch.as_tensor(np.ascontiguousarray(a, np.float32)).to(t.dtype).cuda()
   _KEEP.append(t)
-  return t.data_ptr(), t.numel()
+  return t
 
 
-OUT_BF16_TOL, OUT_F32_TOL = 6e-3, 2e-4
+class Out:
+  """An output of rows x cols elements (row stride ld) inside a sentinel-filled buffer: LEAD guard bytes before it,
+  ld - cols padding elements per row and `extra` whole rows after it."""
+
+  def __init__(self, rows, cols, bf16, ld=None, extra=3):
+    import torch
+    self.rows, self.cols, self.ld, self.es = rows, cols, ld or cols, 2 if bf16 else 4
+    self.body = rows * self.ld * self.es
+    self.raw = torch.full((LEAD + self.body + extra * self.ld * self.es + 64,), SENT, dtype=torch.uint8, device='cuda')
+    self.ptr = self.raw.data_ptr() + LEAD
+
+  def reset(self):
+    self.raw.fill_(SENT)
+
+  def read(self, what):
+    """The logical region as float64; asserts every other byte still holds the sentinel."""
+    h = self.raw.cpu().numpy()
+    assert (h[:LEAD] == SENT).all() and (h[LEAD + self.body:] == SENT).all(), f'{what}: store outside the output rows'
+    body = h[LEAD:LEAD + self.body].view(np.uint16 if self.es == 2 else np.uint32).reshape(self.rows, self.ld)
+    assert (body[:, self.cols:] == (0xFFFF if self.es == 2 else 0xFFFFFFFF)).all(), f'{what}: store into the ld padding'
+    v = np.ascontiguousarray(body[:, :self.cols])
+    if self.es == 2:
+      v = (v.astype(np.uint32) << 16).view(np.float32)
+    else:
+      v = v.view(np.float32)
+    return v.astype(np.float64)
+
+  def bits(self):
+    return self.raw.clone()
 
 
-@pytest.mark.parametrize('M,N,K', [(256, 1024, 7744), (512, 1024, 7744), (64, 128, 192), (100, 64, 64)])
-def test_linear_bf16(M, N, K):
+def act(v, a):
+  if a == RELU:
+    return np.maximum(v, 0.)
+  if a == ELU:
+    return np.where(v > 0, v, np.expm1(np.minimum(v, 0.)))
+  if a == TANH:
+    return np.tanh(v)
+  return v
+
+
+def act_grad(y, a):
+  """derivative from the activation's OUTPUT y (the mask of a data gradient)"""
+  if a == RELU:
+    return (y > 0).astype(np.float64)
+  if a == ELU:
+    return np.where(y > 0, 1., y + 1.)
+  if a == TANH:
+    return 1. - y * y
+  return np.ones_like(y)
+
+
+def mask_values(rng, shape, a):
+  """a plausible producer output for activation `a`"""
+  z = rng.standard_normal(shape)
+  return np.maximum(z, 0.) if a == RELU else (np.tanh(z) if a == TANH else act(z, ELU))
+
+
+def mask_factor(y, a):
+  """(g, |g| for the bound): the bound carries |A|.|B| * 2^-4 on top of |g| for a computed (non-ReLU) derivative, whose
+  fp32 evaluation (1 - y*y, y + 1) is exact only to ~2^-23 absolute"""
+  g = act_grad(y, a)
+  return g, np.abs(g) + (0. if a == RELU else 2. ** -4)
+
+
+def _check(what, got, ref, absr, out_bf16, c_acc=C_ACC):
+  got = np.asarray(got, np.float64)
+  assert got.shape == ref.shape, (what, got.shape, ref.shape)
+  assert np.isfinite(got).all(), f'{what}: {int((~np.isfinite(got)).sum())} non-finite elements'
+  err = np.abs(got - ref)
+  bound = c_acc * absr + (C_OUT_BF16 if out_bf16 else 0.) * np.abs(ref)
+  acc_err = np.maximum(err - (C_OUT_BF16 * np.abs(ref) if out_bf16 else 0.), 0.)
+  ratio = float((acc_err / np.maximum(absr, 1e-300)).max()) if err.size else 0.
+  used = float((err / np.maximum(bound, 1e-300)).max()) if err.size else 0.
+  print(f'bf16-bound {what}: |err|/(|A||B|) {ratio:.2e}, {used:.3f} of the bound')
+  bad = err > bound
+  if bad.any():
+    i = np.unravel_index(int(np.argmax(err - bound)), err.shape)
+    raise AssertionError(f'{what}: {int(bad.sum())} of {err.size} elements outside the bound; worst at {i}: got {got[i]!r} '
+                         f'want {ref[i]!r} bound {bound[i]:.3e}')
+
+
+def _assert_rejects(what, ref, broken, absr, out_bf16, c_acc=C_ACC):
+  """the bound must fail a result that lost part of its reduction (by at least 2x somewhere, so the rounding noise of a
+  real broken kernel cannot hide it)"""
+  bound = c_acc * absr + (C_OUT_BF16 if out_bf16 else 0.) * np.abs(ref)
+  r = float((np.abs(broken - ref) / np.maximum(bound, 1e-300)).max())
+  print(f'bf16-bound {what}: a broken kernel would exceed the bound {r:.1f}x')
+  assert r >= 2., f'{what}: the bound would accept it (worst |diff| / bound = {r:.2f})'
+
+
+# ------------------------------------------------------------------------------ launch signature
+def _sig_name(name):
+  m = re.search(r'b200rl::(\w+)(<[^>]*>)?', name)
+  return (m.group(1) + (m.group(2) or '')).replace(' ', '') if m else None
+
+
+def run(fn, profile=True):
+  """(launch-count delta, sorted library kernel names seen by torch.profiler) of fn()"""
   import torch
-  from acme_b200 import _capi
-  rng = np.random.default_rng(M + N + K)
+  lib = _capi().load()
+  torch.cuda.synchronize()
+  if not profile:
+    n0 = lib.b200rl_launch_count()
+    fn()
+    torch.cuda.synchronize()
+    return lib.b200rl_launch_count() - n0, None
+  from torch.profiler import ProfilerActivity, profile as prof_ctx
+  with prof_ctx(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+    n0 = lib.b200rl_launch_count()
+    fn()
+    torch.cuda.synchronize()
+    n1 = lib.b200rl_launch_count()
+  names = sorted(n for n in (_sig_name(e.name) for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA) if n)
+  return n1 - n0, names
+
+
+def assert_sig(what, got, want):
+  """want: kernel-name prefixes (template arguments up to BN, STAGES left out)"""
+  launches, names = got
+  assert launches == len(want), f'{what}: {launches} launches, expected {len(want)} ({want}); profiler saw {names}'
+  if names is not None:
+    assert len(names) == len(want) and all(any(n.startswith(w) for n in names) for w in want) and \
+        all(any(n.startswith(w) for w in want) for n in names), f'{what}: kernels {names}, expected {want}'
+
+
+def _capi():
+  from acme_b200 import _capi as c
+  return c
+
+
+def stream():
+  return _capi().current_stream()
+
+
+class Workspace:
+  """split-K workspace filled with the sentinel: `slabs(M, N)` = the number of leading [M][N] fp32 partial slabs that were
+  written completely, asserting that nothing after them was touched"""
+
+  def __init__(self, off=0, nbytes=WS_BYTES):
+    import torch
+    self.buf = torch.full((nbytes + off,), SENT, dtype=torch.uint8, device='cuda')
+    self.off = off
+    self.ptr, self.bytes = self.buf.data_ptr() + off, nbytes
+
+  def reset(self):
+    self.buf.fill_(SENT)
+
+  def slabs(self, what, M, N, splits):
+    import torch
+    words = self.buf[self.off:self.off + self.bytes // 4 * 4].view(torch.int32)
+    n = M * N
+    used = splits * n if splits > 1 else 0
+    assert not bool((words[used:] != -1).any()), f'{what}: workspace written past {splits} partial slab(s)'
+    if splits > 1:
+      assert bool((words[:used] != -1).all()), f'{what}: not all of the {splits} expected partial slabs were written'
+      return words[:used].view(torch.float32).view(splits, M, N).double().cpu().numpy()
+    return None
+
+
+def split_plan(M, N, K, KE, BN, wsb, allow=True):
+  """launch_h's split-K rule -> (splits, k-blocks per split)"""
+  tiles = -(-M // 128) * -(-N // BN)
+  kb = -(-K // KE)
+  s = 1
+  if allow and 2 * tiles <= SMS and kb >= 16:
+    s = max(1, min(-(-SMS // tiles), kb // 8, 64))
+    s = max(1, min(s, wsb // (M * N * 4) if wsb else 0))
+  kps = -(-kb // s)
+  return -(-kb // kps), kps
+
+
+def check_partials(what, slabs, kps, KE, K, partial_ref):
+  """slab s = the fp32 sum over k-blocks [s * kps, (s + 1) * kps): partial_ref(lo, hi) -> (ref, |ref| bound) over k-range
+  [lo, hi)"""
+  for s in range(slabs.shape[0]):
+    lo, hi = s * kps * KE, min(K, (s + 1) * kps * KE)
+    ref, absr = partial_ref(lo, hi)
+    _check(f'{what} split {s} partial (k {lo}..{hi})', slabs[s], ref, absr, False)
+
+
+def drop_ranges(K, KE, splits, kps):
+  """k-ranges a broken kernel might lose: one 64-wide block in the middle, the last (ragged) block, one whole split"""
+  kb = -(-K // KE)
+  blk = 64 // KE
+  mid = (kb // 2) // blk * blk
+  out = [('one 64-wide k-block', mid * KE, min(K, (mid + blk) * KE)), ('the last k-block', (kb - 1) * KE, K)]
+  if splits > 1:
+    s = splits // 2
+    out.append((f'split {s}', s * kps * KE, min(K, (s + 1) * kps * KE)))
+  return out
+
+
+# ------------------------------------------------------------------------------ dense layers
+def lin_ref(x, w, b, lo=0, hi=None):
+  """x @ w^T over k in [lo, hi) (+ b): (value, |x| @ |w|^T (+ |b|))"""
+  hi = x.shape[1] if hi is None else hi
+  xs, ws = x[:, lo:hi], w[:, lo:hi]
+  v, a = xs @ ws.T, np.abs(xs) @ np.abs(ws).T
+  if b is not None:
+    v, a = v + b, a + np.abs(b)
+  return v, a
+
+
+# M, N, K, splits, options; splits from launch_h (min(ceil(148 / tiles), kblocks / 8, 64, ws / (M N 4)), then rounded
+# through kps = ceil(kblocks / splits))
+LINEAR_FWD = [
+    (256, 1024, 7744, 10, {}),                        # the learner's target pass
+    (512, 1024, 7744, 5, {}),                         # the online pass over [o_tm1; o_t]
+    (768, 1024, 7744, 4, {}),
+    (1, 1024, 7744, 14, {}),                          # 15 rounded to 14
+    (64, 18, 7752, 14, {'acts': [NONE, TANH]}),       # BN = 32; ragged last k-block inside the last split
+    (129, 100, 1024, 2, {'acts': [ELU, RELU]}),       # ragged M and N
+    (300, 200, 136, 1, {'acts': [TANH, NONE]}),       # ragged N and K
+    (100, 64, 64, 1, {'acts': [RELU, ELU]}),
+    (33, 1, 512, 1, {'acts': [NONE, RELU], 'ldy': 9}),
+    (256, 1024, 7744, 3, {'wsb': 3 * 256 * 1024 * 4}),   # the workspace caps the split count
+    (256, 1024, 7744, 1, {'ws': None}),               # no workspace: no split
+    (256, 512, 512, 1, {'ldx': 1024, 'ldy': 1024, 'acts': [RELU, TANH]}),
+]
+
+
+@pytest.mark.parametrize('M,N,K,splits,opt', LINEAR_FWD, ids=lambda v: None if not isinstance(v, dict) else
+                         '-'.join(f'{k}{"" if k == "acts" else v[k]}' for k in v) or 'default')
+def test_linear_fwd_bf16(M, N, K, splits, opt):
+  import torch
+  c = _capi()
+  rng = np.random.default_rng(M * 7 + N * 3 + K)
   x, w = bf(rng.standard_normal((M, K))), bf(rng.standard_normal((N, K)) / np.sqrt(K))
-  b = rng.standard_normal(N).astype(np.float32)
-  dy = bf(rng.standard_normal((M, N)))
-  xd, wd, dyd = dev(x, torch.bfloat16), dev(w, torch.bfloat16), dev(dy, torch.bfloat16)
-  wsp, wsb = ws()
-  st = _capi.current_stream()
-  # forward, fp32 and bf16 outputs
-  y = np.maximum(x @ w.T + b, 0)
-  y32 = torch.empty(M, N, device='cuda')
-  _capi.call('b200rl_linear_fwd_bf16', M, N, K, xd.data_ptr(), K, wd.data_ptr(), dev(b).data_ptr(), y32.data_ptr(), N, 0,
-             _capi.ACT_RELU, wsp, wsb, st)
-  close(y32.cpu().numpy(), y, OUT_F32_TOL, 'linear fwd (fp32 out)')
-  y16 = torch.empty(M, N, device='cuda', dtype=torch.bfloat16)
-  _capi.call('b200rl_linear_fwd_bf16', M, N, K, xd.data_ptr(), K, wd.data_ptr(), dev(b).data_ptr(), y16.data_ptr(), N, 1,
-             _capi.ACT_RELU, wsp, wsb, st)
-  close(y16.float().cpu().numpy(), y, OUT_BF16_TOL, 'linear fwd (bf16 out)')
-  # data gradient with the ReLU mask of a bf16 producer output
-  mask = bf(rng.standard_normal((M, K)))
-  dx = (dy @ w) * (mask > 0)
-  dx16 = torch.empty(M, K, device='cuda', dtype=torch.bfloat16)
-  _capi.call('b200rl_linear_dgrad_bf16', M, N, K, dyd.data_ptr(), N, wd.data_ptr(), dx16.data_ptr(), K, 1,
-             dev(mask, torch.bfloat16).data_ptr(), 1, _capi.ACT_RELU, wsp, wsb, st)
-  close(dx16.float().cpu().numpy(), dx, OUT_BF16_TOL, 'linear dgrad')
-  # weight gradient + bias gradient (fp32 outputs)
-  dw, db = dy.T @ x, dy.sum(0)
-  dwd, dbd = torch.empty(N, K, device='cuda'), torch.empty(N, device='cuda')
-  _capi.call('b200rl_linear_wgrad_bf16', M, N, K, dyd.data_ptr(), N, xd.data_ptr(), K, dwd.data_ptr(), dbd.data_ptr(), wsp, wsb, st)
-  close(dwd.cpu().numpy(), dw, OUT_F32_TOL, 'linear wgrad')
-  close(dbd.cpu().numpy(), db, OUT_F32_TOL, 'linear bias grad')
+  b = rng.standard_normal(N).astype(np.float32).astype(np.float64)
+  ldx, acts = opt.get('ldx', K), opt.get('acts', [RELU, RELU])
+  xd, wd, bd = mat_dev(x, ldx), mat_dev(w), dev(b.astype(np.float32))
+  ws = Workspace()
+  wsp, wsb = (ws.ptr, opt.get('wsb', ws.bytes)) if 'ws' not in opt else (None, 0)
+  BN = 32 if N <= 32 else (64 if N <= 64 else 128)
+  plan, kps = split_plan(M, N, K, 64, BN, wsb)
+  assert plan == splits, f'split rule gives {plan}, the table says {splits}'
+  pre, absr = lin_ref(x, w, b)
+  want = [f'hgemm_kernel<64,0,0,{BN},'] + (['splitk_finish_kernel'] if splits > 1 else [])
+  for i, (out_bf16, a) in enumerate(((0, acts[0]), (1, acts[1]))):
+    y = Out(M, N, out_bf16, ld=opt.get('ldy', N))
+    ws.reset()
+    sig = run(lambda: c.call('b200rl_linear_fwd_bf16', M, N, K, xd.data_ptr(), ldx, wd.data_ptr(), bd.data_ptr(), y.ptr, y.ld,
+                             out_bf16, a, wsp, wsb, stream()), profile=i == 0)
+    what = f'linear fwd {M}x{N}x{K} {"bf16" if out_bf16 else "fp32"} out act {a}'
+    assert_sig(what, sig, want)
+    ref = act(pre, a)
+    _check(what, y.read(what), ref, absr, out_bf16)
+    if wsp:
+      slabs = ws.slabs(what, M, N, splits)
+      if i == 0 and splits > 1:
+        check_partials(what, slabs, kps, 64, K, lambda lo, hi: lin_ref(x, w, None, lo, hi))
+    if i == 0 and K >= 1024:
+      for how, lo, hi in drop_ranges(K, 64, splits, kps):
+        _assert_rejects(f'{what} without {how}', ref, act(pre - lin_ref(x, w, None, lo, hi)[0], a), absr, out_bf16)
 
 
+# M, N (reduction), K, BN, lddy, lddx, [(dx_bf16, mask_bf16 or None = no mask, mask_act)]; never split
+LINEAR_DGRAD = [
+    (256, 1024, 7744, 64, 1024, 7744, [(1, 1, RELU), (0, 0, TANH)]),      # BN 128 -> 64: fewer than 148 tiles
+    (512, 1024, 7744, 128, 1024, 7744, [(1, 1, RELU), (0, 1, ELU)]),
+    (129, 100, 128, 64, 104, 136, [(1, 1, TANH), (0, 0, RELU), (1, 0, ELU), (0, None, NONE)]),   # ragged reduction
+    (1, 64, 64, 64, 64, 64, [(1, 1, RELU), (0, 0, TANH)]),
+]
+
+
+@pytest.mark.parametrize('M,N,K,BN,lddy,lddx,cfgs', LINEAR_DGRAD, ids=lambda v: 'cfgs' if isinstance(v, list) else None)
+def test_linear_dgrad_bf16(M, N, K, BN, lddy, lddx, cfgs):
+  c = _capi()
+  rng = np.random.default_rng(M + N + K)
+  dy, w = bf(rng.standard_normal((M, N))), bf(rng.standard_normal((N, K)) / np.sqrt(N))
+  dyd, wd = mat_dev(dy, lddy), mat_dev(w)
+  ws = Workspace()
+  acc, absr = dy @ w, np.abs(dy) @ np.abs(w)
+  for i, (dx_bf16, mask_bf16, ma) in enumerate(cfgs):
+    what = f'linear dgrad {M}x{N}x{K} dx {"bf16" if dx_bf16 else "fp32"} mask {mask_bf16} act {ma}'
+    if mask_bf16 is None:
+      mptr, g, ag = None, 1., 1.
+    else:
+      ym = mask_values(rng, (M, K), ma)
+      ym = bf(ym) if mask_bf16 else ym.astype(np.float32).astype(np.float64)
+      mptr = mat_dev(ym, lddx, bf16=bool(mask_bf16)).data_ptr()        # the mask shares dx's row stride
+      g, ag = mask_factor(ym, ma)
+    dx = Out(M, K, dx_bf16, ld=lddx)
+    sig = run(lambda: c.call('b200rl_linear_dgrad_bf16', M, N, K, dyd.data_ptr(), lddy, wd.data_ptr(), dx.ptr, lddx, dx_bf16,
+                             mptr, mask_bf16 or 0, ma, ws.ptr, ws.bytes, stream()), profile=i == 0)
+    assert_sig(what, sig, [f'hgemm_kernel<64,0,1,{BN},'])
+    ref = acc * g
+    _check(what, dx.read(what), ref, absr * ag, dx_bf16)
+    ws.slabs(what, M, K, 1)
+    if i == 0 and N >= 1024:
+      for how, lo, hi in drop_ranges(N, 64, 1, 1):
+        _assert_rejects(f'{what} without {how}', ref, (acc - dy[:, lo:hi] @ w[lo:hi]) * g, absr * ag, dx_bf16)
+
+
+# M (reduction), N, K, splits, lddy, ldx
+LINEAR_WGRAD = [
+    (256, 1024, 7744, 1, 1024, 7744),
+    (4096, 64, 64, 8, 72, 64),
+    (2000, 64, 128, 4, 64, 136),        # ragged reduction in the last split
+    (33, 64, 128, 1, 72, 136),
+    (1, 128, 64, 1, 128, 64),
+]
+
+
+@pytest.mark.parametrize('M,N,K,splits,lddy,ldx', LINEAR_WGRAD)
+def test_linear_wgrad_bf16(M, N, K, splits, lddy, ldx):
+  c = _capi()
+  rng = np.random.default_rng(M + 2 * N + K)
+  dy, x = bf(rng.standard_normal((M, N))), bf(rng.standard_normal((M, K)))
+  dyd, xd = mat_dev(dy, lddy), mat_dev(x, ldx)
+  ws = Workspace()
+  BN = 128 if K >= 128 else 64
+  plan, kps = split_plan(N, K, M, 64, BN, ws.bytes)
+  assert plan == splits, f'split rule gives {plan}, the table says {splits}'
+  what = f'linear wgrad {M}x{N}x{K}'
+  ref, absr = dy.T @ x, np.abs(dy).T @ np.abs(x)
+  dw = Out(N, K, False)
+  hg = [f'hgemm_kernel<64,1,1,{BN},'] + (['splitk_finish_kernel'] if splits > 1 else [])
+  assert_sig(what, run(lambda: c.call('b200rl_linear_wgrad_bf16', M, N, K, dyd.data_ptr(), lddy, xd.data_ptr(), ldx, dw.ptr, None,
+                                      ws.ptr, ws.bytes, stream())), hg)
+  _check(what, dw.read(what), ref, absr, False)
+  slabs = ws.slabs(what, N, K, splits)
+  if splits > 1:
+    check_partials(what, slabs, kps, 64, M, lambda lo, hi: (dy[lo:hi].T @ x[lo:hi], np.abs(dy[lo:hi]).T @ np.abs(x[lo:hi])))
+  if M >= 1024:
+    for how, lo, hi in drop_ranges(M, 64, splits, kps):
+      _assert_rejects(f'{what} without {how}', ref, ref - dy[lo:hi].T @ x[lo:hi], absr, False)
+  # with the bias gradient: the same dw bit for bit, plus one column-sum launch
+  first = dw.bits()
+  dw.reset()
+  db = Out(1, N, False)
+  ws.reset()
+  assert_sig(what + ' + db', run(lambda: c.call('b200rl_linear_wgrad_bf16', M, N, K, dyd.data_ptr(), lddy, xd.data_ptr(), ldx, dw.ptr,
+                                                db.ptr, ws.ptr, ws.bytes, stream())), hg + ['colsum_vec_kernel<true>'])
+  assert bool((dw.bits() == first).all()), f'{what}: dw changed when db was requested'
+  _check(what + ' db', db.read(what + ' db')[0], dy.sum(0), np.abs(dy).sum(0), False)
+
+
+# ------------------------------------------------------------------------------ convolutions
 def _geom(B, H, C, k, s, Cout):
-  from acme_b200 import _capi, networks
+  from acme_b200 import networks
   oh, pad = networks.tf_same_pad(H, k, s)
-  return _capi.ConvGeom(B=B, H=H, W=H, C=C, kh=k, kw=k, stride=s, pad_top=pad, pad_left=pad, OH=oh, OW=oh, Cout=Cout), oh, pad
+  return _capi().ConvGeom(B=B, H=H, W=H, C=C, kh=k, kw=k, stride=s, pad_top=pad, pad_left=pad, OH=oh, OW=oh, Cout=Cout), oh, pad
 
 
-def _torch_conv(x_nhwc, w_ohwi, b, k, s, H, oh, pad):
-  """TF-SAME convolution in PyTorch-CPU fp32 (explicit asymmetric padding); returns (y NHWC, autograd handles)."""
+def _padded(x, k, s, H, oh, pad):
   import torch
   import torch.nn.functional as F
-  xt = torch.tensor(x_nhwc).permute(0, 3, 1, 2).contiguous().requires_grad_(True)
-  wt = torch.tensor(w_ohwi).permute(0, 3, 1, 2).contiguous().requires_grad_(True)
-  bt = torch.tensor(b).requires_grad_(True)
   total = max((oh - 1) * s + k - H, 0)
-  xp = F.pad(xt, (pad, total - pad, pad, total - pad))
-  y = F.conv2d(xp, wt, bt, stride=s)
-  return y, xt, wt, bt
+  return F.pad(torch.from_numpy(np.ascontiguousarray(x)).permute(0, 3, 1, 2), (pad, total - pad, pad, total - pad))
 
 
-@pytest.mark.parametrize('B,H,C,k,s,Cout', [(6, 21, 32, 4, 2, 64), (6, 11, 64, 3, 1, 64), (40, 21, 32, 4, 2, 64),
-                                             (40, 11, 64, 3, 1, 64)])
-def test_conv_bf16(B, H, C, k, s, Cout):
-  """conv2 / conv3 of the Atari torso (atari.py:45-48): forward + ReLU, data gradient with the producer's ReLU mask,
-  weight and bias gradients."""
+def conv_fwd_ref(x, w, k, s, H, oh, pad):
+  """TF-SAME convolution in fp64 (explicit asymmetric padding): NHWC x, OHWI w -> NHWC"""
+  import torch.nn.functional as F
   import torch
-  from acme_b200 import _capi
-  rng = np.random.default_rng(B + H + C)
+  return F.conv2d(_padded(x, k, s, H, oh, pad), torch.from_numpy(np.ascontiguousarray(w)).permute(0, 3, 1, 2),
+                  stride=s).permute(0, 2, 3, 1).numpy()
+
+
+def conv_wgrad_ref(x, dy, k, s, H, oh, pad, C):
+  """sum over pixels of patch x dy -> OHWI"""
+  import torch
+  xp = _padded(x, k, s, H, oh, pad)
+  dyt = torch.from_numpy(np.ascontiguousarray(dy)).permute(0, 3, 1, 2)
+  return torch.nn.grad.conv2d_weight(xp, (dy.shape[3], C, k, k), dyt, stride=s).permute(0, 2, 3, 1).numpy()
+
+
+def conv_dgrad_ref(dy, w, k, s, H, oh, pad):
+  import torch
+  total = max((oh - 1) * s + k - H, 0)
+  B, C = dy.shape[0], w.shape[3]
+  dyt = torch.from_numpy(np.ascontiguousarray(dy)).permute(0, 3, 1, 2)
+  dxp = torch.nn.grad.conv2d_input((B, C, H + total, H + total), torch.from_numpy(np.ascontiguousarray(w)).permute(0, 3, 1, 2),
+                                   dyt, stride=s)
+  return dxp[:, :, pad:pad + H, pad:pad + H].permute(0, 2, 3, 1).numpy()
+
+
+def wk(w, lo, hi):
+  """OHWI weights with only the flattened reduction indices [lo, hi) kept: (tap, channel) order = the kernels' k order"""
+  f = np.zeros_like(w).reshape(w.shape[0], -1)
+  f[:, lo:hi] = w.reshape(w.shape[0], -1)[:, lo:hi]
+  return f.reshape(w.shape)
+
+
+def wgrad_range(x, dy, lo, hi, k, s, H, oh, pad, C):
+  """weight gradient (value, |x| |dy| bound) over the flattened output pixels [lo, hi) only -- the k-range of a weight
+  gradient's split or k-block; computed on the images that range touches"""
+  hw, Cout = oh * oh, dy.shape[-1]
+  b0, b1 = lo // hw, (hi - 1) // hw + 1
+  d = np.zeros(((b1 - b0) * hw, Cout))
+  d[lo - b0 * hw:hi - b0 * hw] = dy.reshape(-1, Cout)[lo:hi]
+  d = d.reshape(b1 - b0, oh, oh, Cout)
+  return (conv_wgrad_ref(x[b0:b1], d, k, s, H, oh, pad, C), conv_wgrad_ref(np.abs(x[b0:b1]), np.abs(d), k, s, H, oh, pad, C))
+
+
+# B, H, C, k, s, Cout, splits
+CONV_FWD = [
+    (1, 21, 32, 4, 2, 64, 2), (6, 21, 32, 4, 2, 64, 2), (256, 21, 32, 4, 2, 64, 1), (512, 21, 32, 4, 2, 64, 1),   # conv2
+    (1, 11, 64, 3, 1, 64, 1), (40, 11, 64, 3, 1, 64, 1), (256, 11, 64, 3, 1, 64, 1), (512, 11, 64, 3, 1, 64, 1),  # conv3
+    (6, 11, 64, 3, 1, 32, 1), (40, 21, 32, 4, 2, 128, 2), (6, 11, 128, 3, 1, 128, 2),
+    (6, 13, 32, 4, 2, 64, 2),           # odd H: asymmetric SAME padding (1 top / left, 2 bottom / right)
+]
+
+
+@pytest.mark.parametrize('B,H,C,k,s,Cout,splits', CONV_FWD)
+def test_conv_fwd_bf16(B, H, C, k, s, Cout, splits):
+  c = _capi()
+  rng = np.random.default_rng(B + H + C + Cout)
   g, oh, pad = _geom(B, H, C, k, s, Cout)
+  K, M, KE = k * k * C, B * oh * oh, 32 if C == 32 else 64
   x = bf(np.maximum(rng.standard_normal((B, H, H, C)), 0))
-  w = bf(rng.standard_normal((Cout, k, k, C)) / np.sqrt(k * k * C))
-  b = (rng.standard_normal(Cout) * 0.1).astype(np.float32)
-  y, xt, wt, bt = _torch_conv(x, w, b, k, s, H, oh, pad)
-  yr = torch.relu(y)
-  dy = bf(rng.standard_normal((B, oh, oh, Cout)) * (yr.permute(0, 2, 3, 1).detach().numpy() > 0))   # d(pre-activation)
-  y.backward(torch.tensor(dy).permute(0, 3, 1, 2))
-  wsp, wsb = ws()
-  st = _capi.current_stream()
-  xd, wd, dyd = dev(x, torch.bfloat16), dev(w, torch.bfloat16), dev(dy, torch.bfloat16)
-  yd = torch.empty(B, oh, oh, Cout, device='cuda', dtype=torch.bfloat16)
-  _capi.call('b200rl_conv2d_fwd_bf16', xd.data_ptr(), 0, wd.data_ptr(), dev(b).data_ptr(), yd.data_ptr(), 1, g, _capi.ACT_RELU,
-             wsp, wsb, st)
-  close(yd.float().cpu().numpy(), yr.permute(0, 2, 3, 1).detach().numpy(), OUT_BF16_TOL, 'conv fwd')
-  dxd = torch.empty(B, H, H, C, device='cuda', dtype=torch.bfloat16)
-  _capi.call('b200rl_conv2d_dgrad_bf16', dyd.data_ptr(), wd.data_ptr(), dxd.data_ptr(), 1, g, xd.data_ptr(), 1, _capi.ACT_RELU, st)
-  close(dxd.float().cpu().numpy(), xt.grad.permute(0, 2, 3, 1).numpy() * (x > 0), OUT_BF16_TOL, 'conv dgrad')
-  dwd, dbd = torch.empty(Cout, k, k, C, device='cuda'), torch.empty(Cout, device='cuda')
-  _capi.call('b200rl_conv2d_wgrad_bf16', xd.data_ptr(), 0, dyd.data_ptr(), dwd.data_ptr(), dbd.data_ptr(), g, wsp, wsb, st)
-  close(dwd.cpu().numpy(), wt.grad.permute(0, 2, 3, 1).numpy(), OUT_F32_TOL, 'conv wgrad')
-  close(dbd.cpu().numpy(), bt.grad.numpy(), OUT_F32_TOL, 'conv bias grad')
+  w = bf(rng.standard_normal((Cout, k, k, C)) / np.sqrt(K))
+  b = (rng.standard_normal(Cout) * 0.1).astype(np.float32).astype(np.float64)
+  xd, wd, bd = dev(x, _bf16()), dev(w, _bf16()), dev(b.astype(np.float32))
+  acc, absr = conv_fwd_ref(x, w, k, s, H, oh, pad), conv_fwd_ref(np.abs(x), np.abs(w), k, s, H, oh, pad) + np.abs(b)
+  pre = (acc + b).reshape(M, Cout)
+  absr, acc = absr.reshape(M, Cout), acc.reshape(M, Cout)
+  ws = Workspace()
+  plan, kps = split_plan(M, Cout, K, KE, Cout, ws.bytes)
+  assert plan == splits, f'split rule gives {plan}, the table says {splits}'
+  want = [f'hgemm_kernel<{KE},0,0,{Cout},'] + (['splitk_finish_kernel'] if splits > 1 else [])
+  a2 = (NONE, ELU, TANH)[(B + H) % 3]
+  for i, (out_bf16, a) in enumerate(((1, RELU), (0, a2))):
+    what = f'conv fwd B{B} H{H} C{C} k{k} s{s} Cout{Cout} {"bf16" if out_bf16 else "fp32"} out act {a}'
+    y = Out(M, Cout, out_bf16)
+    ws.reset()
+    assert_sig(what, run(lambda: c.call('b200rl_conv2d_fwd_bf16', xd.data_ptr(), 0, wd.data_ptr(), bd.data_ptr(), y.ptr, out_bf16, g,
+                                        a, ws.ptr, ws.bytes, stream()), profile=i == 0), want)
+    ref = act(pre, a)
+    _check(what, y.read(what), ref, absr, out_bf16)
+    slabs = ws.slabs(what, M, Cout, splits)
+    if i == 0 and splits > 1:
+      check_partials(what, slabs, kps, KE, K, lambda lo, hi: (
+          conv_fwd_ref(x, wk(w, lo, hi), k, s, H, oh, pad).reshape(M, Cout),
+          conv_fwd_ref(np.abs(x), np.abs(wk(w, lo, hi)), k, s, H, oh, pad).reshape(M, Cout)))
+    if i == 0 and K >= 1024:
+      for how, lo, hi in drop_ranges(K, KE, splits, kps):
+        lost = conv_fwd_ref(x, wk(w, lo, hi), k, s, H, oh, pad).reshape(M, Cout)
+        _assert_rejects(f'{what} without {how}', ref, act(pre - lost, a), absr, out_bf16)
 
 
-@pytest.mark.parametrize('B', [5, 33])
-def test_conv1_rows_bf16(B):
-  """First layer on uint8 frames (atari.py:44, atari_wrapper.py:303-304): integer-valued bf16 row image, 1/255 applied to
-  the accumulator; forward and weight gradient."""
-  import ctypes
+def _bf16():
   import torch
-  from acme_b200 import _capi
-  rng = np.random.default_rng(B)
-  H, C, k, s, Cout = 84, 4, 8, 4, 32
+  return torch.bfloat16
+
+
+# B, H, C, k, s, Cout, splits
+CONV_WGRAD = [(B, H, C, k, s, Cout, sp) for (H, C, k, s) in ((21, 32, 4, 2), (11, 64, 3, 1)) for Cout in (32, 64)
+              for B, sp in ((1, 1), (256, 35 if C == 32 else 29))]
+
+
+@pytest.mark.parametrize('B,H,C,k,s,Cout,splits', CONV_WGRAD)
+def test_conv_wgrad_bf16(B, H, C, k, s, Cout, splits):
+  """all four (C, Cout) template pairs: <64,1,1,64>, <64,2,1,64>, <64,2,2,32>, <64,1,2,32>"""
+  c = _capi()
+  rng = np.random.default_rng(B + H + C + 3 * Cout)
   g, oh, pad = _geom(B, H, C, k, s, Cout)
+  K, P = k * k * C, B * oh * oh
+  x = bf(np.maximum(rng.standard_normal((B, H, H, C)), 0))
+  dy = bf(rng.standard_normal((B, oh, oh, Cout)))
+  xd, dyd = dev(x, _bf16()), dev(dy, _bf16())
+  ws = Workspace()
+  BN = Cout
+  plan, kps = split_plan(K, Cout, P, 64, BN, ws.bytes)
+  assert plan == splits, f'split rule gives {plan}, the table says {splits}'
+  what = f'conv wgrad B{B} H{H} C{C} k{k} s{s} Cout{Cout}'
+  wr = lambda lo, hi: wgrad_range(x, dy, lo, hi, k, s, H, oh, pad, C)
+  ref, absr = (r.reshape(Cout, K) for r in wr(0, P))
+  am, bm = 1 if C == 64 else 2, 1 if Cout == 64 else 2
+  hg = [f'hgemm_kernel<64,{am},{bm},{BN},'] + (['splitk_finish_kernel'] if splits > 1 else [])
+  dw = Out(Cout, K, False)
+  assert_sig(what, run(lambda: c.call('b200rl_conv2d_wgrad_bf16', xd.data_ptr(), 0, dyd.data_ptr(), dw.ptr, None, g, ws.ptr,
+                                      ws.bytes, stream())), hg)
+  _check(what, dw.read(what), ref, absr, False)
+  slabs = ws.slabs(what, K, Cout, splits)
+  if splits > 1:   # partial slabs hold dW^T: [(tap, channel)][Cout]
+    check_partials(what, slabs, kps, 64, P, lambda lo, hi: tuple(r.reshape(Cout, K).T for r in wr(lo, hi)))
+  if P >= 1024:
+    for how, lo, hi in drop_ranges(P, 64, splits, kps):
+      _assert_rejects(f'{what} without {how}', ref, ref - wr(lo, hi)[0].reshape(Cout, K), absr, False)
+  first = dw.bits()
+  dw.reset()
+  db = Out(1, Cout, False)
+  ws.reset()
+  assert_sig(what + ' + db', run(lambda: c.call('b200rl_conv2d_wgrad_bf16', xd.data_ptr(), 0, dyd.data_ptr(), dw.ptr, db.ptr, g,
+                                                ws.ptr, ws.bytes, stream())), hg + ['colsum_vec_kernel<true>'])
+  assert bool((dw.bits() == first).all()), f'{what}: dw changed when db was requested'
+  d2 = dy.reshape(-1, Cout)
+  _check(what + ' db', db.read(what + ' db')[0], d2.sum(0), np.abs(d2).sum(0), False)
+
+
+# B, H, C, k, s, Cout, dx_bf16, mask_bf16 (None: no mask), mask_act
+CONV_DGRAD = [
+    (1, 21, 32, 4, 2, 64, 1, 1, RELU), (6, 21, 32, 4, 2, 64, 0, 0, RELU), (256, 21, 32, 4, 2, 64, 1, 1, RELU),   # conv2
+    (6, 20, 32, 4, 2, 64, 1, 0, ELU),                                                                            # even H
+    (1, 11, 64, 3, 1, 64, 0, 1, TANH), (6, 11, 64, 3, 1, 64, 1, None, NONE), (256, 11, 64, 3, 1, 64, 1, 1, RELU),  # conv3
+    (6, 11, 128, 3, 1, 128, 0, 0, RELU), (6, 13, 64, 4, 2, 128, 1, 1, TANH), (1, 10, 128, 3, 2, 64, 1, 0, RELU),
+    (256, 13, 32, 4, 2, 128, 0, 1, ELU),
+]
+
+
+@pytest.mark.parametrize('B,H,C,k,s,Cout,dx_bf16,mask_bf16,ma', CONV_DGRAD)
+def test_conv_dgrad_bf16(B, H, C, k, s, Cout, dx_bf16, mask_bf16, ma):
+  """one stride-1 sub-problem per stride phase; odd H gives the phases unequal pixel counts"""
+  c = _capi()
+  rng = np.random.default_rng(B + H + C + Cout + s)
+  g, oh, pad = _geom(B, H, C, k, s, Cout)
+  w = bf(rng.standard_normal((Cout, k, k, C)) / np.sqrt(k * k * Cout))
+  dy = bf(rng.standard_normal((B, oh, oh, Cout)))
+  wd, dyd = dev(w, _bf16()), dev(dy, _bf16())
+  M = B * H * H
+  if mask_bf16 is None:
+    mptr, gm, ag = None, 1., 1.
+  else:
+    ym = mask_values(rng, (M, C), ma)
+    ym = bf(ym) if mask_bf16 else ym.astype(np.float32).astype(np.float64)
+    mptr = mat_dev(ym, bf16=bool(mask_bf16)).data_ptr()
+    gm, ag = mask_factor(ym, ma)
+  acc = conv_dgrad_ref(dy, w, k, s, H, oh, pad).reshape(M, C)
+  absr = conv_dgrad_ref(np.abs(dy), np.abs(w), k, s, H, oh, pad).reshape(M, C) * ag
+  ref = acc * gm
+  what = f'conv dgrad B{B} H{H} C{C} k{k} s{s} Cout{Cout} dx {"bf16" if dx_bf16 else "fp32"} mask {mask_bf16} act {ma}'
+  dx = Out(M, C, dx_bf16)
+  assert_sig(what, run(lambda: c.call('b200rl_conv2d_dgrad_bf16', dyd.data_ptr(), wd.data_ptr(), dx.ptr, dx_bf16, g, mptr,
+                                      mask_bf16 or 0, ma, stream())), [f'hconv_dgrad_kernel<{C}>'])
+  _check(what, dx.read(what), ref, absr, dx_bf16)
+  red = -(-k // s) ** 2 * Cout     # reduction length of the largest stride phase
+  if red >= 1024:
+    co = np.zeros_like(w)
+    co[:64, k // 2, k // 2] = w[:64, k // 2, k // 2]      # one 64-wide k-block: 64 output channels of one tap
+    lost = conv_dgrad_ref(dy, co, k, s, H, oh, pad).reshape(M, C)
+    _assert_rejects(f'{what} without one 64-wide k-block', ref, (acc - lost) * gm, absr, dx_bf16)
+
+
+# ------------------------------------------------------------------------------ first layer (uint8 frames, row image)
+# B, H, Cout, forward persistent, weight-gradient splits
+CONV1_ROWS = [
+    (1, 84, 32, False, 1), (5, 84, 32, False, 4), (33, 84, 32, False, 26),
+    (171, 84, 32, False, 63),   # 590 tiles: one tile per CTA
+    (172, 84, 32, True, 63),    # 593 tiles >= 4 x 148: persistent CTAs with resident weights
+    (256, 84, 32, True, 63),    # weight gradient: 64 splits (SPLITK_MAX) rounded to 63
+    (512, 84, 32, True, 63),
+    (33, 84, 64, False, 26),    # Cout = 64: weights too large to stay resident, never persistent
+    (5, 20, 32, False, 1),
+]
+
+
+@pytest.mark.parametrize('B,H,Cout,pers,wsplits', CONV1_ROWS)
+def test_conv1_rows_bf16(B, H, Cout, pers, wsplits):
+  """First layer on uint8 frames (atari.py:44, atari_wrapper.py:303-304): integer-valued bf16 row image, 1/255 applied to
+  the accumulator; forward, weight and bias gradients."""
+  import torch
+  c = _capi()
+  rng = np.random.default_rng(B + H + Cout)
+  C, k, s = 4, 8, 4
+  g, oh, pad = _geom(B, H, C, k, s, Cout)
+  K, M = k * k * C, B * oh * oh
   frames = rng.integers(0, 256, (B, H, H, C), dtype=np.uint8)
-  w = bf(rng.standard_normal((Cout, k, k, C)) / np.sqrt(k * k * C))
-  b = (rng.standard_normal(Cout) * 0.1).astype(np.float32)
-  x = (frames.astype(np.float32) / np.float32(255)).astype(np.float32)
-  y, xt, wt, bt = _torch_conv(x, w, b, k, s, H, oh, pad)
-  yr = torch.relu(y)
-  dy = bf(rng.standard_normal((B, oh, oh, Cout)) * (yr.permute(0, 2, 3, 1).detach().numpy() > 0))
-  y.backward(torch.tensor(dy).permute(0, 3, 1, 2))
-  nbytes = int(_capi.load().b200rl_conv2d_rows_bf16_bytes(ctypes.byref(g)))
+  w = bf(rng.standard_normal((Cout, k, k, C)) / np.sqrt(K))
+  b = (rng.standard_normal(Cout) * 0.1).astype(np.float32).astype(np.float64)
+  x = frames.astype(np.float64) / 255.
+  nbytes = int(c.load().b200rl_conv2d_rows_bf16_bytes(ctypes.byref(g)))
   assert nbytes > 0
   rows = torch.empty(nbytes, dtype=torch.uint8, device='cuda')
-  st = _capi.current_stream()
-  _capi.call('b200rl_conv2d_rows_bf16_from_u8', dev(frames).data_ptr(), g, rows.data_ptr(), nbytes, st)
-  wsp, wsb = ws()
-  yd = torch.empty(B, oh, oh, Cout, device='cuda', dtype=torch.bfloat16)
-  _capi.call('b200rl_conv2d_fwd_bf16', rows.data_ptr(), 1, dev(w, torch.bfloat16).data_ptr(), dev(b).data_ptr(), yd.data_ptr(), 1,
-             g, _capi.ACT_RELU, wsp, wsb, st)
-  close(yd.float().cpu().numpy(), yr.permute(0, 2, 3, 1).detach().numpy(), OUT_BF16_TOL, 'conv1 fwd')
-  dwd, dbd = torch.empty(Cout, k, k, C, device='cuda'), torch.empty(Cout, device='cuda')
-  _capi.call('b200rl_conv2d_wgrad_bf16', rows.data_ptr(), 1, dev(dy, torch.bfloat16).data_ptr(), dwd.data_ptr(), dbd.data_ptr(),
-             g, wsp, wsb, st)
-  close(dwd.cpu().numpy(), wt.grad.permute(0, 2, 3, 1).numpy(), OUT_F32_TOL, 'conv1 wgrad')
-  close(dbd.cpu().numpy(), bt.grad.numpy(), OUT_F32_TOL, 'conv1 bias grad')
+  c.call('b200rl_conv2d_rows_bf16_from_u8', dev(frames).data_ptr(), g, rows.data_ptr(), nbytes, stream())
+  wd, bd = dev(w, _bf16()), dev(b.astype(np.float32))
+  ws = Workspace()
+  # forward (never split: 8 k-blocks)
+  what = f'conv1 fwd B{B} H{H} Cout{Cout}'
+  acc = conv_fwd_ref(x, w, k, s, H, oh, pad).reshape(M, Cout)
+  absr = conv_fwd_ref(x, np.abs(w), k, s, H, oh, pad).reshape(M, Cout) + np.abs(b)
+  y = Out(M, Cout, True)
+  want = ['hgemm_pers_kernel<32,0,32,' if pers else f'hgemm_kernel<32,0,0,{Cout},']
+  assert_sig(what, run(lambda: c.call('b200rl_conv2d_fwd_bf16', rows.data_ptr(), 1, wd.data_ptr(), bd.data_ptr(), y.ptr, 1, g, RELU,
+                                      ws.ptr, ws.bytes, stream())), want)
+  _check(what, y.read(what), act(acc + b, RELU), absr, True)
+  ws.slabs(what, M, Cout, 1)
+  # weight gradient: dy of the bf16 dataflow
+  dy = bf(rng.standard_normal((B, oh, oh, Cout)) * (acc.reshape(B, oh, oh, Cout) + b > 0))
+  dyd = dev(dy, _bf16())
+  plan, kps = split_plan(K, Cout, M, 64, Cout, ws.bytes)
+  assert plan == wsplits, f'split rule gives {plan}, the table says {wsplits}'
+  what = f'conv1 wgrad B{B} H{H} Cout{Cout}'
+  wr = lambda lo, hi: wgrad_range(x, dy, lo, hi, k, s, H, oh, pad, C)
+  ref, absr = (r.reshape(Cout, K) for r in wr(0, M))
+  hg = [f'hgemm_kernel<64,2,{2 if Cout == 32 else 1},{Cout},'] + (['splitk_finish_kernel'] if wsplits > 1 else [])
+  dw, db = Out(Cout, K, False), Out(1, Cout, False)
+  ws.reset()
+  assert_sig(what, run(lambda: c.call('b200rl_conv2d_wgrad_bf16', rows.data_ptr(), 1, dyd.data_ptr(), dw.ptr, None, g, ws.ptr,
+                                      ws.bytes, stream())), hg)
+  _check(what, dw.read(what), ref, absr, False)
+  slabs = ws.slabs(what, K, Cout, wsplits)
+  if wsplits > 1:   # raw integer-pixel sums: the 1/255 is applied when the partials are combined
+    check_partials(what, slabs, kps, 64, M, lambda lo, hi: tuple(255. * r.reshape(Cout, K).T for r in wr(lo, hi)))
+  if M >= 1024:
+    for how, lo, hi in drop_ranges(M, 64, wsplits, kps):
+      _assert_rejects(f'{what} without {how}', ref, ref - wr(lo, hi)[0].reshape(Cout, K), absr, False)
+  first = dw.bits()
+  dw.reset()
+  ws.reset()
+  assert_sig(what + ' + db', run(lambda: c.call('b200rl_conv2d_wgrad_bf16', rows.data_ptr(), 1, dyd.data_ptr(), dw.ptr, db.ptr, g,
+                                                ws.ptr, ws.bytes, stream()), profile=False), hg + ['colsum_vec_kernel<true>'])
+  assert bool((dw.bits() == first).all()), f'{what}: dw changed when db was requested'
+  d2 = dy.reshape(-1, Cout)
+  _check(what + ' db', db.read(what + ' db')[0], d2.sum(0), np.abs(d2).sum(0), False)
+
+
+def test_conv1_wgrad_unaligned_workspace():
+  """A split-K weight gradient of the first layer with a workspace that is only 4-byte aligned: the partial sums take the
+  per-element store path, which must still write the raw partials (the 1/255 belongs to the combining pass)."""
+  import torch
+  c = _capi()
+  rng = np.random.default_rng(3)
+  B, H, C, k, s, Cout = 33, 84, 4, 8, 4, 32
+  g, oh, pad = _geom(B, H, C, k, s, Cout)
+  K, M = k * k * C, B * oh * oh
+  frames = rng.integers(0, 256, (B, H, H, C), dtype=np.uint8)
+  x = frames.astype(np.float64) / 255.
+  nbytes = int(c.load().b200rl_conv2d_rows_bf16_bytes(ctypes.byref(g)))
+  rows = torch.empty(nbytes, dtype=torch.uint8, device='cuda')
+  c.call('b200rl_conv2d_rows_bf16_from_u8', dev(frames).data_ptr(), g, rows.data_ptr(), nbytes, stream())
+  dy = bf(rng.standard_normal((B, oh, oh, Cout)))
+  ws = Workspace(off=4)
+  dw = Out(Cout, K, False)
+  assert_sig('conv1 wgrad, unaligned workspace', run(lambda: c.call(
+      'b200rl_conv2d_wgrad_bf16', rows.data_ptr(), 1, dev(dy, _bf16()).data_ptr(), dw.ptr, None, g, ws.ptr, ws.bytes, stream())),
+      ['hgemm_kernel<64,2,2,32,', 'splitk_finish_kernel'])
+  ref, absr = (r.reshape(Cout, K) for r in wgrad_range(x, dy, 0, M, k, s, H, oh, pad, C))
+  _check('conv1 wgrad, unaligned workspace', dw.read('conv1 wgrad'), ref, absr, False)
+  ws.slabs('conv1 wgrad, unaligned workspace', K, Cout, 26)
+
+
 
 
 def test_fused_head_td_matches_unfused_kernels():
@@ -268,3 +810,176 @@ def test_gather_rows_equals_gather_plus_conversion(hw):
   assert torch.equal(ds.o_both, o_both) and torch.equal(ds.R, R) and torch.equal(ds.D, D) and torch.equal(ds.a_tm1, a)
   assert torch.equal(rows, want)
   server.stop()
+
+
+# ------------------------------------------------------------------------------ column sums, fp32 -> bf16
+@pytest.mark.parametrize('M,N,ld', [(1, 32, 32), (121, 64, 72), (30976, 64, 64), (112896, 32, 40), (256, 1024, 1032),
+                                    (30976, 4, 8)])
+def test_colsum_bf16(M, N, ld):
+  c = _capi()
+  rng = np.random.default_rng(M + N)
+  x = bf(rng.standard_normal((M, N)))
+  xd = mat_dev(x, ld)
+  ws = Workspace()
+  out = Out(1, N, False)
+  assert_sig(f'colsum {M}x{N}', run(lambda: c.call('b200rl_colsum_bf16', M, N, xd.data_ptr(), ld, out.ptr, ws.ptr, ws.bytes,
+                                                   stream())), ['colsum_vec_kernel<true>'])
+  _check(f'colsum {M}x{N} ld {ld}', out.read('colsum')[0], x.sum(0), np.abs(x).sum(0), False)
+
+
+@pytest.mark.parametrize('n', [0, 8, 64, 8_000_000])
+def test_bf16_from_f32_rounds_to_nearest_even(n):
+  import torch
+  c = _capi()
+  rng = np.random.default_rng(n)
+  src = (rng.standard_normal(n) * np.exp2(rng.integers(-140, 120, n))).astype(np.float32)
+  # ties to even (up, down, negative), +-0, subnormals, +-Inf, FLT_MAX -> Inf, NaN; then below-tie, more subnormals, NaNs
+  special = np.array([0x3F808000, 0x3F818000, 0x80000000, 0x00000001, 0x7F800000, 0xFF800000, 0x7F7FFFFF, 0x7FC00000,
+                      0xBF808000, 0x3F807FFF, 0x00000000, 0x807FFFFF, 0x00408000, 0xFF7FFFFF, 0x7F7F8000, 0x7F800001],
+                     np.uint32).view(np.float32)
+  src[:min(n, special.size)] = special[:n]
+  if not n:    # nothing to convert: no launch, nothing written
+    s, out = dev(np.zeros(8, np.float32)), Out(1, 8, True)
+    assert_sig('bf16_from_f32 n=0', run(lambda: c.call('b200rl_bf16_from_f32', 0, s.data_ptr(), out.ptr, stream())), [])
+    assert bool((out.raw == SENT).all())
+    return
+  s = dev(src)
+  out = Out(1, n, True)
+  assert_sig(f'bf16_from_f32 n={n}', run(lambda: c.call('b200rl_bf16_from_f32', n, s.data_ptr(), out.ptr, stream())),
+             ['f32_to_bf16_kernel'])
+  got = out.read('bf16_from_f32')[0]
+  want = torch.from_numpy(src).to(torch.bfloat16).double().numpy()
+  nan = np.isnan(want)
+  assert (np.isnan(got) == nan).all(), 'NaN-ness differs'
+  assert (got[~nan].view(np.uint64) == want[~nan].view(np.uint64)).all(), \
+      f'rounding differs at {np.flatnonzero(got[~nan].view(np.uint64) != want[~nan].view(np.uint64))[:8]}'
+
+
+# ------------------------------------------------------------------------------ shapes outside the kernels
+def _rejects(what, fn_name, out, *args):
+  lib = _capi().load()
+  n0 = lib.b200rl_launch_count()
+  rc = getattr(lib, fn_name)(*args)
+  import torch
+  torch.cuda.synchronize()
+  assert rc == EINVAL, f'{what}: rc {rc}, expected EINVAL'
+  assert lib.b200rl_launch_count() == n0, f'{what}: launched a kernel'
+  assert bool((out.raw == SENT).all()), f'{what}: output written'
+  with pytest.raises(ValueError):
+    _capi().check(rc)
+
+
+def test_shapes_outside_the_kernels_are_rejected():
+  import torch
+  c = _capi()
+  ws = Workspace(nbytes=1 << 20)
+  big = torch.zeros(1 << 20, dtype=torch.bfloat16, device='cuda')
+  p = big.data_ptr()
+  y = Out(64, 256, False)
+  _rejects('linear fwd K < 64', 'b200rl_linear_fwd_bf16', y, 64, 64, 32, p, 32, p, None, y.ptr, 64, 0, RELU, ws.ptr, ws.bytes, None)
+  _rejects('linear fwd ldx * 2 % 16 != 0', 'b200rl_linear_fwd_bf16', y, 64, 64, 64, p, 65, p, None, y.ptr, 64, 0, RELU, ws.ptr,
+           ws.bytes, None)
+  _rejects('linear dgrad K % 64 != 0', 'b200rl_linear_dgrad_bf16', y, 64, 64, 96, p, 64, p, y.ptr, 96, 0, None, 0, 0, ws.ptr,
+           ws.bytes, None)
+  _rejects('linear wgrad N % 64 != 0', 'b200rl_linear_wgrad_bf16', y, 64, 96, 64, p, 96, p, 64, y.ptr, None, ws.ptr, ws.bytes, None)
+  _rejects('colsum N = 100', 'b200rl_colsum_bf16', y, 64, 100, p, 100, y.ptr, ws.ptr, ws.bytes, None)
+  _rejects('bf16_from_f32 n % 8 != 0', 'b200rl_bf16_from_f32', y, 12, p, y.ptr, None)
+  for what, geo, fn in (('conv fwd C = 16', (2, 11, 16, 3, 1, 64), 'fwd'), ('conv fwd Cout = 48', (2, 11, 64, 3, 1, 48), 'fwd'),
+                        ('conv wgrad C = 16', (2, 11, 16, 3, 1, 64), 'wgrad'), ('conv dgrad stride 3', (2, 12, 64, 3, 3, 64), 'dgrad'),
+                        ('conv dgrad Cout = 48', (2, 11, 64, 3, 1, 48), 'dgrad')):
+    g, _, _ = _geom(*geo)
+    if fn == 'fwd':
+      _rejects(what, 'b200rl_conv2d_fwd_bf16', y, p, 0, p, None, y.ptr, 1, ctypes.byref(g), RELU, ws.ptr, ws.bytes, None)
+    elif fn == 'wgrad':
+      _rejects(what, 'b200rl_conv2d_wgrad_bf16', y, p, 0, p, y.ptr, None, ctypes.byref(g), ws.ptr, ws.bytes, None)
+    else:
+      _rejects(what, 'b200rl_conv2d_dgrad_bf16', y, p, p, y.ptr, 1, ctypes.byref(g), None, 0, 0, None)
+
+
+# ------------------------------------------------------------------------------ launch ordering
+def test_pdl_and_graph_capture_leave_results_bit_identical():
+  """fc1 forward -> data gradient -> weight + bias gradient, then conv3 data gradient -> conv2 weight gradient on one
+  stream: eager with programmatic dependent launch at its default, eager with it off, and captured in a CUDA graph
+  (replayed twice) give the same bits.  Split-K combines its partials in a fixed order.  Then two split-K GEMMs on two
+  streams at once, each with its own workspace, equal the two run one after the other."""
+  import torch
+  c = _capi()
+  lib = c.load()
+  rng = np.random.default_rng(11)
+  M, N, K = 256, 1024, 7744
+  x = dev(bf(rng.standard_normal((M, K))), _bf16())
+  w = dev(bf(rng.standard_normal((N, K)) / 88.), _bf16())
+  b = dev(rng.standard_normal(N).astype(np.float32))
+  dy = dev(bf(rng.standard_normal((M, N))), _bf16())
+  g3, _, _ = _geom(M, 11, 64, 3, 1, 64)
+  g2, _, _ = _geom(M, 21, 32, 4, 2, 64)
+  dy3 = dev(bf(rng.standard_normal((M, 11, 11, 64))), _bf16())
+  w3 = dev(bf(rng.standard_normal((64, 3, 3, 64)) / 24.), _bf16())
+  m3 = dev(bf(np.maximum(rng.standard_normal((M, 11, 11, 64)), 0)), _bf16())
+  x2 = dev(bf(np.maximum(rng.standard_normal((M, 21, 21, 32)), 0)), _bf16())
+  ws = torch.zeros(WS_BYTES, dtype=torch.uint8, device='cuda')
+  outs = dict(y=torch.empty(M, N, dtype=torch.bfloat16, device='cuda'), dx=torch.empty(M, K, dtype=torch.bfloat16, device='cuda'),
+              dw=torch.empty(N, K, device='cuda'), db=torch.empty(N, device='cuda'),
+              dx3=torch.empty(M, 11, 11, 64, dtype=torch.bfloat16, device='cuda'), dw2=torch.empty(64, 4, 4, 32, device='cuda'),
+              db2=torch.empty(64, device='cuda'))
+  o = {k: v.data_ptr() for k, v in outs.items()}
+
+  def chain():
+    st = stream()
+    c.call('b200rl_linear_fwd_bf16', M, N, K, x.data_ptr(), K, w.data_ptr(), b.data_ptr(), o['y'], N, 1, RELU, ws.data_ptr(), WS_BYTES, st)
+    c.call('b200rl_linear_dgrad_bf16', M, N, K, dy.data_ptr(), N, w.data_ptr(), o['dx'], K, 1, x.data_ptr(), 1, RELU, ws.data_ptr(),
+           WS_BYTES, st)
+    c.call('b200rl_linear_wgrad_bf16', M, N, K, dy.data_ptr(), N, x.data_ptr(), K, o['dw'], o['db'], ws.data_ptr(), WS_BYTES, st)
+    c.call('b200rl_conv2d_dgrad_bf16', dy3.data_ptr(), w3.data_ptr(), o['dx3'], 1, g3, m3.data_ptr(), 1, RELU, st)
+    c.call('b200rl_conv2d_wgrad_bf16', x2.data_ptr(), 0, o['dx3'], o['dw2'], o['db2'], g2, ws.data_ptr(), WS_BYTES, st)
+
+  def snapshot():
+    torch.cuda.synchronize()
+    res = {k: v.clone() for k, v in outs.items()}
+    for v in outs.values():
+      v.view(torch.uint8).fill_(SENT)
+    return res
+
+  def same(a, bb, what):
+    for k in a:
+      assert torch.equal(a[k].view(torch.uint8), bb[k].view(torch.uint8)), f'{k} differs: {what}'
+
+  chain()
+  ref = snapshot()
+  try:
+    lib.b200rl_debug_set_pdl(0)
+    chain()
+    same(ref, snapshot(), 'PDL off vs on')
+  finally:
+    lib.b200rl_debug_set_pdl(-1)
+  graph = torch.cuda.CUDAGraph()
+  with torch.cuda.graph(graph):
+    chain()
+  for i in range(2):
+    graph.replay()
+    same(ref, snapshot(), f'graph replay {i} vs eager')
+  del graph
+  # two split-K GEMMs concurrently on two streams
+  shapes = ((256, 1024, 7744), (512, 1024, 7744))
+  ins = [(dev(bf(rng.standard_normal((m, k))), _bf16()), dev(bf(rng.standard_normal((n, k)) / 88.), _bf16())) for m, n, k in shapes]
+  ys = [torch.empty(m, n, device='cuda') for m, n, _ in shapes]
+  wss = [torch.empty(WS_BYTES, dtype=torch.uint8, device='cuda') for _ in shapes]
+
+  def gemm(i, st):
+    (m, n, k), (xi, wi) = shapes[i], ins[i]
+    c.call('b200rl_linear_fwd_bf16', m, n, k, xi.data_ptr(), k, wi.data_ptr(), None, ys[i].data_ptr(), n, 0, NONE, wss[i].data_ptr(),
+           WS_BYTES, st)
+
+  for i in range(2):
+    gemm(i, stream())
+  torch.cuda.synchronize()
+  serial = [y.clone() for y in ys]
+  for y in ys:
+    y.fill_(float('nan'))
+  streams = [torch.cuda.Stream() for _ in shapes]
+  for i, s in enumerate(streams):
+    s.wait_stream(torch.cuda.current_stream())
+    gemm(i, s.cuda_stream)
+  torch.cuda.synchronize()
+  for i in range(2):
+    assert torch.equal(ys[i], serial[i]), f'GEMM {shapes[i]} differs when run beside another split-K GEMM'

@@ -605,13 +605,16 @@ def _scale_err(got, want):
   return float(np.abs(got - want).max() / max(np.abs(want).max(), 1e-30))
 
 
-@pytest.mark.parametrize('precision', [0, 1, 2])
-def test_dqn_learner_c2_shape_parity(precision):
+@pytest.mark.parametrize('precision,use_cuda_graph', [pytest.param(0, False, id='0'), pytest.param(1, False, id='1'),
+                                                    pytest.param(2, False, id='2'), pytest.param(2, True, id='bf16-graph')])
+def test_dqn_learner_c2_shape_parity(precision, use_cuda_graph):
   """BASELINE configs[1] shapes (84x84x4 uint8, A=18, B=256, n=3) through the WHOLE learner in both precisions:
   K1 indices bit-exact, then TD errors, loss, importance weights, new priorities (the quantities north_star names) and
   the parameter gradients against the oracle, for 3 updates on injected uniform draws.  Before every update the oracle
   adopts the device learner's parameters and Adam moments, so each update is compared from an identical state
-  (`acme/agents/tf/dqn/learning.py:121-154`)."""
+  (`acme/agents/tf/dqn/learning.py:121-154`).  'bf16-graph' is the benchmarked configuration: the step captured in one
+  CUDA graph (programmatic dependent launch, side streams), 4 updates of which the last two replay the graph; there the
+  draws cannot be injected, so the oracle samples with the learner's own device Philox stream (dataset seed, counter)."""
   import json
   import os
   import torch
@@ -642,18 +645,24 @@ def test_dqn_learner_c2_shape_parity(precision):
   onet, otgt = onets.DQNAtariNetwork(A), onets.DQNAtariNetwork(A)
   ds = replay.ReplayDataset(table, B, seed=7)
   learner = dqn.DQNLearner(net, tgt, 0.99, 0.2, 1e-3, target_update_period=100, dataset=ds,
-                           replay_client=replay.Client(server), logger=loggers.NoOpLogger(), use_cuda_graph=False)
+                           replay_client=replay.Client(server), logger=loggers.NoOpLogger(), use_cuda_graph=use_cuda_graph)
   ol = olearner.DQNOracleLearner(onet, otgt, 0.99, 0.2, 1e-3, 100)
   measured = []
-  for step in range(3):
+  counter = torch.zeros(1, dtype=torch.int64, device='cuda')
+  u_dev = torch.empty(B, device='cuda')
+  for step in range(4 if use_cuda_graph else 3):
     onet.load(net.variables())
     otgt.load(tgt.variables())
     ol.opt.m, ol.opt.v, ol.opt.t = _export_flat(net, learner._m), _export_flat(net, learner._v), step
     ol.num_steps = step
-    u = rng.random(B, dtype=np.float32)
+    if use_cuda_graph:   # the uniforms the learner is about to draw (device Philox keyed by (seed, call counter))
+      _capi.call('b200rl_uniform', u_dev.data_ptr(), B, 7, counter.data_ptr(), step, _capi.current_stream())
+      u = u_dev.cpu().numpy()
+    else:
+      u = rng.random(B, dtype=np.float32)
     keys, pos, prob = oracle.sample(u, True)
     ref = ol.step(*oracle.gather(pos), prob)
-    learner.step(uniforms=torch.as_tensor(u).cuda())
+    learner.step(uniforms=None if use_cuda_graph else torch.as_tensor(u).cuda())
     torch.cuda.synchronize()
     np.testing.assert_array_equal(ds.idx.cpu().numpy(), pos)                       # sampled indices: bit-exact
     np.testing.assert_array_equal(ds.keys.cpu().numpy().view(np.uint64), keys)
@@ -681,7 +690,7 @@ def test_dqn_learner_c2_shape_parity(precision):
   out = os.environ.get('B200RL_PARITY_DIR')
   if out:
     os.makedirs(out, exist_ok=True)
-    mode = {0: 'fp32', 1: 'tf32', 2: 'bf16'}[precision]
+    mode = {0: 'fp32', 1: 'tf32', 2: 'bf16'}[precision] + ('_graph' if use_cuda_graph else '')
     with open(os.path.join(out, f'parity_c2_{mode}.json'), 'w') as f:
       json.dump(dict(mode=mode, B=B, A=A, tolerances=tolv, measured=measured), f, indent=1)
   server.stop()
