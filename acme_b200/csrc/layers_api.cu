@@ -97,6 +97,13 @@ static int check_geom(const b200rl_conv_geom* g) {
   B200RL_REQUIRE((int64_t)g->B * g->H * g->W < (1ll << 31) && (int64_t)g->B * g->OH * g->OW < (1ll << 31), "too many pixels");
   return B200RL_OK;
 }
+// The convolution loaders of every precision read an fp32 activation / gradient / filter as float4 (im2col of x; dy and
+// w of the data gradient) and a uint8 frame as one 4-byte pixel (C % 4 == 0), with no alignment test on the device.
+// A misaligned pointer is therefore rejected here, before anything is launched.
+static int check_conv_ptr(const void* p, int u8, const char* what) {
+  B200RL_REQUIRE(((uintptr_t)p & (u8 ? 3 : 15)) == 0, "%s must be %d-byte aligned", what, u8 ? 4 : 16);
+  return B200RL_OK;
+}
 
 #define PRECISION_SWITCH(simt_call, tc_call)                                                   \
   if (precision == 0) return simt_call;                                                        \
@@ -108,6 +115,7 @@ extern "C" int b200rl_conv2d_fwd(const void* x, int x_u8, const float* w, const 
                                  const b200rl_conv_geom* g, int act, int precision, void* ws, int64_t wsb, void* stream) {
   B200RL_REQUIRE(x && w && y, "null argument");
   if (int rc = check_geom(g)) return rc;
+  if (int rc = check_conv_ptr(x, x_u8 == 1, "conv input x")) return rc;
   if (x_u8 == 2) {   // a row image from b200rl_conv2d_rows_from_u8
     B200RL_REQUIRE(precision == 1, "row images are a tensor-core-mode input");
     int rc = tma_conv_fwd_rows((const float*)x, w, bias, y, *g, act, ws, wsb, as_stream(stream));
@@ -126,6 +134,7 @@ extern "C" int b200rl_conv2d_wgrad(const void* x, int x_u8, const float* dy, flo
                                    const b200rl_conv_geom* g, int precision, void* ws, int64_t wsb, void* stream) {
   B200RL_REQUIRE(x && dy && dw, "null argument");
   if (int rc = check_geom(g)) return rc;
+  if (int rc = check_conv_ptr(x, x_u8 == 1, "conv input x")) return rc;
   if (x_u8 == 2) {
     B200RL_REQUIRE(precision == 1, "row images are a tensor-core-mode input");
     int rc = tma_conv_wgrad_rows((const float*)x, dy, dw, db, *g, ws, wsb, as_stream(stream));
@@ -148,6 +157,7 @@ extern "C" int b200rl_conv2d_rows_from_u8(const void* x_u8, const b200rl_conv_ge
                                           void* stream) {
   B200RL_REQUIRE(x_u8 && rows, "null argument");
   if (int rc = check_geom(g)) return rc;
+  if (int rc = check_conv_ptr(x_u8, 1, "uint8 frames")) return rc;
   int rc = tma_rows_from_u8((const uint8_t*)x_u8, *g, rows, rows_bytes, as_stream(stream));
   B200RL_REQUIRE(rc != 1, "geometry not eligible for a row image, buffer too small or not 128-byte aligned");
   return rc;
@@ -157,6 +167,8 @@ extern "C" int b200rl_conv2d_dgrad(const float* dy, const float* w, float* dx, c
                                    const float* mask_y, int mask_act, int precision, void* ws, int64_t wsb, void* stream) {
   B200RL_REQUIRE(dy && w && dx, "null argument");
   if (int rc = check_geom(g)) return rc;
+  if (int rc = check_conv_ptr(dy, 0, "conv dgrad dy")) return rc;
+  if (int rc = check_conv_ptr(w, 0, "conv dgrad w")) return rc;
   if (precision == 1 && g_use_tma) {
     int rc = tma_conv_dgrad(dy, w, dx, *g, mask_y, mask_act, ws, wsb, as_stream(stream));
     if (rc != 1) return rc;

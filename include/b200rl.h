@@ -257,6 +257,9 @@ int b200rl_learner_tail(int64_t n_bytes_a, void* dst_a, const void* src_a, int64
  * ws / ws_bytes: caller-owned scratch (split-K partial sums, column-sum partials, and for a first-layer convolution
  * on uint8 frames in precision 1 the zero-padded fp32 row image, B * (H + pad) * (W + pad) * C * 4 bytes); one workspace
  * per stream -- calls on different streams must not share it.
+ * Alignment (every precision): the convolution entry points read fp32 x (forward, weight gradient, row image) and the
+ * data gradient's dy and w as 16-byte vectors, and uint8 frames as 4-byte pixels; a pointer that is not 16-byte
+ * (fp32) / 4-byte (uint8) aligned returns B200RL_EINVAL without launching.  Dense layers take any 4-byte alignment.
  * ------------------------------------------------------------------------------------------ */
 typedef struct b200rl_conv_geom {
   int32_t B, H, W, C;       /* input NHWC                         */

@@ -218,96 +218,23 @@ def test_copy_if_period_and_step_counter():
 
 
 # ------------------------------------------------------------------------------------ K6 layers
-@pytest.mark.parametrize('precision', [0, 1])
-@pytest.mark.parametrize('H,C,k,s,Cout,u8,B', [(84, 4, 8, 4, 32, True, 5), (21, 32, 4, 2, 64, False, 5),
-                                               (11, 64, 3, 1, 64, False, 5), (12, 8, 3, 2, 16, False, 5),
-                                               (20, 32, 5, 2, 32, False, 13), (17, 64, 3, 2, 96, False, 11)])
-def test_conv_fwd_wgrad_dgrad_vs_torch_cpu(H, C, k, s, Cout, u8, B, precision):
-  import torch
-  from acme_b200 import _capi, networks
-  from oracle import nets as onets
-  rng = np.random.default_rng(H + C)
-  OH, pad = networks.tf_same_pad(H, k, s)
-  g = _capi.ConvGeom(B=B, H=H, W=H, C=C, kh=k, kw=k, stride=s, pad_top=pad, pad_left=pad, OH=OH, OW=OH, Cout=Cout)
-  x_raw = rng.integers(0, 256, (B, H, H, C), dtype=np.uint8) if u8 else rng.standard_normal((B, H, H, C)).astype(np.float32)
-  x_f = (x_raw.astype(np.float32) / np.float32(255)) if u8 else x_raw
-  w_hwio = (rng.standard_normal((k, k, C, Cout)) / np.sqrt(k * k * C)).astype(np.float32)
-  bias = rng.standard_normal(Cout).astype(np.float32)
-  xt = torch.tensor(x_f, requires_grad=True)
-  wt = torch.tensor(w_hwio, requires_grad=True)
-  bt = torch.tensor(bias, requires_grad=True)
-  y_ref = torch.relu(onets._conv_same(xt, wt, bt, s))
-  dy_post = rng.standard_normal(tuple(y_ref.shape)).astype(np.float32)
-  y_ref.backward(torch.tensor(dy_post))
-  ws = empty(64 << 20, dtype=torch.uint8)
-  w_ohwi = dev(w_hwio.transpose(3, 0, 1, 2))
-  y = empty(B, OH, OH, Cout)
-  xd = dev(x_raw)
-  _capi.call('b200rl_conv2d_fwd', xd.data_ptr(), int(u8), w_ohwi.data_ptr(), dev(bias).data_ptr(), y.data_ptr(), g,
-             _capi.ACT_RELU, precision, ws.data_ptr(), ws.numel(), _capi.current_stream())
-  close(y.cpu().numpy(), y_ref.detach().numpy(), name='conv fwd', **tol(precision))
-  dy_pre = dev(dy_post * (y_ref.detach().numpy() > 0))
-  dw, db = empty(Cout, k, k, C), empty(Cout)
-  _capi.call('b200rl_conv2d_wgrad', xd.data_ptr(), int(u8), dy_pre.data_ptr(), dw.data_ptr(), db.data_ptr(), g, precision,
-             ws.data_ptr(), ws.numel(), _capi.current_stream())
-  close(dw.cpu().numpy().transpose(1, 2, 3, 0), wt.grad.numpy(), name='conv wgrad', **tol(precision, atol_scale=2e-6))
-  close(db.cpu().numpy(), bt.grad.numpy(), atol_scale=2e-6, name='conv bias grad')
-  if u8 and precision == 1:
-    # the same frames through a shared row image (x_u8 = 2): identical kernels, identical bits
-    import ctypes
-    nbytes = int(_capi.load().b200rl_conv2d_rows_bytes(ctypes.byref(g)))
-    assert nbytes > 0
-    rows = empty(nbytes, dtype=torch.uint8)
-    _capi.call('b200rl_conv2d_rows_from_u8', xd.data_ptr(), g, rows.data_ptr(), nbytes, _capi.current_stream())
-    y2, dw2, db2 = empty(B, OH, OH, Cout), empty(Cout, k, k, C), empty(Cout)
-    _capi.call('b200rl_conv2d_fwd', rows.data_ptr(), 2, w_ohwi.data_ptr(), dev(bias).data_ptr(), y2.data_ptr(), g,
-               _capi.ACT_RELU, precision, ws.data_ptr(), ws.numel(), _capi.current_stream())
-    _capi.call('b200rl_conv2d_wgrad', rows.data_ptr(), 2, dy_pre.data_ptr(), dw2.data_ptr(), db2.data_ptr(), g, precision,
-               ws.data_ptr(), ws.numel(), _capi.current_stream())
-    assert torch.equal(y2, y) and torch.equal(dw2, dw) and torch.equal(db2, db)
-  if C % 4 == 0 and not u8:
-    dx = empty(B, H, H, C)
-    _capi.call('b200rl_conv2d_dgrad', dy_pre.data_ptr(), w_ohwi.data_ptr(), dx.data_ptr(), g, None, 0, precision,
-               ws.data_ptr(), ws.numel(), _capi.current_stream())
-    close(dx.cpu().numpy(), xt.grad.numpy(), name='conv dgrad', **tol(precision, atol_scale=2e-6))
-    # with the producer layer's ReLU derivative fused (mask = that layer's output)
-    prev = rng.standard_normal((B, H, H, C)).astype(np.float32)
-    _capi.call('b200rl_conv2d_dgrad', dy_pre.data_ptr(), w_ohwi.data_ptr(), dx.data_ptr(), g, dev(prev).data_ptr(),
-               _capi.ACT_RELU, precision, ws.data_ptr(), ws.numel(), _capi.current_stream())
-    close(dx.cpu().numpy(), xt.grad.numpy() * (prev > 0), name='conv dgrad masked', **tol(precision, atol_scale=2e-6))
-
-
-@pytest.mark.parametrize('precision', [0, 1])
-@pytest.mark.parametrize('M,N,K', [(256, 1024, 7744), (10, 50, 50), (256, 18, 512), (256, 1, 512), (33, 51, 256), (300, 200, 136)])
-def test_linear_fwd_dgrad_wgrad(M, N, K, precision):
-  import torch
+# single layers against an fp64 reference: test_gpu_fp32_layers.py (precisions 0 and 1), test_gpu_bf16_layers.py
+@pytest.mark.parametrize('act', [0, 1, 2, 3])
+def test_act_bwd_matches_fp32_derivative(act):
+  """b200rl_act_bwd: dy *= act'(y) from the activation's output, bit for bit the fp32 expression (learner_math.cu is built
+  without multiply-add contraction): ReLU y > 0, ELU y > 0 ? 1 : y + 1, tanh 1 - y * y; ACT_NONE leaves dy untouched."""
   from acme_b200 import _capi
-  rng = np.random.default_rng(M + N)
-  x = rng.standard_normal((M, K)).astype(np.float32)
-  w = (rng.standard_normal((N, K)) / np.sqrt(K)).astype(np.float32)
-  b = rng.standard_normal(N).astype(np.float32)
-  xt, wt, bt = torch.tensor(x, requires_grad=True), torch.tensor(w, requires_grad=True), torch.tensor(b, requires_grad=True)
-  y_ref = torch.nn.functional.elu(xt @ wt.T + bt)
-  dy_post = rng.standard_normal((M, N)).astype(np.float32)
-  y_ref.backward(torch.tensor(dy_post))
-  ws = empty(64 << 20, dtype=torch.uint8)
-  y = empty(M, N)
-  st = _capi.current_stream()
-  _capi.call('b200rl_linear_fwd', M, N, K, dev(x).data_ptr(), K, dev(w).data_ptr(), dev(b).data_ptr(), y.data_ptr(), N,
-             _capi.ACT_ELU, precision, ws.data_ptr(), ws.numel(), st)
-  close(y.cpu().numpy(), y_ref.detach().numpy(), name='linear fwd', **tol(precision))
-  if precision == 1:   # feed the exact fp32 activation to the backward checks
-    y.copy_(dev(y_ref.detach().numpy()))
-  dy = dev(dy_post)
-  _capi.call('b200rl_act_bwd', M * N, dy.data_ptr(), y.data_ptr(), _capi.ACT_ELU, st)
-  dx, dw, db = empty(M, K), empty(N, K), empty(N)
-  _capi.call('b200rl_linear_dgrad', M, N, K, dy.data_ptr(), N, dev(w).data_ptr(), dx.data_ptr(), K, None, 0, precision,
-             ws.data_ptr(), ws.numel(), st)
-  _capi.call('b200rl_linear_wgrad', M, N, K, dy.data_ptr(), N, dev(x).data_ptr(), K, dw.data_ptr(), db.data_ptr(), precision,
-             ws.data_ptr(), ws.numel(), st)
-  close(dx.cpu().numpy(), xt.grad.numpy(), name='linear dgrad', **tol(precision, atol_scale=2e-6))
-  close(dw.cpu().numpy(), wt.grad.numpy(), name='linear wgrad', **tol(precision, atol_scale=2e-6))
-  close(db.cpu().numpy(), bt.grad.numpy(), atol_scale=2e-6, name='linear bias grad')
+  rng = np.random.default_rng(act)
+  n = 100_003
+  z = rng.standard_normal(n).astype(np.float32)
+  y = {0: z, 1: np.maximum(z, 0), 2: np.where(z > 0, z, np.expm1(np.minimum(z, 0))), 3: np.tanh(z)}[act].astype(np.float32)
+  y[:4] = np.array([0., -0., 1e-30, -1.], np.float32)
+  dy = rng.standard_normal(n).astype(np.float32)
+  one = np.float32(1)
+  g = {0: np.ones_like(y), 1: (y > 0).astype(np.float32), 2: np.where(y > 0, one, y + one), 3: one - y * y}[act]
+  d, yd = dev(dy), dev(y)
+  _capi.call('b200rl_act_bwd', n, d.data_ptr(), yd.data_ptr(), act, _capi.current_stream())
+  np.testing.assert_array_equal(d.cpu().numpy(), (dy * g.astype(np.float32)).astype(np.float32))
 
 
 def test_layernorm_tanh_and_small_ops():
