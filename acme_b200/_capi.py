@@ -122,6 +122,9 @@ PROTOTYPES = {
                                          c_i64, c_vp]),
     'b200rl_colsum_bf16': (c_int, [c_i32, c_i32, c_vp, c_i32, c_vp, c_vp, c_i64, c_vp]),
     'b200rl_linear_wgrad_bf16': (c_int, [c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    'b200rl_layernorm_tanh_fwd_bf16': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'b200rl_dense_head_bwd_bf16': (c_int, [c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_i32, c_vp, c_int, c_vp,
+                                           c_vp, c_vp, c_i64, c_vp]),
     'b200rl_layernorm_tanh_fwd': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_layernorm_tanh_bwd': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_tanh_to_spec_fwd': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]),
@@ -159,7 +162,7 @@ TD_IS_WEIGHTS_F32 = 1
 #   0  fp32 FFMA: the 1e-5 parity mode
 #   1  tcgen05 with fp32 tensors: tf32 operands fetched by TMA where eligible, bf16 operands converted on the fly otherwise
 #   2  bf16 dataflow: activations, weight shadows and back-propagated gradients in bf16 (kind::f16), fp32 master weights /
-#      accumulation / optimizer; networks that do not implement it treat 2 as 1
+#      accumulation / optimizer (DQNAtariNetwork and the LayerNormMLP networks)
 PRECISION_FP32, PRECISION_TC, PRECISION_BF16FLOW = 0, 1, 2
 PRECISION_BF16 = PRECISION_TC      # historical name of mode 1
 

@@ -13,6 +13,9 @@ namespace b200rl {
 
 void set_error(const char* fmt, ...);
 void count_launch();
+// gemm_simt.cu: index in [0, 64) of `s` for the per-stream last-CTA tickets of single-launch reductions (-1 once 64
+// streams have been seen)
+int ticket_for(cudaStream_t s);
 
 #define B200RL_CUDA_OK(expr)                                                              \
   do {                                                                                    \

@@ -451,7 +451,7 @@ colsum_vec_kernel(int M, int N, const void* __restrict__ x, int ld, int rows_per
 
 // kernels on one stream never overlap, so a ticket per stream is race-free (also inside a captured graph, whose
 // nodes keep the capture-time stream order)
-static int ticket_for(cudaStream_t s) {
+int ticket_for(cudaStream_t s) {
   static std::mutex mu;
   static std::vector<cudaStream_t> seen;
   std::lock_guard<std::mutex> lk(mu);

@@ -912,11 +912,140 @@ __global__ void duelling_head_bwd_finish_kernel(int A, int H, int segs, const fl
   else { if (k < H) dwa[(size_t)(r - 1) * H + k] = t; else dba[r - 1] = t; }
 }
 
-// snt.LayerNorm(axis=slice(1,None), scale, offset) + tanh (acme/tf/networks/continuous.py:55-58); CTA per row
+// Backward of a dense head with N <= 64 outputs in the bf16 dataflow (the C51, scalar-critic and policy heads of
+// LayerNormMLP): the bf16 GEMMs need N >= 64 (data gradient) and N % 64 == 0 (weight gradient).  One launch computes
+//   dx[M,K] = (dy[M,N] @ w[N,K]) * act'(mask)  as bf16,   dw[N,K] = dy^T @ x,   db[N] = colsum(dy)  in fp32.
+// CTA (kb, mb) owns columns [64 kb, 64 kb + 64) and rows [mb * rows_per_cta, ...), walked in chunks of 32 rows staged in
+// shared memory as fp32 (bf16 -> fp32 is exact); every sum is a chain of fmaf in ascending n or m.  With one row slice
+// the CTA writes dw / db directly.  With several, each writes a partial slab and the CTA of column block kb that finishes
+// last (a per-stream, per-column-block ticket reset on the way out, so the kernel is CUDA-graph safe) adds the slabs in
+// slice order: the order of every addition is fixed by indices, never by arrival.
+constexpr int kHbRows = 32, kHbCols = 64, kHbMaxColBlocks = 32;
+__device__ unsigned int g_head_tickets[64 * kHbMaxColBlocks];
+
+__device__ __forceinline__ void bf16x8_to_f32(uint4 u, float* v) {
+  const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[j]));
+    v[2 * j] = f.x;
+    v[2 * j + 1] = f.y;
+  }
+}
+
+__global__ void __launch_bounds__(256)
+dense_head_bwd_bf16_kernel(int M, int N, int K, const float* __restrict__ dy, int lddy, const __nv_bfloat16* __restrict__ x,
+                           int ldx, const __nv_bfloat16* __restrict__ w, __nv_bfloat16* __restrict__ dx, int lddx,
+                           const __nv_bfloat16* __restrict__ mask, int mask_act, float* __restrict__ dw,
+                           float* __restrict__ db, int rows_per_cta, float* __restrict__ partial, int ticket) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ float w_s[64][kHbCols];
+  __shared__ float dy_s[kHbRows][64];
+  __shared__ float x_s[kHbRows][kHbCols];
+  __shared__ bool last;
+  const int kb = blockIdx.x, mb = blockIdx.y;
+  const int k0 = kb * kHbCols, kc = min(kHbCols, K - k0);          // kc % 8 == 0
+  const int m0 = mb * rows_per_cta, m1 = min(M, m0 + rows_per_cta);
+  const int t = threadIdx.x, col = t & (kHbCols - 1), rg = t >> 6;  // rg: row group 0..3
+  const bool grads = dw || db;
+  for (int i = t; i < 64 * (kHbCols / 8); i += 256) {
+    const int n = i / (kHbCols / 8), c8 = (i % (kHbCols / 8)) * 8;
+    float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    if (n < N && c8 < kc) bf16x8_to_f32(__ldg(reinterpret_cast<const uint4*>(w + (size_t)n * K + k0 + c8)), v);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) w_s[n][c8 + j] = v[j];
+  }
+  float acc_w[16], acc_b = 0.f;
+#pragma unroll
+  for (int j = 0; j < 16; ++j) acc_w[j] = 0.f;
+  for (int r0 = m0; r0 < m1; r0 += kHbRows) {
+    const int rows = min(kHbRows, m1 - r0);
+    __syncthreads();   // the previous chunk has been consumed
+    for (int i = t; i < kHbRows * 64; i += 256) {
+      const int r = i >> 6, n = i & 63;
+      dy_s[r][n] = (r < rows && n < N) ? dy[(size_t)(r0 + r) * lddy + n] : 0.f;
+    }
+    if (dw) {
+      const int r = t / (kHbCols / 8), c8 = (t % (kHbCols / 8)) * 8;   // 256 threads = 32 rows x 8 vectors
+      float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+      if (r < rows && c8 < kc) bf16x8_to_f32(__ldg(reinterpret_cast<const uint4*>(x + (size_t)(r0 + r) * ldx + k0 + c8)), v);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) x_s[r][c8 + j] = v[j];
+    }
+    __syncthreads();
+    if (col < kc) {
+      float a[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+      for (int n = 0; n < N; ++n) {
+        const float wv = w_s[n][col];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) a[j] = fmaf(dy_s[rg + 4 * j][n], wv, a[j]);
+      }
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const int r = rg + 4 * j;
+        if (r < rows) {
+          const size_t o = (size_t)(r0 + r) * lddx + k0 + col;
+          float v = a[j];
+          if (mask) v = v * act_grad_from_output(__bfloat162float(mask[o]), mask_act);
+          dx[o] = __float2bfloat16_rn(v);
+        }
+      }
+      if (dw)
+        for (int r = 0; r < rows; ++r) {
+          const float xv = x_s[r][col];
+#pragma unroll
+          for (int j = 0; j < 16; ++j) acc_w[j] = fmaf(dy_s[r][rg + 4 * j], xv, acc_w[j]);
+        }
+    }
+    if (db && kb == 0 && t < N)
+      for (int r = 0; r < rows; ++r) acc_b = acc_b + dy_s[r][t];
+  }
+  if (!grads) return;
+  if (gridDim.y == 1) {
+    if (dw && col < kc)
+#pragma unroll
+      for (int j = 0; j < 16; ++j)
+        if (rg + 4 * j < N) dw[(size_t)(rg + 4 * j) * K + k0 + col] = acc_w[j];
+    if (db && kb == 0 && t < N) db[t] = acc_b;
+    return;
+  }
+  // partial layout: [kb][mb][64][64] dw slabs, then [mb][64] bias sums
+  float* slab = partial + ((size_t)kb * gridDim.y + mb) * (64 * kHbCols);
+  float* bpart = partial + (size_t)gridDim.x * gridDim.y * (64 * kHbCols);
+  if (dw)
+#pragma unroll
+    for (int j = 0; j < 16; ++j) slab[(rg + 4 * j) * kHbCols + col] = acc_w[j];
+  if (db && kb == 0 && t < 64) bpart[mb * 64 + t] = acc_b;
+  __threadfence();
+  __syncthreads();
+  unsigned int* tk = &g_head_tickets[ticket * kHbMaxColBlocks + kb];
+  if (t == 0) last = atomicAdd(tk, 1u) == gridDim.y - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  if (dw && col < kc)
+    for (int j = 0; j < 16; ++j) {
+      const int n = rg + 4 * j;
+      if (n >= N) break;
+      float s = 0.f;
+      for (int q = 0; q < (int)gridDim.y; ++q) s = s + __ldcg(partial + ((size_t)kb * gridDim.y + q) * (64 * kHbCols) + n * kHbCols + col);
+      dw[(size_t)n * K + k0 + col] = s;
+    }
+  if (db && kb == 0 && t < N) {
+    float s = 0.f;
+    for (int q = 0; q < (int)gridDim.y; ++q) s = s + __ldcg(bpart + q * 64 + t);
+    db[t] = s;
+  }
+  if (t == 0) *tk = 0;
+}
+
+// snt.LayerNorm(axis=slice(1,None), scale, offset) + tanh (acme/tf/networks/continuous.py:55-58); CTA per row.
+// y_bf16 (nullable): also store RN-bf16(y), the operand of the next layer in the bf16 dataflow.
 __global__ void __launch_bounds__(256)
 layernorm_tanh_fwd_kernel(int N, const float* __restrict__ x, const float* __restrict__ scale,
                           const float* __restrict__ offset, float eps, float* __restrict__ y,
-                          float* __restrict__ xhat, float* __restrict__ rstd) {
+                          float* __restrict__ xhat, float* __restrict__ rstd, __nv_bfloat16* __restrict__ y_bf16) {
   pdl_launch_dependents();
   pdl_wait();
   __shared__ float scratch[32];
@@ -932,7 +1061,9 @@ layernorm_tanh_fwd_kernel(int N, const float* __restrict__ x, const float* __res
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     float xh = (xr[i] - mean) * rs;
     xhat[(size_t)b * N + i] = xh;
-    y[(size_t)b * N + i] = tanhf(xh * scale[i] + offset[i]);
+    const float yv = tanhf(xh * scale[i] + offset[i]);
+    y[(size_t)b * N + i] = yv;
+    if (y_bf16) y_bf16[(size_t)b * N + i] = __float2bfloat16_rn(yv);
   }
   if (threadIdx.x == 0) rstd[b] = rs;
 }
@@ -1427,7 +1558,47 @@ extern "C" int b200rl_duelling_head_wgrad(int32_t B, int32_t A, int32_t H, const
 extern "C" int b200rl_layernorm_tanh_fwd(int32_t B, int32_t N, const float* x, const float* scale, const float* offset,
                                          float eps, float* y, float* xhat, float* rstd, void* stream) {
   B200RL_REQUIRE(x && scale && offset && y && xhat && rstd && B >= 1 && N >= 1, "bad argument");
-  B200RL_CUDA_OK(launch_pdl_small(layernorm_tanh_fwd_kernel, dim3(B), dim3(256), 0, as_stream(stream), N, x, scale, offset, eps, y, xhat, rstd));
+  B200RL_CUDA_OK(launch_pdl_small(layernorm_tanh_fwd_kernel, dim3(B), dim3(256), 0, as_stream(stream), N, x, scale, offset, eps, y, xhat, rstd,
+                                  (__nv_bfloat16*)nullptr));
+  B200RL_LAUNCH_OK();
+  return B200RL_OK;
+}
+extern "C" int b200rl_layernorm_tanh_fwd_bf16(int32_t B, int32_t N, const float* x, const float* scale, const float* offset,
+                                              float eps, float* y, void* y_bf16, float* xhat, float* rstd, void* stream) {
+  B200RL_REQUIRE(x && scale && offset && y && y_bf16 && xhat && rstd && B >= 1 && N >= 1, "bad argument");
+  B200RL_CUDA_OK(launch_pdl_small(layernorm_tanh_fwd_kernel, dim3(B), dim3(256), 0, as_stream(stream), N, x, scale, offset, eps, y, xhat, rstd,
+                                  (__nv_bfloat16*)y_bf16));
+  B200RL_LAUNCH_OK();
+  return B200RL_OK;
+}
+
+extern "C" int b200rl_dense_head_bwd_bf16(int32_t M, int32_t N, int32_t K, const float* dy, int32_t lddy, const void* x_bf16,
+                                          int32_t ldx, const void* w_bf16, void* dx_bf16, int32_t lddx, const void* mask_bf16,
+                                          int mask_act, float* dw, float* db, void* ws, int64_t ws_bytes, void* stream) {
+  B200RL_REQUIRE(dy && w_bf16 && dx_bf16 && (x_bf16 || !dw), "null argument");
+  B200RL_REQUIRE(M >= 1 && N >= 1 && N <= 64 && K >= 8 && K % 8 == 0 && lddy >= N && lddx >= K,
+                 "dense head backward: N = %d must be in [1, 64] and K = %d a multiple of 8", N, K);
+  B200RL_REQUIRE(lddx % 8 == 0 && (!dw || (ldx >= K && ldx % 8 == 0)) &&
+                     (((uintptr_t)w_bf16 | (uintptr_t)dx_bf16 | (uintptr_t)mask_bf16 | (uintptr_t)(dw ? x_bf16 : nullptr)) & 15) == 0,
+                 "dense head backward: bf16 rows must be 16-byte aligned");
+  cudaStream_t st = as_stream(stream);
+  const int kblocks = ceil_div(K, kHbCols);
+  // row slices: enough CTAs for the latency-bound batch sizes, at most 32 partial slabs per column block
+  int slices = std::min(ceil_div(M, kHbRows), (dw || db) ? 32 : 4096);
+  int ticket = -1;
+  if ((dw || db) && slices > 1) {
+    const int64_t per = ((int64_t)kblocks * 64 * kHbCols + 64) * 4;
+    if (kblocks <= kHbMaxColBlocks && ws) slices = (int)std::min<int64_t>(slices, ws_bytes / per);
+    else slices = 1;
+    if (slices > 1) ticket = ticket_for(st);
+    if (ticket < 0) slices = 1;
+  }
+  slices = std::max(slices, 1);
+  const int rpc = ceil_div(M, slices);
+  slices = ceil_div(M, rpc);
+  B200RL_CUDA_OK(launch_pdl_small(dense_head_bwd_bf16_kernel, dim3(kblocks, slices), dim3(256), 0, st, M, N, K, dy, lddy,
+                                  (const __nv_bfloat16*)x_bf16, ldx, (const __nv_bfloat16*)w_bf16, (__nv_bfloat16*)dx_bf16, lddx,
+                                  (const __nv_bfloat16*)mask_bf16, mask_act, dw, db, rpc, (float*)ws, ticket < 0 ? 0 : ticket));
   B200RL_LAUNCH_OK();
   return B200RL_OK;
 }

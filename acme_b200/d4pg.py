@@ -106,6 +106,9 @@ class D4PGLearner(core.Learner, core.Saveable):
     for src, dst in ((P, TP), (C, TC)):
       _capi.call('b200rl_copy_if_period', src.params.size * 4, _capi.ptr(dst.params.flat), _capi.ptr(src.params.flat),
                  _capi.ptr(self._num_steps), self._period, 0, st)
+      if dst.params.shadow is not None:   # bf16 dataflow: the target's weight operands follow its parameters
+        _capi.call('b200rl_copy_if_period', src.params.size * 2, _capi.ptr(dst.params.shadow), _capi.ptr(src.params.shadow),
+                   _capi.ptr(self._num_steps), self._period, 0, st)
     ds.sample_raw(uniforms)
     o0, a0, o1 = self._views()
     # The step is ~100 small launch-bound kernels; its three chains are independent until the critic loss, so they run
@@ -184,7 +187,7 @@ class D4PGLearner(core.Learner, core.Saveable):
                    _capi.ptr(scale), _capi.ptr(norm), st)
         gs = _capi.ptr(scale)
       _capi.call('b200rl_adam', net.params.size, _capi.ptr(net.params.flat), _capi.ptr(net.params.grad), _capi.ptr(m),
-                 _capi.ptr(v), _capi.ptr(self._num_steps), lr, 0.9, 0.999, 1e-8, self._eps_mode, gs, None, st)
+                 _capi.ptr(v), _capi.ptr(self._num_steps), lr, 0.9, 0.999, 1e-8, self._eps_mode, gs, _capi.ptr(net.params.shadow), st)
 
     # the two networks' clip + Adam are independent: policy on a side stream beside the critic
     if self._concurrent:
@@ -285,6 +288,8 @@ class D4PGLearner(core.Learner, core.Saveable):
     self._pm.copy_(t(state['policy_opt'][0])); self._pv.copy_(t(state['policy_opt'][1]))
     self._cm.copy_(t(state['critic_opt'][0])); self._cv.copy_(t(state['critic_opt'][1]))
     self._num_steps.fill_(int(state['num_steps']))
+    for net in (self._policy, self._critic, self._tpolicy, self._tcritic):
+      net.params.refresh_shadow()
 
 
 class DDPGLearner(D4PGLearner):

@@ -148,6 +148,11 @@ class Network:
     self.params = ParamStore(device)
     self._ws = None
 
+  @property
+  def flow(self) -> bool:
+    """precision 2: the bf16 dataflow"""
+    return self.precision == _capi.PRECISION_BF16FLOW
+
   def _finalize(self):
     import torch
     _capi.require_device(self.device)
@@ -294,10 +299,6 @@ class DQNAtariNetwork(Network):
   # ---- buffers.  In the bf16 dataflow (precision 2) activations y1..y3 and the back-propagated gradients dh, dy1..dy3
   # are bf16; the hidden row h (consumed by the duelling head in fp32), q, value / advantage and everything the loss
   # touches stay fp32.
-  @property
-  def flow(self) -> bool:
-    return self.precision == _capi.PRECISION_BF16FLOW
-
   def make_buffers(self, B: int):
     import torch
     dev = torch.device('cuda', self.device)
@@ -721,12 +722,20 @@ class MLPQNetwork(Network):
 
 # =============================================================================== D4PG networks
 class LayerNormMLP(Network):
-  """Linear -> LayerNorm -> tanh -> [Linear -> ELU]* -> optional linear head (continuous.py:37-68)."""
+  """Linear -> LayerNorm -> tanh -> [Linear -> ELU]* -> optional linear head (continuous.py:37-68).
+
+  Precision 2 (bf16 dataflow): the first layer (K = the input width, whose bf16 rows are not 16-byte multiples) and its
+  LayerNorm stay fp32; the LayerNorm also writes a bf16 copy of y0.  The hidden ELU layers read bf16 activations and the
+  bf16 weight shadow and pass bf16 gradients back (tcgen05 kind::f16); the head's forward is a bf16 GEMM with an fp32
+  output, its backward one `b200rl_dense_head_bwd_bf16` launch.  Weight gradients, biases and the master weights are fp32.
+  """
 
   def __init__(self, input_dim: int, sizes, head_dim: int, head_name: str, head_scale: Optional[float],
                device: int, precision: int, seed: int):
     super().__init__(device, precision)
     self.in_dim, self.sizes, self.head_dim, self.head = int(input_dim), [int(s) for s in sizes], int(head_dim), head_name
+    if self.flow:
+      self._check_bf16_shapes()
     P = self.params
     d = self.in_dim
     self._export = {}
@@ -757,6 +766,21 @@ class LayerNormMLP(Network):
       P.set(f'{head_name}.w', _truncated_normal(rng, (self.head_dim, d), 1 / math.sqrt(d)))
     else:  # NearZeroInitializedLinear: VarianceScaling(scale) -> truncated normal over fan_in
       P.set(f'{head_name}.w', _truncated_normal(rng, (self.head_dim, d), math.sqrt(head_scale / d) / .87962566103423978))
+    if self.flow:
+      P.ensure_shadow()
+
+  def _check_bf16_shapes(self):
+    """The shapes the bf16 entry points accept (b200rl.h), checked before anything is allocated."""
+    s = self.sizes
+    if len(s) < 2:
+      raise ValueError(f'precision 2 needs at least two hidden layers (the head reads a bf16 ELU layer); sizes = {s}')
+    if s[0] % 64 != 0:
+      raise ValueError(f'precision 2 needs the first hidden size to be a multiple of 64 (the K of the bf16 GEMMs); sizes = {s}')
+    if any(h < 64 or h > 1024 or h & (h - 1) for h in s[1:]):
+      raise ValueError(f'precision 2 needs hidden sizes after the first to be powers of two in [64, 1024] (bf16 GEMM N and '
+                       f'the bf16 bias column sum); sizes = {s}')
+    if not 1 <= self.head_dim <= 64:
+      raise ValueError(f'precision 2 needs a head of 1 to 64 outputs (b200rl_dense_head_bwd_bf16); head_dim = {self.head_dim}')
 
   def make_buffers(self, B: int):
     import torch
@@ -764,20 +788,76 @@ class LayerNormMLP(Network):
     f = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
     h0 = self.sizes[0]
     bufs = dict(B=B, x=f(B, self.in_dim), z0=f(B, h0), y0=f(B, h0), xhat=f(B, h0), rstd=f(B), out=f(B, self.head_dim))
+    a = (lambda *shape: torch.empty(shape, dtype=torch.bfloat16, device=dev)) if self.flow else f
+    if self.flow:
+      bufs['y0_bf16'] = a(B, h0)
     for i in range(1, len(self.sizes)):
-      bufs[f'y{i}'] = f(B, self.sizes[i])
+      bufs[f'y{i}'] = a(B, self.sizes[i])
     return bufs
 
   def make_grad_buffers(self, B: int):
     import torch
     dev = torch.device('cuda', self.device)
     f = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
+    a = (lambda *shape: torch.empty(shape, dtype=torch.bfloat16, device=dev)) if self.flow else f
     g = dict(dz0=f(B, self.sizes[0]), dx=f(B, self.in_dim))
     for i in range(len(self.sizes)):
-      g[f'dy{i}'] = f(B, self.sizes[i])
+      g[f'dy{i}'] = a(B, self.sizes[i]) if i > 0 else f(B, self.sizes[i])   # dy0 feeds the fp32 LayerNorm backward
     return g
 
+  def _forward_flat_bf16(self, x_ptr: int, bufs):
+    B, P, st = bufs['B'], self.params, _capi.current_stream()
+    ws, wsb = self.ws
+    h0 = self.sizes[0]
+    _capi.call('b200rl_linear_fwd', B, h0, self.in_dim, x_ptr, self.in_dim, P.p('l0.w'), P.p('l0.b'), bufs['z0'].data_ptr(), h0,
+               ACT_NONE, _capi.PRECISION_TC, ws, wsb, st)
+    _capi.call('b200rl_layernorm_tanh_fwd_bf16', B, h0, bufs['z0'].data_ptr(), P.p('ln.scale'), P.p('ln.offset'), 1e-5,
+               bufs['y0'].data_ptr(), bufs['y0_bf16'].data_ptr(), bufs['xhat'].data_ptr(), bufs['rstd'].data_ptr(), st)
+    x, d = bufs['y0_bf16'].data_ptr(), h0
+    for i in range(1, len(self.sizes)):
+      y = bufs[f'y{i}']
+      _capi.call('b200rl_linear_fwd_bf16', B, self.sizes[i], d, x, d, P.sp(f'l{i}.w'), P.p(f'l{i}.b'), y.data_ptr(), self.sizes[i],
+                 1, ACT_ELU, ws, wsb, st)
+      x, d = y.data_ptr(), self.sizes[i]
+    _capi.call('b200rl_linear_fwd_bf16', B, self.head_dim, d, x, d, P.sp(f'{self.head}.w'), P.p(f'{self.head}.b'),
+               bufs['out'].data_ptr(), self.head_dim, 0, ACT_NONE, ws, wsb, st)
+    return bufs['out']
+
+  def _backward_flat_bf16(self, x_ptr: int, bufs, gbufs, dout_ptr: int, param_grads: bool, input_grad: bool):
+    B, P, st = bufs['B'], self.params, _capi.current_stream()
+    ws, wsb = self.ws
+    n = len(self.sizes)
+    d_last = self.sizes[-1]
+    last = bufs[f'y{n - 1}'].data_ptr()
+    dy = gbufs[f'dy{n - 1}'].data_ptr()
+    _capi.call('b200rl_dense_head_bwd_bf16', B, self.head_dim, d_last, dout_ptr, self.head_dim, last, d_last,
+               P.sp(f'{self.head}.w'), dy, d_last, last, ACT_ELU, P.g(f'{self.head}.w') if param_grads else None,
+               P.g(f'{self.head}.b') if param_grads else None, ws, wsb, st)
+    for i in range(n - 1, 0, -1):
+      hdim, d = self.sizes[i], self.sizes[i - 1]
+      x = bufs[f'y{i - 1}'].data_ptr() if i > 1 else bufs['y0_bf16'].data_ptr()
+      if param_grads:
+        _capi.call('b200rl_linear_wgrad_bf16', B, hdim, d, dy, hdim, x, d, P.g(f'l{i}.w'), P.g(f'l{i}.b'), ws, wsb, st)
+      dx = gbufs[f'dy{i - 1}'].data_ptr()
+      # into y0 (tanh(LN(.)), handled by the fp32 LayerNorm backward): fp32, no mask
+      _capi.call('b200rl_linear_dgrad_bf16', B, hdim, d, dy, hdim, P.sp(f'l{i}.w'), dx, d, int(i > 1), x if i > 1 else None, 1,
+                 ACT_ELU, ws, wsb, st)
+      dy = dx
+    h0 = self.sizes[0]
+    _capi.call('b200rl_layernorm_tanh_bwd', B, h0, dy, bufs['y0'].data_ptr(), bufs['xhat'].data_ptr(),
+               bufs['rstd'].data_ptr(), P.p('ln.scale'), gbufs['dz0'].data_ptr(),
+               P.g('ln.scale') if param_grads else None, P.g('ln.offset') if param_grads else None, st)
+    dz0 = gbufs['dz0'].data_ptr()
+    if param_grads:
+      _capi.call('b200rl_linear_wgrad', B, h0, self.in_dim, dz0, h0, x_ptr, self.in_dim, P.g('l0.w'), P.g('l0.b'),
+                 _capi.PRECISION_TC, ws, wsb, st)
+    if input_grad:
+      _capi.call('b200rl_linear_dgrad', B, h0, self.in_dim, dz0, h0, P.p('l0.w'), gbufs['dx'].data_ptr(), self.in_dim, None,
+                 ACT_NONE, _capi.PRECISION_TC, ws, wsb, st)
+
   def forward_flat(self, x_ptr: int, bufs):
+    if self.flow:
+      return self._forward_flat_bf16(x_ptr, bufs)
     B, P, st = bufs['B'], self.params, _capi.current_stream()
     h0 = self.sizes[0]
     _linear(B, h0, self.in_dim, x_ptr, self.in_dim, P.p('l0.w'), P.p('l0.b'), bufs['z0'].data_ptr(), h0, ACT_NONE, self)
@@ -795,6 +875,8 @@ class LayerNormMLP(Network):
   def backward_flat(self, x_ptr: int, bufs, gbufs, dout_ptr: int, param_grads: bool = True, input_grad: bool = False):
     """dout: gradient w.r.t. the head output.  Writes params.grad (if param_grads) and gbufs['dx']
     (if input_grad)."""
+    if self.flow:
+      return self._backward_flat_bf16(x_ptr, bufs, gbufs, dout_ptr, param_grads, input_grad)
     B, P, st = bufs['B'], self.params, _capi.current_stream()
     n = len(self.sizes)
     d_last = self.sizes[-1]

@@ -389,6 +389,20 @@ int b200rl_colsum_bf16(int32_t M, int32_t N, const void* x_bf16, int32_t ld, flo
                        void* stream);
 int b200rl_linear_wgrad_bf16(int32_t M, int32_t N, int32_t K, const void* dy_bf16, int32_t lddy, const void* x_bf16,
                              int32_t ldx, float* dw, float* db, void* ws, int64_t ws_bytes, void* stream);
+/* b200rl_layernorm_tanh_fwd (same arithmetic, same y / xhat / rstd) that also stores y_bf16 = RN-bf16(y), [B, N] dense:
+ * the first hidden activation of a LayerNormMLP in the bf16 dataflow */
+int b200rl_layernorm_tanh_fwd_bf16(int32_t B, int32_t N, const float* x, const float* scale, const float* offset, float eps,
+                                   float* y, void* y_bf16, float* xhat, float* rstd, void* stream);
+/* Backward of a dense head with few outputs (the bf16 GEMMs above need N >= 64 / N % 64 == 0), one launch:
+ *   dx[M,K] = (dy[M,N] @ w[N,K]) * act'(mask)   bf16 (mask: bf16, NULL = none, shares dx's row stride)
+ *   dw[N,K] = dy^T @ x[M,K],  db[N] = colsum(dy)   fp32, each nullable (x may be NULL when dw is)
+ * dy fp32.  1 <= N <= 64, K % 8 == 0; x, w, dx, mask 16-byte aligned with row strides (ldx, K, lddx) multiples of 8;
+ * anything else is EINVAL without a launch.  FFMA with fp32 accumulation in a fixed order; dw / db summed over row
+ * slices through `ws` (up to ~33 KB per 64 columns per slice, fewer slices when smaller) with a per-stream last-CTA
+ * ticket: bit-identical across launches, streams and CUDA-graph replay. */
+int b200rl_dense_head_bwd_bf16(int32_t M, int32_t N, int32_t K, const float* dy, int32_t lddy, const void* x_bf16,
+                               int32_t ldx, const void* w_bf16, void* dx_bf16, int32_t lddx, const void* mask_bf16,
+                               int mask_act, float* dw, float* db, void* ws, int64_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------ data-parallel learner (SURVEY §8e)
  * Replaces all_reduce('mean', grads) followed by optimizer.apply on every replica

@@ -1,15 +1,39 @@
 """D4PG learner updates/s on the control-suite-humanoid shape (67-d obs, 21-d act, C51 critic), batch 256, n=5
-(BASELINE.json configs[2]); device-resident timing with CUDA events, whole step as a CUDA graph."""
-import sys, os, json
+(BASELINE.json configs[2]); device-resident timing with CUDA events, whole step as a CUDA graph.
+
+  python tools/d4pg_bench.py --precision tf32,bf16 --steps 300 --reps 3 [--out DIR]
+
+Several precisions (fp32 = 0, tf32 = 1, bf16 = 2, the network `precision` modes) are timed in one process, alternating
+per repetition, so that they share the GPU's state.  Each line reports ms per step for every repetition, kernel launches
+per eager step (`b200rl_launch_count`), and the GPU's name and power limit read in the same run.  `bench.py --workload
+d4pg` keeps measuring precision 1."""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-import numpy as np, torch
+import numpy as np
+import torch
+
 from acme_b200 import _capi, adders, d4pg, dm_env, loggers, networks, replay, specs
 
+PRECISIONS = {'fp32': _capi.PRECISION_FP32, 'tf32': _capi.PRECISION_TC, 'bf16': _capi.PRECISION_BF16FLOW}
 
-def main():
-  prec = _capi.PRECISION_BF16 if (len(sys.argv) < 2 or sys.argv[1] != 'fp32') else _capi.PRECISION_FP32
-  B, OBS, ACT, n, items = 256, 67, 21, 5, 100_000
+
+def gpu_info():
+  name = torch.cuda.get_device_name(0)
+  try:
+    limit = subprocess.run(['nvidia-smi', '-i', '0', '--query-gpu=power.limit', '--format=csv,noheader'], capture_output=True,
+                           text=True, timeout=30).stdout.strip() or None
+  except (OSError, subprocess.SubprocessError):
+    limit = None
+  return name, limit
+
+
+def fill_table(OBS, ACT, n, items):
   rng = np.random.default_rng(0)
   spec = specs.EnvironmentSpec(specs.Array((OBS,), np.float32), specs.BoundedArray((ACT,), np.float32, -1., 1.),
                                specs.Array((), np.float32), specs.BoundedArray((), np.float32, 0., 1.))
@@ -28,26 +52,64 @@ def main():
       adder.add(rng.uniform(-1, 1, ACT).astype(np.float32), ts(*args) if t == T - 1 else ts(args[0], args[1], np.float32(1.)))
       steps += 1
     table.flush()
-  kw = dict(precision=prec) if 'precision' in networks.D4PGPolicy.__init__.__code__.co_varnames else {}
-  policy, critic = networks.D4PGPolicy(OBS, ACT, seed=1, **kw), networks.D4PGCritic(OBS, ACT, seed=2, **kw)
-  ds = replay.ReplayDataset(table, B, seed=11, stratified=False)
-  L = d4pg.D4PGLearner(policy, critic, policy.clone(), critic.clone(), 0.99, target_update_period=100, dataset=ds,
-                       logger=loggers.NoOpLogger())
-  for _ in range(20):
-    L.step(fetch_loss=False) if 'fetch_loss' in L.step.__code__.co_varnames else L.step()
-  torch.cuda.synchronize()
-  K = 300
+  return table, server
+
+
+def main():
+  ap = argparse.ArgumentParser()
+  ap.add_argument('--precision', default='tf32', help='comma-separated subset of fp32, tf32, bf16')
+  ap.add_argument('--steps', type=int, default=300, help='timed updates per repetition')
+  ap.add_argument('--warmup', type=int, default=20)
+  ap.add_argument('--reps', type=int, default=3)
+  ap.add_argument('--out', default=None, help='directory for d4pg_bench_<precision>.json')
+  args = ap.parse_args()
+  names = [p.strip() for p in args.precision.split(',') if p.strip()]
+  for p in names:
+    if p not in PRECISIONS:
+      ap.error(f'unknown precision {p!r} (fp32, tf32, bf16)')
+  B, OBS, ACT, n = 256, 67, 21, 5
+  table, server = fill_table(OBS, ACT, n, 100_000)
+  lib = _capi.load()
+  learners, launches = {}, {}
+  for p in names:
+    policy = networks.D4PGPolicy(OBS, ACT, seed=1, precision=PRECISIONS[p])
+    critic = networks.D4PGCritic(OBS, ACT, seed=2, precision=PRECISIONS[p])
+    ds = replay.ReplayDataset(table, B, seed=11, stratified=False)
+    L = d4pg.D4PGLearner(policy, critic, policy.clone(), critic.clone(), 0.99, target_update_period=100, dataset=ds,
+                         logger=loggers.NoOpLogger())
+    L.step(fetch_loss=False)
+    torch.cuda.synchronize()
+    n0 = lib.b200rl_launch_count()
+    L.step(fetch_loss=False)          # the second update is still eager; the graph is captured at the third
+    torch.cuda.synchronize()
+    launches[p] = int(lib.b200rl_launch_count() - n0)
+    for _ in range(args.warmup):
+      L.step(fetch_loss=False)
+    torch.cuda.synchronize()
+    learners[p] = L
+  ms = {p: [] for p in names}
   e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-  e0.record()
-  for _ in range(K):
-    L.step(fetch_loss=False) if 'fetch_loss' in L.step.__code__.co_varnames else L.step()
-  e1.record(); torch.cuda.synchronize()
-  ms = e0.elapsed_time(e1) / K
-  out = {'workload': 'D4PG humanoid-shaped 67/21, C51 (51 atoms), batch 256, n=5', 'precision': 'fp32' if prec == 0 else 'tc',
-         'updates_per_s': 1e3 / ms, 'ms_per_step': ms}
-  print(json.dumps(out))
-  os.makedirs(os.path.join(ROOT, 'gpurun_out'), exist_ok=True)
-  json.dump(out, open(os.path.join(ROOT, 'gpurun_out', f"d4pg_bench_{out['precision']}.json"), 'w'))
+  for _ in range(args.reps):
+    for p in names:
+      L = learners[p]
+      torch.cuda.synchronize()
+      e0.record()
+      for _ in range(args.steps):
+        L.step(fetch_loss=False)
+      e1.record()
+      torch.cuda.synchronize()
+      ms[p].append(e0.elapsed_time(e1) / args.steps)
+  gpu, power_limit = gpu_info()
+  for p in names:
+    med = float(np.median(ms[p]))
+    out = {'workload': 'D4PG humanoid-shaped 67/21, C51 (51 atoms), batch 256, n=5', 'precision': p,
+           'precision_mode': PRECISIONS[p], 'steps_per_rep': args.steps, 'ms_per_step_reps': ms[p], 'ms_per_step': med,
+           'updates_per_s': 1e3 / med, 'launches_per_eager_step': launches[p], 'gpu': gpu, 'power_limit': power_limit}
+    print(json.dumps(out))
+    if args.out:
+      os.makedirs(args.out, exist_ok=True)
+      with open(os.path.join(args.out, f'd4pg_bench_{p}.json'), 'w') as f:
+        json.dump(out, f, indent=1)
   server.stop()
 
 
