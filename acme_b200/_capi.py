@@ -134,6 +134,13 @@ PROTOTYPES = {
     'b200rl_workspace_bytes': (c_i64, [c_i64]),
     'b200rl_conv2d_rows_bytes': (c_i64, [C.POINTER(ConvGeom)]),
     'b200rl_conv2d_rows_from_u8': (c_int, [c_vp, C.POINTER(ConvGeom), c_vp, c_i64, c_vp]),
+    'b200rl_x3_ws_bytes': (c_i64, [c_int, c_i32, c_i32, c_i32, C.POINTER(ConvGeom), c_int]),
+    'b200rl_linear_fwd_x3': (c_int, [c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i32, c_int, c_vp, c_i64, c_vp]),
+    'b200rl_linear_dgrad_x3': (c_int, [c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_vp, c_i32, c_vp, c_int, c_vp, c_i64, c_vp]),
+    'b200rl_linear_wgrad_x3': (c_int, [c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    'b200rl_conv2d_fwd_x3': (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, C.POINTER(ConvGeom), c_int, c_vp, c_i64, c_vp]),
+    'b200rl_conv2d_wgrad_x3': (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, C.POINTER(ConvGeom), c_vp, c_i64, c_vp]),
+    'b200rl_conv2d_dgrad_x3': (c_int, [c_vp, c_vp, c_vp, C.POINTER(ConvGeom), c_vp, c_int, c_vp, c_i64, c_vp]),
     'b200rl_dp_create': (c_int, [C.POINTER(c_vp), C.POINTER(DpCfg)]),
     'b200rl_dp_destroy': (c_int, [c_vp]),
     'b200rl_dp_buffers': (c_int, [c_vp, C.POINTER(c_vp), C.POINTER(c_vp)]),
@@ -163,7 +170,11 @@ TD_IS_WEIGHTS_F32 = 1
 #   1  tcgen05 with fp32 tensors: tf32 operands fetched by TMA where eligible, bf16 operands converted on the fly otherwise
 #   2  bf16 dataflow: activations, weight shadows and back-propagated gradients in bf16 (kind::f16), fp32 master weights /
 #      accumulation / optimizer (DQNAtariNetwork and the LayerNormMLP networks)
-PRECISION_FP32, PRECISION_TC, PRECISION_BF16FLOW = 0, 1, 2
+#   3  fp32-accurate layers on the bf16 tensor cores: fp32 tensors as in mode 0, every layer call through the `*_x3` entry
+#      points (each operand split into three bf16 planes, six products per fp32 product; the precision-0 tolerance)
+PRECISION_FP32, PRECISION_TC, PRECISION_BF16FLOW, PRECISION_FP32X3 = 0, 1, 2, 3
+# `op` of b200rl_x3_ws_bytes
+X3_LINEAR_FWD, X3_LINEAR_DGRAD, X3_LINEAR_WGRAD, X3_CONV_FWD, X3_CONV_WGRAD, X3_CONV_DGRAD = range(6)
 PRECISION_BF16 = PRECISION_TC      # historical name of mode 1
 
 _lib = None

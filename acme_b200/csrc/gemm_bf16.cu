@@ -684,16 +684,24 @@ static bool make_rows_map(CUtensorMap* m, const bf16* rows, const b200rl_conv_ge
              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-int h_conv_fwd_rows(const bf16* rows, const bf16* w, const float* bias, void* y, const b200rl_conv_geom& g, int act, int out_bf16,
-                    void* ws, int64_t wsb, cudaStream_t s) {
+static int conv_fwd_rows(const bf16* rows, const bf16* w, const float* bias, void* y, const b200rl_conv_geom& g, int act,
+                         int out_bf16, float scale, void* ws, int64_t wsb, cudaStream_t s) {
   const int M = g.B * g.OH * g.OW, K = g.kh * g.kw * g.C;
   if (!rows_eligible(g) || !ok16(w, K)) return 1;
   CUtensorMap ma, mb;
   if (!make_rows_map(&ma, rows, g, rows_view(g), HBM_ROWS) || !make_map_h(&mb, w, g.Cout, K, K, 32, g.Cout)) return 1;
-  Epilogue e = make_epi(y, g.Cout, bias, act, nullptr, 0, 0, 0, out_bf16, 0, 1.0f / 255.0f);
+  Epilogue e = make_epi(y, g.Cout, bias, act, nullptr, 0, 0, 0, out_bf16, 0, scale);
   ConvA conv{1, 32, 1, g.OW, g.OH, 1, g.stride, 0, 0, g.kh};
   if (g.Cout == 32) return launch_h<32, 0, 0, 32>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
   return launch_h<32, 0, 0, 64>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
+}
+int h_conv_fwd_rows(const bf16* rows, const bf16* w, const float* bias, void* y, const b200rl_conv_geom& g, int act, int out_bf16,
+                    void* ws, int64_t wsb, cudaStream_t s) {
+  return conv_fwd_rows(rows, w, bias, y, g, act, out_bf16, 1.0f / 255.0f, ws, wsb, s);
+}
+// the raw fp32 accumulator (no bias, no activation, no 1/255): one product of a split filter, summed by fp32x3.cu's combine
+int h_conv_fwd_rows_raw(const bf16* rows, const bf16* w, float* y, const b200rl_conv_geom& g, void* ws, int64_t wsb, cudaStream_t s) {
+  return conv_fwd_rows(rows, w, nullptr, y, g, B200RL_ACT_NONE, 0, 1.0f, ws, wsb, s);
 }
 int h_conv_wgrad_rows(const bf16* rows, const bf16* dy, float* dw, float* db, const b200rl_conv_geom& g, void* ws, int64_t wsb,
                       cudaStream_t s) {

@@ -89,7 +89,9 @@ static inline int small_dense(int precision, int M, int N, int K) {
 }
 extern "C" int b200rl_debug_set_tma(int on) { g_use_tma = on != 0; return 0; }
 
-static int check_geom(const b200rl_conv_geom* g) {
+// shared with the fp32x3.cu entry points
+namespace b200rl {
+int check_geom(const b200rl_conv_geom* g) {
   B200RL_REQUIRE(g, "null geometry");
   B200RL_REQUIRE(g->B >= 1 && g->H >= 1 && g->W >= 1 && g->C >= 1 && g->Cout >= 1, "bad conv shape");
   B200RL_REQUIRE(g->kh >= 1 && g->kw >= 1 && g->stride >= 1 && g->OH >= 1 && g->OW >= 1, "bad conv filter");
@@ -100,10 +102,11 @@ static int check_geom(const b200rl_conv_geom* g) {
 // The convolution loaders of every precision read an fp32 activation / gradient / filter as float4 (im2col of x; dy and
 // w of the data gradient) and a uint8 frame as one 4-byte pixel (C % 4 == 0), with no alignment test on the device.
 // A misaligned pointer is therefore rejected here, before anything is launched.
-static int check_conv_ptr(const void* p, int u8, const char* what) {
+int check_conv_ptr(const void* p, int u8, const char* what) {
   B200RL_REQUIRE(((uintptr_t)p & (u8 ? 3 : 15)) == 0, "%s must be %d-byte aligned", what, u8 ? 4 : 16);
   return B200RL_OK;
 }
+}  // namespace b200rl
 
 #define PRECISION_SWITCH(simt_call, tc_call)                                                   \
   if (precision == 0) return simt_call;                                                        \

@@ -153,12 +153,41 @@ class Network:
     """precision 2: the bf16 dataflow"""
     return self.precision == _capi.PRECISION_BF16FLOW
 
+  @property
+  def x3(self) -> bool:
+    """precision 3: fp32 tensors, every layer call through the `*_x3` entry points (split bf16 operands)"""
+    return self.precision == _capi.PRECISION_FP32X3
+
+  def _x3_calls(self, B: int):
+    """(op, M, N, K, conv geometry, x_u8) of every `*_x3` layer call a pass at batch B makes."""
+    raise NotImplementedError
+
+  def _size_lanes(self, B: int):
+    """Precision 3: grows the workspace lanes to the largest b200rl_x3_ws_bytes of the layer calls at batch B (in place,
+    so that clones sharing the lanes see them).  Other precisions keep their fixed lanes."""
+    import ctypes
+    import torch
+    if not self.x3:
+      return
+    lib = _capi.load()
+    need = 0
+    for op, M, N, K, g, x_u8 in self._x3_calls(B):
+      n = int(lib.b200rl_x3_ws_bytes(op, M, N, K, ctypes.byref(g) if g is not None else None, x_u8))
+      if n < 0:
+        raise ValueError(f'precision 3: layer call {op} {(M, N, K)} has a shape no path takes')
+      need = max(need, n)
+    if need > self._ws_all[0].numel():
+      dev = torch.device('cuda', self.device)
+      self._ws_all[:] = [torch.empty(need, dtype=torch.uint8, device=dev) for _ in range(3)]
+
   def _finalize(self):
     import torch
     _capi.require_device(self.device)
     self.params.allocate()
     # one split-K / partial-sum workspace per concurrent stream (see Network.lanes)
-    self._ws_all = [torch.empty(96 << 20, dtype=torch.uint8, device=torch.device('cuda', self.device)) for _ in range(3)]
+    # (precision 3: sized by make_buffers from the layer calls at its batch, see _size_lanes)
+    lane_bytes = 0 if self.x3 else 96 << 20
+    self._ws_all = [torch.empty(lane_bytes, dtype=torch.uint8, device=torch.device('cuda', self.device)) for _ in range(3)]
     self._lane = 0
 
   @property
@@ -226,22 +255,51 @@ class Network:
       self.params.set(name, v)
 
 
+# fp32-tensor layer calls: precisions 0 / 1 through the fp32 entry points, precision 3 through the `*_x3` ones
 def _linear(M, N, K, x, ldx, w, b, y, ldy, act, net: Network):
   ws, wsb = net.ws
+  if net.x3:
+    return _capi.call('b200rl_linear_fwd_x3', M, N, K, x, ldx, w, b, y, ldy, act, ws, wsb, _capi.current_stream())
   _capi.call('b200rl_linear_fwd', M, N, K, x, ldx, w, b, y, ldy, act, net.precision, ws, wsb,
              _capi.current_stream())
 
 
 def _linear_dgrad(M, N, K, dy, lddy, w, dx, lddx, mask, mask_act, net: Network):
   ws, wsb = net.ws
+  if net.x3:
+    return _capi.call('b200rl_linear_dgrad_x3', M, N, K, dy, lddy, w, dx, lddx, mask, mask_act, ws, wsb,
+                      _capi.current_stream())
   _capi.call('b200rl_linear_dgrad', M, N, K, dy, lddy, w, dx, lddx, mask, mask_act, net.precision, ws,
              wsb, _capi.current_stream())
 
 
 def _linear_wgrad(M, N, K, dy, lddy, x, ldx, dw, db, net: Network):
   ws, wsb = net.ws
+  if net.x3:
+    return _capi.call('b200rl_linear_wgrad_x3', M, N, K, dy, lddy, x, ldx, dw, db, ws, wsb, _capi.current_stream())
   _capi.call('b200rl_linear_wgrad', M, N, K, dy, lddy, x, ldx, dw, db, net.precision, ws, wsb,
              _capi.current_stream())
+
+
+def _conv_fwd(x, x_u8, w, b, y, g, act, net: Network):
+  ws, wsb = net.ws
+  if net.x3:
+    return _capi.call('b200rl_conv2d_fwd_x3', x, x_u8, w, b, y, g, act, ws, wsb, _capi.current_stream())
+  _capi.call('b200rl_conv2d_fwd', x, x_u8, w, b, y, g, act, net.precision, ws, wsb, _capi.current_stream())
+
+
+def _conv_wgrad(x, x_u8, dy, dw, db, g, net: Network):
+  ws, wsb = net.ws
+  if net.x3:
+    return _capi.call('b200rl_conv2d_wgrad_x3', x, x_u8, dy, dw, db, g, ws, wsb, _capi.current_stream())
+  _capi.call('b200rl_conv2d_wgrad', x, x_u8, dy, dw, db, g, net.precision, ws, wsb, _capi.current_stream())
+
+
+def _conv_dgrad(dy, w, dx, g, mask, mask_act, net: Network):
+  ws, wsb = net.ws
+  if net.x3:
+    return _capi.call('b200rl_conv2d_dgrad_x3', dy, w, dx, g, mask, mask_act, ws, wsb, _capi.current_stream())
+  _capi.call('b200rl_conv2d_dgrad', dy, w, dx, g, mask, mask_act, net.precision, ws, wsb, _capi.current_stream())
 
 
 # =============================================================================== DQN Atari network
@@ -307,7 +365,20 @@ class DQNAtariNetwork(Network):
     bufs = dict(B=B, q=f(B, self.A), h=f(B, 1024), val=f(B, 1), adv=f(B, self.A))
     for i, (k, s, ci, co, h, oh, pad) in enumerate(self.convs, 1):
       bufs[f'y{i}'] = a(B, oh, oh, co)
+    self._size_lanes(B)
     return bufs
+
+  def _x3_calls(self, B: int):
+    X = _capi
+    calls = [(X.X3_LINEAR_FWD, B, 1024, self.flat_dim, None, 0), (X.X3_LINEAR_DGRAD, B, 1024, self.flat_dim, None, 0),
+             (X.X3_LINEAR_WGRAD, B, 1024, self.flat_dim, None, 0)]
+    for i in range(3):
+      g = self.geom(i, B)
+      x_u8s = (1, 2) if i == 0 else (0,)     # conv1 on uint8 frames or on their row image
+      calls += [(op, 0, 0, 0, g, u) for u in x_u8s for op in (X.X3_CONV_FWD, X.X3_CONV_WGRAD)]
+      if i > 0:
+        calls.append((X.X3_CONV_DGRAD, 0, 0, 0, g, 0))
+    return calls
 
   def make_grad_buffers(self, B: int):
     import torch
@@ -322,9 +393,9 @@ class DQNAtariNetwork(Network):
     return g
 
   def rows_frame_bytes(self) -> int:
-    """Bytes of ONE frame in the bf16 row image (bf16 dataflow): a batched image can be sliced per sample range."""
+    """Bytes of ONE frame in the bf16 row image (precisions 2 and 3): a batched image can be sliced per sample range."""
     import ctypes
-    return int(_capi.load().b200rl_conv2d_rows_bf16_bytes(ctypes.byref(self.geom(0, 1)))) if self.flow else 0
+    return int(_capi.load().b200rl_conv2d_rows_bf16_bytes(ctypes.byref(self.geom(0, 1)))) if self.flow or self.x3 else 0
 
   def rows_buffer(self, B: int, slot: str = 'x'):
     """The (cached, zero-initialised) row-image buffer of B frames; None if the geometry has no row image.  Zeroed because
@@ -334,7 +405,7 @@ class DQNAtariNetwork(Network):
     cache = self.__dict__.setdefault('_rows', {})
     if (slot, B) not in cache:
       lib = _capi.load()
-      fn = lib.b200rl_conv2d_rows_bf16_bytes if self.flow else lib.b200rl_conv2d_rows_bytes
+      fn = lib.b200rl_conv2d_rows_bf16_bytes if self.flow or self.x3 else lib.b200rl_conv2d_rows_bytes
       nbytes = int(fn(ctypes.byref(self.geom(0, B))))
       cache[(slot, B)] = (torch.zeros(nbytes, dtype=torch.uint8, device=torch.device('cuda', self.device)) if nbytes > 0 else None)
     return cache[(slot, B)]
@@ -342,8 +413,8 @@ class DQNAtariNetwork(Network):
   def prepare_frames(self, obs, slot: str = 'x'):
     """uint8 frames -> the row image that first-layer calls accept, built ONCE for all the passes over the same frames
     (two networks on o_t; forward + weight gradient on o_tm1).  Precision 1: zero-padded fp32 rows x/255
-    (`b200rl_conv2d_rows_from_u8`); precision 2: zero-padded bf16 rows of the integer pixel values
-    (`b200rl_conv2d_rows_bf16_from_u8`).  None when not applicable (fp32 mode, float frames, geometry not eligible):
+    (`b200rl_conv2d_rows_from_u8`); precisions 2 and 3: zero-padded bf16 rows of the integer pixel values
+    (`b200rl_conv2d_rows_bf16_from_u8`, exact in bf16).  None when not applicable (fp32 mode, float frames, geometry not eligible):
     callers then pass the frames themselves."""
     import ctypes
     import torch
@@ -355,7 +426,7 @@ class DQNAtariNetwork(Network):
       if self.flow:
         raise ValueError('the bf16 dataflow needs the Atari first-layer geometry (C = 4, kw * C = 32)')
       return None
-    name = 'b200rl_conv2d_rows_bf16_from_u8' if self.flow else 'b200rl_conv2d_rows_from_u8'
+    name = 'b200rl_conv2d_rows_bf16_from_u8' if self.flow or self.x3 else 'b200rl_conv2d_rows_from_u8'
     _capi.call(name, obs.data_ptr(), self.geom(0, B), buf.data_ptr(), buf.numel(), _capi.current_stream())
     return buf
 
@@ -393,9 +464,7 @@ class DQNAtariNetwork(Network):
       x, x_u8 = rows.data_ptr(), 2
     for i in range(3):
       y = bufs[f'y{i + 1}']
-      g = self.geom(i, B)
-      _capi.call('b200rl_conv2d_fwd', x, x_u8, P.p(f'conv{i + 1}.w'), P.p(f'conv{i + 1}.b'), y.data_ptr(),
-                 g, ACT_RELU, self.precision, ws, wsb, st)
+      _conv_fwd(x, x_u8, P.p(f'conv{i + 1}.w'), P.p(f'conv{i + 1}.b'), y.data_ptr(), self.geom(i, B), ACT_RELU, self)
       x, x_u8 = y.data_ptr(), 0
     if before_fc1 is not None:
       before_fc1()
@@ -491,8 +560,7 @@ class DQNAtariNetwork(Network):
       x, x_u8 = rows.data_ptr(), 2
     else:
       x, x_u8 = obs.data_ptr(), int(obs.dtype == torch.uint8)
-    _capi.call('b200rl_conv2d_wgrad', x, x_u8, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b'), g, self.precision, ws, wsb,
-               _capi.current_stream())
+    _conv_wgrad(x, x_u8, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b'), g, self)
 
   def _conv_dgrad(self, i, bufs, gbufs):
     B, P = bufs['B'], self.params
@@ -503,8 +571,7 @@ class DQNAtariNetwork(Network):
       _capi.call('b200rl_conv2d_dgrad_bf16', dy, P.sp(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), 1, g,
                  bufs[f'y{i}'].data_ptr(), 1, ACT_RELU, _capi.current_stream())
     else:
-      _capi.call('b200rl_conv2d_dgrad', dy, P.p(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), g, bufs[f'y{i}'].data_ptr(),
-                 ACT_RELU, self.precision, ws, wsb, _capi.current_stream())
+      _conv_dgrad(dy, P.p(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), g, bufs[f'y{i}'].data_ptr(), ACT_RELU, self)
 
   def backward(self, obs, bufs, gbufs, dq, side_stream=None, rows=None):
     """Accumulates nothing: overwrites params.grad with d(loss)/d(params) given dq [B, A].  `rows`: the row image of
@@ -684,7 +751,13 @@ class MLPQNetwork(Network):
     for i, hdim in enumerate(self.sizes):
       bufs[f'y{i}'] = torch.empty((B, hdim), dtype=torch.float32, device=dev)
     bufs['q'] = bufs[f'y{len(self.sizes) - 1}']
+    self._size_lanes(B)
     return bufs
+
+  def _x3_calls(self, B: int):
+    dims = [self.in_dim] + self.sizes
+    return [(op, B, dims[i + 1], dims[i], None, 0) for i in range(len(self.sizes))
+            for op in (_capi.X3_LINEAR_FWD, _capi.X3_LINEAR_DGRAD, _capi.X3_LINEAR_WGRAD)]
 
   def make_grad_buffers(self, B: int):
     import torch
@@ -793,7 +866,13 @@ class LayerNormMLP(Network):
       bufs['y0_bf16'] = a(B, h0)
     for i in range(1, len(self.sizes)):
       bufs[f'y{i}'] = a(B, self.sizes[i])
+    self._size_lanes(B)
     return bufs
+
+  def _x3_calls(self, B: int):
+    dims = [self.in_dim] + self.sizes + [self.head_dim]
+    return [(op, B, dims[i + 1], dims[i], None, 0) for i in range(len(dims) - 1)
+            for op in (_capi.X3_LINEAR_FWD, _capi.X3_LINEAR_DGRAD, _capi.X3_LINEAR_WGRAD)]
 
   def make_grad_buffers(self, B: int):
     import torch

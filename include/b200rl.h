@@ -404,6 +404,53 @@ int b200rl_dense_head_bwd_bf16(int32_t M, int32_t N, int32_t K, const float* dy,
                                int32_t ldx, const void* w_bf16, void* dx_bf16, int32_t lddx, const void* mask_bf16,
                                int mask_act, float* dw, float* db, void* ws, int64_t ws_bytes, void* stream);
 
+/* ------------------------------------------------------------------ K6, precision 3 (fp32-accurate on the bf16 tensor cores)
+ * The fp32 entry points above, minus `precision`, with fp32 operands, outputs, masks, biases and parameter gradients.
+ * Every operand value x is split, in fp32, into three bf16 planes hi = RN(x), mid = RN(x - hi), lo = RN(x - hi - mid)
+ * (both subtractions exact), and a * b is computed as the six bf16 products hi hi + hi mid + mid hi + hi lo + mid mid +
+ * lo hi in the fp32 accumulator (three products against conv1's integer row image, which is exact in bf16).
+ * Tolerance: the dropped terms and the split residual are O(2^-25 |a||b|); the rest is the tensor cores' fp32
+ * accumulation: |err| <= 2^-16 * (|A|.|B|) elementwise, the precision-0 bound (measured up to 7.5e-6 |A|.|B| on B200).
+ * That accumulation is not round-to-nearest: sums whose products all share one sign can exceed the bound (measured
+ * 1.8e-5 .. 3.9e-5 of the sum); the bound holds for operands of mixed signs.
+ * Range: finite inputs of normal magnitude, |x| in [2^-96, 2^96]; a non-finite input gives a non-finite output.
+ * Path, chosen from the shape alone (the same rule decides b200rl_x3_ws_bytes):
+ *   (a) planes concatenated along the reduction (dense forward: K, data gradient: N, weight gradient: M; conv forward:
+ *       Cin, weight gradient: the batch, data gradient: Cout), zero-padded (K and N to multiples of 8, Cin and Cout to
+ *       multiples of 32), and ONE bf16 GEMM of the b200rl_*_bf16 family with its own epilogue (bias, activation, mask):
+ *       dense layers of >= 2^26 multiply-adds with  forward: 6 * roundup(K, 8) >= 64;  data gradient: K % 64 == 0 and
+ *       6 * roundup(N, 8) >= 64;  weight gradient: N % 64 == 0 and K % 64 == 0.  Convolutions with  forward (fp32 x):
+ *       Cout in {32, 64, 128};  weight gradient (fp32 x): C == 32 or C % 64 == 0, Cout in {32, 64};  weight gradient on
+ *       frames (x_u8 = 1 / 2, first-layer geometry: the row image three times along the batch);  data gradient:
+ *       stride <= 2, stride <= kh and kw, C in {32, 64, 128}.
+ *   (b) conv forward on frames (x_u8 = 1 / 2, first-layer geometry C = 4, kw * C = 32, Cout in {32, 64}): one raw fp32
+ *       bf16 launch per filter plane, then one combine kernel (lo + mid + hi, then 1/255, bias, activation).
+ *   (c) everything else: the precision-0 FFMA path, unchanged.
+ * Bias gradients are the fp32 column sums of the unsplit dy.  x_u8: 0 = fp32 NHWC, 1 = uint8 frames, 2 = the integer bf16
+ * row image of b200rl_conv2d_rows_bf16_from_u8.  Alignment as at precision 0.  ws: at least b200rl_x3_ws_bytes(op, ...)
+ * bytes, 256-byte aligned (paths a / b); one workspace per stream.  Anything else is B200RL_EINVAL without a launch.
+ * Results are bit-identical across repeats, streams, programmatic dependent launch on / off and CUDA-graph replay. */
+#define B200RL_X3_LINEAR_FWD 0
+#define B200RL_X3_LINEAR_DGRAD 1
+#define B200RL_X3_LINEAR_WGRAD 2
+#define B200RL_X3_CONV_FWD 3
+#define B200RL_X3_CONV_WGRAD 4
+#define B200RL_X3_CONV_DGRAD 5
+/* workspace bytes one call of `op` needs: M, N, K for the dense ops, g and x_u8 for the convolutions; -1 = bad shape */
+int64_t b200rl_x3_ws_bytes(int op, int32_t M, int32_t N, int32_t K, const b200rl_conv_geom* g, int x_u8);
+int b200rl_linear_fwd_x3(int32_t M, int32_t N, int32_t K, const float* x, int32_t ldx, const float* w, const float* bias,
+                         float* y, int32_t ldy, int act, void* ws, int64_t ws_bytes, void* stream);
+int b200rl_linear_dgrad_x3(int32_t M, int32_t N, int32_t K, const float* dy, int32_t lddy, const float* w, float* dx,
+                           int32_t lddx, const float* mask_y, int mask_act, void* ws, int64_t ws_bytes, void* stream);
+int b200rl_linear_wgrad_x3(int32_t M, int32_t N, int32_t K, const float* dy, int32_t lddy, const float* x, int32_t ldx,
+                           float* dw, float* db, void* ws, int64_t ws_bytes, void* stream);
+int b200rl_conv2d_fwd_x3(const void* x, int x_u8, const float* w, const float* bias, float* y, const b200rl_conv_geom* g,
+                         int act, void* ws, int64_t ws_bytes, void* stream);
+int b200rl_conv2d_wgrad_x3(const void* x, int x_u8, const float* dy, float* dw, float* db, const b200rl_conv_geom* g,
+                           void* ws, int64_t ws_bytes, void* stream);
+int b200rl_conv2d_dgrad_x3(const float* dy, const float* w, float* dx, const b200rl_conv_geom* g, const float* mask_y,
+                           int mask_act, void* ws, int64_t ws_bytes, void* stream);
+
 /* ------------------------------------------------------------------ data-parallel learner (SURVEY §8e)
  * Replaces all_reduce('mean', grads) followed by optimizer.apply on every replica
  * (acme/agents/tf/crr/recurrent_learning.py:346-359, the reference's only multi-replica learner) by ONE kernel
