@@ -47,6 +47,7 @@ PROTOTYPES = {
     'b200rl_writer_close': (c_int, [c_vp, c_i32]),
     'b200rl_writer_append_stream': (c_int, [c_vp, c_i32, c_i64, c_vp, c_int, c_vp, c_vp, c_vp, c_vp,
                                             c_vp, c_i32, c_f64, c_vp]),
+    'b200rl_writer_append_multi': (c_int, [c_vp, c_i64, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_f64, c_vp]),
     'b200rl_replay_flush': (c_int, [c_vp, c_vp]),
     'b200rl_replay_sample': (c_int, [c_vp, c_i32, c_vp, c_int, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_replay_sample_philox': (c_int, [c_vp, c_i32, c_u64, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp]),
@@ -69,6 +70,8 @@ PROTOTYPES = {
     'b200rl_replay_set_global_mass': (c_int, [c_vp, c_vp]),
     'b200rl_replay_set_weights': (c_int, [c_vp, c_i64, c_vp, c_vp]),
     'b200rl_uniform': (c_int, [c_vp, c_i32, c_u64, c_vp, c_i64, c_vp]),
+    'b200rl_epsilon_greedy': (c_int, [c_i32, c_i32, c_vp, c_i64, c_f32, c_u64, c_vp, c_vp, c_vp, c_vp]),
+    'b200rl_gaussian_explore': (c_int, [c_i32, c_i32, c_vp, c_f32, c_vp, c_vp, c_u64, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_dqn_td': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_f32, c_f32,
                               c_f64, c_f32, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp]),
     'b200rl_is_weight_max': (c_int, [c_i32, c_vp, c_f64, c_vp, c_i32, c_vp]),

@@ -8,7 +8,7 @@ Behaviour contract (SURVEY App. A.3, from `acme/agents/agent.py:45-89`; pinned b
   * `observations_per_step >= 1` -> period = int(ratio), burst = 1; a ratio below one -> period = 1, burst = int(1/ratio).
 """
 
-from typing import List, Tuple
+from typing import Dict, List, Tuple
 
 from acme_b200 import core
 
@@ -64,3 +64,47 @@ class Agent(core.Actor, core.VariableSource):
 
   def get_variables(self, names: List[str]):
     return self._learner.get_variables(names)
+
+
+class BatchedAgent(Agent):
+  """An Agent whose actor acts for N environments at once (`actors.BatchedActor`), driven by
+  `environment_loop.BatchedEnvironmentLoop`.  After each step of the N environments, `update()` runs exactly the learner
+  updates `Agent` would run for the same N observations fed one at a time with an `update()` after each: every
+  observation is counted and the schedule's `due()` summed (a single `due()` per step would skip periods)."""
+
+  _due = 0
+
+  @property
+  def num_envs(self) -> int:
+    return self._actor.num_envs
+
+  def select_actions(self, observations):
+    return self._actor.select_actions(observations)
+
+  def observe_first(self, timesteps):
+    self._actor.observe_first(timesteps)
+
+  def observe(self, actions, next_timesteps):
+    for _ in next_timesteps:
+      self._schedule.saw_observation()
+      self._due += self._schedule.due()
+    self._actor.observe(actions, next_timesteps)
+
+  def update(self):
+    n, self._due = self._due, 0
+    if n == 0:
+      return
+    for _ in range(n):
+      self._learner.step()
+    self._actor.update()
+
+  _variants: Dict[type, type] = {}
+
+  @classmethod
+  def variant_of(cls, agent_cls: type) -> type:
+    """`agent_cls` (an Agent subclass whose constructor builds the actor) with the batched acting protocol."""
+    if issubclass(agent_cls, cls):
+      return agent_cls
+    if agent_cls not in cls._variants:
+      cls._variants[agent_cls] = type(f'Batched{agent_cls.__name__}', (cls, agent_cls), {'__module__': agent_cls.__module__})
+    return cls._variants[agent_cls]

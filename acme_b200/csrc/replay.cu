@@ -942,28 +942,27 @@ extern "C" int b200rl_writer_close(b200rl_replay* h, int32_t writer) {
   return B200RL_OK;
 }
 
-extern "C" int b200rl_writer_append_stream(b200rl_replay* h, int32_t writer, int64_t n, const void* obs,
-                                           int obs_on_device, const void* act, const float* rew,
-                                           const float* disc, const uint8_t* first,
-                                           const uint8_t* last, int32_t n_step, double priority,
-                                           void* stream_) {
-  B200RL_REQUIRE(h && obs && rew && disc && first && last, "null argument");
-  B200RL_LOCK(h);
+// Stream insert of `n` timesteps; element i belongs to writer writers[i] (or to `writer` for every element when `writers` is
+// NULL).  A writer's elements are consecutive timesteps of its stream in array order.
+static int append_stream_impl(b200rl_replay* h, int64_t n, const int32_t* writers, int32_t writer, const void* obs,
+                              int obs_on_device, const void* act, const float* rew, const float* disc, const uint8_t* first,
+                              const uint8_t* last, int32_t n_step, double priority, cudaStream_t stream) {
+  B200RL_REQUIRE(obs && rew && disc && first && last, "null argument");
   B200RL_REQUIRE(n_step >= 1 && n_step <= h->cfg.max_window, "n_step must be in [1, max_window]");
   B200RL_REQUIRE(n >= 0 && n <= h->S, "a stream chunk cannot exceed slot_capacity");
-  Writer* w = get_writer(h, writer);
-  if (!w) return B200RL_EINVAL;
+  for (int64_t i = 0; i < (writers ? n : 1); ++i)   // every writer id before any state changes
+    if (!get_writer(h, writers ? writers[i] : writer)) return B200RL_EINVAL;
   int rc = ensure_device(h);
   if (rc) return rc;
-  cudaStream_t stream = as_stream(stream_);
-  cudaStream_t saved = g_implicit_stream;
-  g_implicit_stream = stream;
   // obs_on_device: 0 = host observations as the signature has them; 1 = device observations as the signature has them;
   // 2 = device SINGLE FRAMES [n][obs_bytes / frame_stack] (frame-deduplicated tables: what the ring stores)
   B200RL_REQUIRE(obs_on_device != 2 || h->F > 1, "obs_on_device = 2 (single frames) needs a frame-deduplicated table");
+  cudaStream_t saved = g_implicit_stream;
+  g_implicit_stream = stream;
   const int32_t ob = h->cfg.obs_bytes;
   if (obs_on_device) {
-    // pending host-staged observations must land first (slot order), then one or two D2D runs
+    // pending host-staged observations must land first (slot order), then one or two D2D runs: element i takes slot
+    // slot_head + i, whichever writer it belongs to
     rc = flush_impl(h, stream);
     if (rc) { g_implicit_stream = saved; return rc; }
     int64_t firsti = (int64_t)(h->slot_head % (uint64_t)h->S);
@@ -988,6 +987,7 @@ extern "C" int b200rl_writer_append_stream(b200rl_replay* h, int32_t writer, int
   }
   const uint8_t* acts = (const uint8_t*)act;
   for (int64_t i = 0; i < n && rc == 0; ++i) {
+    Writer* w = &h->writers[writers ? writers[i] : writer];
     if (first[i]) {  // a FIRST timestep: any unfinished episode of this writer is abandoned
       w->hist.clear();
       w->k = 0;
@@ -1035,6 +1035,27 @@ extern "C" int b200rl_writer_append_stream(b200rl_replay* h, int32_t writer, int
   if (rc == 0) rc = flush_impl(h, stream);
   g_implicit_stream = saved;
   return rc;
+}
+
+extern "C" int b200rl_writer_append_stream(b200rl_replay* h, int32_t writer, int64_t n, const void* obs,
+                                           int obs_on_device, const void* act, const float* rew,
+                                           const float* disc, const uint8_t* first,
+                                           const uint8_t* last, int32_t n_step, double priority,
+                                           void* stream_) {
+  B200RL_REQUIRE(h, "null argument");
+  B200RL_LOCK(h);
+  return append_stream_impl(h, n, nullptr, writer, obs, obs_on_device, act, rew, disc, first, last, n_step, priority,
+                            as_stream(stream_));
+}
+
+extern "C" int b200rl_writer_append_multi(b200rl_replay* h, int64_t n, const int32_t* writers, const void* obs,
+                                          int obs_on_device, const void* act, const float* rew, const float* disc,
+                                          const uint8_t* first, const uint8_t* last, int32_t n_step, double priority,
+                                          void* stream_) {
+  B200RL_REQUIRE(h && writers, "null argument");
+  B200RL_LOCK(h);
+  return append_stream_impl(h, n, writers, -1, obs, obs_on_device, act, rew, disc, first, last, n_step, priority,
+                            as_stream(stream_));
 }
 
 extern "C" int b200rl_replay_reset(b200rl_replay* h, void* stream_) {

@@ -336,12 +336,17 @@ class D4PG(agent.Agent):
 
   _learner_cls = D4PGLearner
 
+  def __new__(cls, *args, num_envs: int = 1, **kwargs):
+    return super().__new__(agent.BatchedAgent.variant_of(cls) if num_envs > 1 else cls)
+
   def __init__(self, environment_spec: specs.EnvironmentSpec, policy_network: networks.D4PGPolicy,
                critic_network: networks.D4PGCritic, discount: float = 0.99, batch_size: int = 256,
                prefetch_size: int = 4, target_update_period: int = 100, min_replay_size: int = 1000,
                max_replay_size: int = 1000000, samples_per_insert: float = 32.0, n_step: int = 5,
                sigma: float = 0.3, clipping: bool = True, logger: loggers.Logger = None, checkpoint: bool = False,
-               seed: int = 0, use_cuda_graph: bool = True):
+               seed: int = 0, use_cuda_graph: bool = True, num_envs: int = 1):
+    """num_envs > 1: the agent is an `agent.BatchedAgent` acting for that many environments at once through
+    `actors.BatchedActor` (Gaussian exploration on the device), to be driven by `environment_loop.BatchedEnvironmentLoop`."""
     table = replay.Table(name=replay.DEFAULT_PRIORITY_TABLE, sampler=replay.selectors.Uniform(),
                          remover=replay.selectors.Fifo(), max_size=max_replay_size,
                          rate_limiter=replay.rate_limiters.MinSize(1),
@@ -349,12 +354,16 @@ class D4PG(agent.Agent):
                          discount=discount, device=critic_network.device)
     self._server = replay.Server([table], port=None)
     address = f'localhost:{self._server.port}'
-    # the reference passes priority_fns={table: lambda x: 1.} (agent.py:108): the default does the same
-    adder = adders.NStepTransitionAdder(client=replay.Client(address), n_step=n_step, discount=discount)
     dataset = replay.make_reverb_dataset(server_address=address, batch_size=batch_size, prefetch_size=prefetch_size,
                                          seed=seed, stratified=False)
     aspec = environment_spec.actions
-    actor = actors.FeedForwardActor(GaussianNoisePolicy(policy_network, sigma, aspec.minimum, aspec.maximum, seed), adder)
+    if num_envs > 1:
+      actor = actors.BatchedActor(actors.BatchedGaussianNoise(policy_network, sigma, aspec.minimum, aspec.maximum, seed),
+                                  table, num_envs, n_step, use_cuda_graph=use_cuda_graph)
+    else:
+      # the reference passes priority_fns={table: lambda x: 1.} (agent.py:108): the default does the same
+      adder = adders.NStepTransitionAdder(client=replay.Client(address), n_step=n_step, discount=discount)
+      actor = actors.FeedForwardActor(GaussianNoisePolicy(policy_network, sigma, aspec.minimum, aspec.maximum, seed), adder)
     learner = self._learner_cls(policy_network, critic_network, policy_network.clone(), critic_network.clone(), discount,
                                 target_update_period, dataset, clipping=clipping, logger=logger, checkpoint=checkpoint,
                                 use_cuda_graph=use_cuda_graph)

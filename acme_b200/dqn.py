@@ -1011,14 +1011,20 @@ class DQNLearner(core.Learner, core.Saveable):
 class DQN(agent.Agent):
   """`acme/agents/tf/dqn/agent.py:36-167` with the replay, adder, dataset and learner of this package."""
 
+  def __new__(cls, *args, num_envs: int = 1, **kwargs):
+    return super().__new__(agent.BatchedAgent.variant_of(cls) if num_envs > 1 else cls)
+
   def __init__(self, environment_spec: specs.EnvironmentSpec, network, batch_size: int = 256,
                prefetch_size: int = 4, target_update_period: int = 100, samples_per_insert: float = 32.0,
                min_replay_size: int = 1000, max_replay_size: int = 1000000,
                importance_sampling_exponent: float = 0.2, priority_exponent: float = 0.6, n_step: int = 5,
                epsilon: Optional[float] = None, learning_rate: float = 1e-3, discount: float = 0.99,
                logger: loggers.Logger = None, checkpoint: bool = False, checkpoint_subpath: str = '~/acme/',
-               seed: int = 0, use_cuda_graph: bool = True, slot_capacity: Optional[int] = None, frame_stack: int = 0):
-    """frame_stack: see `replay.Table` -- store one frame per step when the observations are AtariWrapper frame stacks."""
+               seed: int = 0, use_cuda_graph: bool = True, slot_capacity: Optional[int] = None, frame_stack: int = 0,
+               num_envs: int = 1):
+    """frame_stack: see `replay.Table` -- store one frame per step when the observations are AtariWrapper frame stacks.
+    num_envs > 1: the agent is an `agent.BatchedAgent` acting for that many environments at once through
+    `actors.BatchedActor` (ε-greedy on the device), to be driven by `environment_loop.BatchedEnvironmentLoop`."""
     table = replay.Table(
         name=replay.DEFAULT_PRIORITY_TABLE, sampler=replay.selectors.Prioritized(priority_exponent),
         remover=replay.selectors.Fifo(), max_size=max_replay_size,
@@ -1028,13 +1034,17 @@ class DQN(agent.Agent):
         frame_stack=frame_stack)
     self._server = replay.Server([table], port=None)
     address = f'localhost:{self._server.port}'
-    adder = adders.NStepTransitionAdder(client=replay.Client(address), n_step=n_step, discount=discount)
     replay_client = replay.TFClient(address)
     dataset = replay.make_reverb_dataset(server_address=address, batch_size=batch_size,
                                          prefetch_size=prefetch_size, seed=seed)
-    policy = actors.EpsilonGreedyPolicy(network, 0.05 if epsilon is None else epsilon, seed=seed)
+    epsilon = 0.05 if epsilon is None else epsilon
+    if num_envs > 1:
+      actor = actors.BatchedActor(actors.BatchedEpsilonGreedy(network, epsilon, seed=seed), table, num_envs, n_step,
+                                  use_cuda_graph=use_cuda_graph)
+    else:
+      adder = adders.NStepTransitionAdder(client=replay.Client(address), n_step=n_step, discount=discount)
+      actor = actors.FeedForwardActor(actors.EpsilonGreedyPolicy(network, epsilon, seed=seed), adder)
     target_network = network.clone()                 # deep-copied parameters (agent.py:127)
-    actor = actors.FeedForwardActor(policy, adder)
     learner = DQNLearner(network=network, target_network=target_network, discount=discount,
                          importance_sampling_exponent=importance_sampling_exponent,
                          learning_rate=learning_rate, target_update_period=target_update_period,

@@ -248,6 +248,42 @@ class Table:
   def reset(self):
     _capi.call('b200rl_replay_reset', self.handle, _capi.current_stream())
 
+  def open_writer(self) -> int:
+    """A new writer id on this table (`b200rl_writer_open`), for append_multi."""
+    w = C.c_int32()
+    _capi.call('b200rl_writer_open', self.handle, C.byref(w))
+    return w.value
+
+  def append_multi(self, writers, obs, act, reward, discount, first, last, n_step: int, priority: float = 1.0):
+    """One step of many episodes in one insert (`b200rl_writer_append_multi`): element i is the next timestep of writer
+    writers[i], with NStepTransitionAdder's items over `n_step` and raw priority `priority`.  obs: [n, *obs_shape] -- a
+    CUDA tensor is read on the device, anything else as host rows; act [n, *action_shape] (host), the action taken from
+    obs[i] (ignored where last[i]); reward / discount [n], what followed it; first / last [n] bools.  Only transition
+    tables without extras whose observation and action are single arrays."""
+    if self.is_sequence or self.has_extras or not (self.obs_packer.single and self.act_packer.single):
+      raise ValueError(f'table {self.name!r}: append_multi writes transition tables without extras whose observation '
+                       'and action are single arrays')
+    writers = np.ascontiguousarray(writers, np.int32)
+    n = writers.size
+    on_device = bool(getattr(obs, 'is_cuda', False))
+    if on_device:
+      if not obs.is_contiguous() or obs.numel() * obs.element_size() != n * self.obs_packer.nbytes:
+        raise ValueError(f'obs must be {n} contiguous rows of {self.obs_packer.nbytes} bytes')
+    else:
+      obs = np.ascontiguousarray(obs, self.obs_packer.leaves[0][1])
+      if obs.nbytes != n * self.obs_packer.nbytes:
+        raise ValueError(f'obs must be {n} rows of {self.obs_packer.nbytes} bytes')
+    act = np.ascontiguousarray(act, self.act_packer.leaves[0][1])
+    if act.nbytes != n * self.act_packer.nbytes:
+      raise ValueError(f'act must be {n} rows of {self.act_packer.nbytes} bytes')
+    rew = np.ascontiguousarray(reward, np.float32).reshape(n)
+    disc = np.ascontiguousarray(discount, np.float32).reshape(n)
+    first = np.ascontiguousarray(first, np.uint8).reshape(n)
+    last = np.ascontiguousarray(last, np.uint8).reshape(n)
+    _capi.call('b200rl_writer_append_multi', self.handle, n, writers.ctypes.data, _capi.ptr(obs), int(on_device),
+               act.ctypes.data, rew.ctypes.data, disc.ctypes.data, first.ctypes.data, last.ctypes.data, int(n_step),
+               float(priority), _capi.current_stream())
+
   def tree_levels(self):
     L, F, S = C.c_int32(), C.c_int32(), C.c_int32()
     _capi.call('b200rl_replay_tree_levels', self.handle, C.byref(L), C.byref(F), C.byref(S))

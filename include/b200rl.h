@@ -92,6 +92,15 @@ int b200rl_writer_append_stream(b200rl_replay* h, int32_t writer, int64_t n, con
                                 int obs_on_device, const void* act, const float* rew,
                                 const float* disc, const uint8_t* first, const uint8_t* last,
                                 int32_t n_step, double priority, void* stream);
+/* b200rl_writer_append_stream with a writer per element: element i belongs to writers[i] (one step of many episodes in
+ * one call, e.g. N environments stepped in lockstep).  A writer may appear several times; its elements are consecutive
+ * timesteps of its stream, processed in array order.  Per element everything is as in b200rl_writer_append_stream
+ * (FIRST / LAST, pending act / rew / disc, n-step item enumeration and drain, constant raw priority); element i's
+ * observation takes the i-th slot allocated by the call, so device observations still land in one or two D2D runs.
+ * Every writer id is checked before anything is changed. */
+int b200rl_writer_append_multi(b200rl_replay* h, int64_t n, const int32_t* writers, const void* obs, int obs_on_device,
+                               const void* act, const float* rew, const float* disc, const uint8_t* first,
+                               const uint8_t* last, int32_t n_step, double priority, void* stream);
 /* Make everything appended so far visible to sample/gather (H2D of staged slots + tree insert). */
 int b200rl_replay_flush(b200rl_replay* h, void* stream);
 
@@ -179,6 +188,27 @@ int b200rl_replay_set_weights(b200rl_replay* h, int64_t n, const float* weights_
 /* Philox4x32-10 uniforms in [0,1): out[i] = f(seed, *step_dev + step_offset, i). */
 int b200rl_uniform(float* out_dev, int32_t n, uint64_t seed, const int64_t* step_dev,
                    int64_t step_offset, void* stream);
+
+/* Exploration of the batched actor.  Both read the draw counter from device memory (a captured act step draws fresh
+ * numbers on every replay once the counter is advanced, e.g. by b200rl_step_increment) and draw
+ * u[i] = the i-th element b200rl_uniform(seed, counter_dev) would write.
+ *
+ * b200rl_epsilon_greedy: trfl.epsilon_greedy(q, epsilon).sample() for N rows of q (fp32, row stride ldq), this package's
+ * statement of trfl's distribution (epsilon / A on every action plus (1 - epsilon) / k on each of the k actions tied at
+ * the row maximum).  Row r draws u0 = u[2r], u1 = u[2r + 1]:
+ *   u0 < epsilon:  action = min(floor(fl(u1 * A)), A - 1)
+ *   otherwise:     action = the min(floor(fl(u1 * k)), k - 1)-th of the k actions equal to the row maximum, in index order.
+ * (The batch-1 EpsilonGreedyPolicy takes the first maximum; the two differ only on exact ties.)  u_out (nullable, [N][2])
+ * receives (u0, u1).  One warp per row.
+ *
+ * b200rl_gaussian_explore: the arithmetic of the Gaussian-noise behaviour policy, a, out, z_out f32 [N][A], lo / hi f32 [A]
+ * (the action spec's bounds): out = clip(fl(a + fl(z * sigma)), lo, hi), product and sum rounded separately (no FMA), as
+ * NumPy float32 does, with z[r][j] = sqrtf(-2 logf(1 - u[2m])) * cosf(fl(2 pi * u[2m + 1])), m = r * A + j (precise
+ * logf / cosf / sqrtf; 1 - u > 0 because the draws have 24 bits).  z_out (nullable) receives the noise.  out may alias a. */
+int b200rl_epsilon_greedy(int32_t N, int32_t A, const float* q, int64_t ldq, float epsilon, uint64_t seed,
+                          const int64_t* counter_dev, int32_t* actions_out, float* u_out, void* stream);
+int b200rl_gaussian_explore(int32_t N, int32_t A, const float* a, float sigma, const float* lo, const float* hi, uint64_t seed,
+                            const int64_t* counter_dev, float* out, float* z_out, void* stream);
 
 /* K4.  dqn/learning.py:127-154 + trfl.double_qlearning + losses/huber.py:48-57.
  * wmax_dev (nullable): device scalar (f64) holding the GLOBAL max importance weight for data-parallel
