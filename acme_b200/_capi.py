@@ -80,6 +80,10 @@ PROTOTYPES = {
     'b200rl_c51_loss': (c_int, [c_i32, c_i32, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_f32, c_f32,
                                 c_vp, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_td_learning': (c_int, [c_i32, c_vp, c_vp, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'b200rl_c51_loss_weighted': (c_int, [c_i32, c_i32, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_f32, c_vp, c_f64, c_vp, c_f32,
+                                         c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'b200rl_td_learning_weighted': (c_int, [c_i32, c_vp, c_vp, c_vp, c_vp, c_f32, c_vp, c_f64, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp,
+                                            c_vp, c_vp, c_vp]),
     'b200rl_c51_mean_fwd': (c_int, [c_i32, c_i32, c_f32, c_f32, c_vp, c_vp, c_vp]),
     'b200rl_c51_mean_bwd': (c_int, [c_i32, c_i32, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_dpg_action_grad': (c_int, [c_i32, c_i32, c_vp, c_f32, c_int, c_f32, c_vp, c_vp, c_vp, c_vp]),

@@ -120,6 +120,50 @@ dqn_td_kernel(int B, int A, const float* __restrict__ q_tm1, const float* __rest
 }
 
 // ------------------------------------------------------------------------------------------ K5
+// Prioritized form of the critic losses (b200rl_c51_loss_weighted / b200rl_td_learning_weighted): the kernels below are
+// templated on W.  W = false is the uniform loss; W = true adds, per sample, the importance weight of b200rl_dqn_td
+// (flags 0) against the precomputed batch maximum, the weighted loss, the priority and the weighted gradient, and the
+// batch mean of the weighted losses in the same launch: every warp that has written its samples' losses counts them on a
+// per-stream ticket, and the warp that brings the count to B adds loss_ps[0..B) in index order (lane l takes l, l + 32,
+// ... sequentially, then a fixed butterfly) and resets the ticket, so the mean is bit-identical across launches, streams
+// and graph replays.
+struct IsWeighted {
+  const float* prob;
+  double beta;
+  const double* wmax;
+  float* weight;
+  float* priority;
+  float* loss_mean;
+  int ticket;   // slot in g_loss_tickets
+  int B;
+};
+__device__ unsigned int g_loss_tickets[64];
+
+__device__ __forceinline__ float is_weight_of(const IsWeighted& iw, int b) {
+  return is_weight_norm(is_weight_raw(iw.prob[b], iw.beta, 0), *iw.wmax, 0);   // learning.py:138-143
+}
+
+// called by all 32 lanes of a warp after its `n` samples' loss_ps have been written (by any of its lanes)
+__device__ __forceinline__ void weighted_mean_tail(const IsWeighted& iw, const float* loss_ps, int n) {
+  const unsigned full = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  if (!iw.loss_mean || n == 0) return;
+  __threadfence();
+  __syncwarp();
+  unsigned int old = 0;
+  if (lane == 0) old = atomicAdd(&g_loss_tickets[iw.ticket], (unsigned int)n);
+  old = __shfl_sync(full, old, 0);
+  if (old + (unsigned int)n != (unsigned int)iw.B) return;
+  __threadfence();
+  float s = 0.f;
+  for (int i = lane; i < iw.B; i += 32) s = __fadd_rn(s, __ldcg(loss_ps + i));
+  for (int o = 16; o; o >>= 1) s = __fadd_rn(s, __shfl_xor_sync(full, s, o));
+  if (lane == 0) {
+    *iw.loss_mean = s / (float)iw.B;
+    g_loss_tickets[iw.ticket] = 0u;
+  }
+}
+
 // acme/tf/losses/distributional.py:22-83.  One CTA per sample; thread i owns atom i and evaluates
 // the dense projection row sum_j clip(1 - |clip(z'_j) - z_i| / delta_i, 0, 1) * p_j with p, z' in
 // shared memory -- the reference's arithmetic without materialising [B,K,K].
@@ -129,11 +173,12 @@ __device__ __forceinline__ float atom_value(int i, int K, float vmin, float vmax
   return (float)((double)vmin + (double)i * step);   // np.linspace(..., dtype=float32)
 }
 
+template <bool W>
 __global__ void c51_loss_kernel(int K, float vmin, float vmax, const float* __restrict__ logits_tm1,
                                 const float* __restrict__ logits_t, const float* __restrict__ R,
                                 const float* __restrict__ D, float gamma, float grad_scale,
                                 float* __restrict__ target_out, float* __restrict__ loss_ps,
-                                float* __restrict__ dlogits) {
+                                float* __restrict__ dlogits, IsWeighted iw) {
   pdl_launch_dependents();
   pdl_wait();
   extern __shared__ float sm[];
@@ -178,8 +223,20 @@ __global__ void c51_loss_kernel(int K, float vmin, float vmax, const float* __re
   float contrib = on ? -tgt * (l1 - lse) : 0.f;
   float loss = block_reduce(contrib, SumF(), 0.f, scratch);
   float tsum = block_reduce(tgt, SumF(), 0.f, scratch);
-  if (on && dlogits) dlogits[(size_t)b * K + i] = ((e1 / s1) * tsum - tgt) * grad_scale;
-  if (i == 0 && loss_ps) loss_ps[b] = loss;
+  if constexpr (W) {
+    const float w = is_weight_of(iw, b);
+    const float gs = __fmul_rn(w, grad_scale);
+    if (on && dlogits) dlogits[(size_t)b * K + i] = ((e1 / s1) * tsum - tgt) * gs;
+    if (i == 0) {
+      loss_ps[b] = __fmul_rn(loss, w);
+      iw.weight[b] = w;
+      iw.priority[b] = loss;
+    }
+    if (threadIdx.x < 32) weighted_mean_tail(iw, loss_ps, 1);
+  } else {
+    if (on && dlogits) dlogits[(size_t)b * K + i] = ((e1 / s1) * tsum - tgt) * grad_scale;
+    if (i == 0 && loss_ps) loss_ps[b] = loss;
+  }
 }
 
 // K5, K <= 64: ONE WARP per sample (lane owns atoms lane and lane + 32), no block barriers, and the projection row of
@@ -190,11 +247,12 @@ __global__ void c51_loss_kernel(int K, float vmin, float vmax, const float* __re
 // (dg < 0 -- never produced by the learners -- takes the dense loop).  At B = 65,536 the dense one-CTA-per-sample kernel
 // ran at 3 % of the HBM roofline, bound by 2,601 IEEE divisions per sample.
 constexpr int kC51WarpsPerCta = 8;
+template <bool W>
 __global__ void __launch_bounds__(32 * kC51WarpsPerCta)
 c51_loss_warp_kernel(int B, int K, float vmin, float vmax, const float* __restrict__ logits_tm1,
                      const float* __restrict__ logits_t, const float* __restrict__ R, const float* __restrict__ D,
                      float gamma, float grad_scale, float* __restrict__ target_out, float* __restrict__ loss_ps,
-                     float* __restrict__ dlogits) {
+                     float* __restrict__ dlogits, IsWeighted iw) {
   pdl_launch_dependents();
   pdl_wait();
   __shared__ float s_p[kC51WarpsPerCta][64], s_zc[kC51WarpsPerCta][64];
@@ -264,21 +322,54 @@ c51_loss_warp_kernel(int B, int K, float vmin, float vmax, const float* __restri
   const float lse = m1 + logf(s1);
   const float loss = wsum((on0 ? -t0 * (l0 - lse) : 0.f) + (on1 ? -t1 * (l1 - lse) : 0.f));
   const float tsum = wsum(t0 + t1);
-  if (dlogits) {
-    if (on0) dlogits[row + i0] = ((f0 / s1) * tsum - t0) * grad_scale;
-    if (on1) dlogits[row + i1] = ((f1 / s1) * tsum - t1) * grad_scale;
+  if constexpr (W) {
+    const float w = is_weight_of(iw, b);
+    const float gs = __fmul_rn(w, grad_scale);
+    if (dlogits) {
+      if (on0) dlogits[row + i0] = ((f0 / s1) * tsum - t0) * gs;
+      if (on1) dlogits[row + i1] = ((f1 / s1) * tsum - t1) * gs;
+    }
+    if (lane == 0) {
+      loss_ps[b] = __fmul_rn(loss, w);
+      iw.weight[b] = w;
+      iw.priority[b] = loss;                                          // the unweighted cross-entropy
+    }
+    weighted_mean_tail(iw, loss_ps, 1);
+  } else {
+    if (dlogits) {
+      if (on0) dlogits[row + i0] = ((f0 / s1) * tsum - t0) * grad_scale;
+      if (on1) dlogits[row + i1] = ((f1 / s1) * tsum - t1) * grad_scale;
+    }
+    if (lane == 0 && loss_ps) loss_ps[b] = loss;
   }
-  if (lane == 0 && loss_ps) loss_ps[b] = loss;
 }
 
 // trfl.td_learning as called at acme/agents/tf/ddpg/learning.py:193 (public trfl formula; trfl is not in the tree):
 // target = r + pcont * v_t (stop-gradient), td = target - v_tm1, loss = 0.5 td^2; d(mean loss)/d v_tm1 = -td / B.
+template <bool W>
 __global__ void td_learning_kernel(int B, const float* __restrict__ v_tm1, const float* __restrict__ v_t,
                                    const float* __restrict__ R, const float* __restrict__ D, float gamma, float grad_scale,
-                                   float* __restrict__ td_out, float* __restrict__ loss_ps, float* __restrict__ dv) {
+                                   float* __restrict__ td_out, float* __restrict__ loss_ps, float* __restrict__ dv,
+                                   IsWeighted iw) {
   pdl_launch_dependents();
   pdl_wait();
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if constexpr (W) {
+    // every lane stays for the warp's mean tail
+    if (b < B) {
+      const float pcont = __fmul_rn(gamma, D[b]);
+      const float target = __fadd_rn(R[b], __fmul_rn(pcont, v_t[b]));
+      const float td = __fsub_rn(target, v_tm1[b]);
+      const float w = is_weight_of(iw, b);
+      if (td_out) td_out[b] = td;
+      loss_ps[b] = __fmul_rn(__fmul_rn(0.5f, __fmul_rn(td, td)), w);
+      iw.weight[b] = w;
+      iw.priority[b] = fabsf(td);                                     // dqn/learning.py:152 (no epsilon)
+      if (dv) dv[b] = -td * __fmul_rn(w, grad_scale);
+    }
+    weighted_mean_tail(iw, loss_ps, __popc(__ballot_sync(0xffffffffu, b < B)));
+    return;
+  }
   if (b >= B) return;
   const float pcont = __fmul_rn(gamma, D[b]);                        // discount * d_t, learning.py:169,193
   const float target = __fadd_rn(R[b], __fmul_rn(pcont, v_t[b]));
@@ -1254,11 +1345,11 @@ extern "C" int b200rl_c51_loss(int32_t B, int32_t K, float vmin, float vmax, con
   B200RL_REQUIRE(B >= 1 && K >= 2 && K <= 1024, "bad shape");
   static const int dense_env = getenv("B200RL_C51_DENSE") ? atoi(getenv("B200RL_C51_DENSE")) : 0;
   if (K <= 64 && !dense_env) {
-    B200RL_CUDA_OK(launch_pdl_small(c51_loss_warp_kernel, dim3((B + kC51WarpsPerCta - 1) / kC51WarpsPerCta), dim3(32 * kC51WarpsPerCta), 0, as_stream(stream), B, K, vmin, vmax, logits_tm1, logits_t, R, D, gamma, grad_scale, target, loss_ps, dlogits));
+    B200RL_CUDA_OK(launch_pdl_small(c51_loss_warp_kernel<false>, dim3((B + kC51WarpsPerCta - 1) / kC51WarpsPerCta), dim3(32 * kC51WarpsPerCta), 0, as_stream(stream), B, K, vmin, vmax, logits_tm1, logits_t, R, D, gamma, grad_scale, target, loss_ps, dlogits, IsWeighted{}));
   } else {
     int threads = ((K + 31) / 32) * 32;
-    B200RL_CUDA_OK(launch_pdl_small(c51_loss_kernel, dim3(B), dim3(threads), 3 * K * sizeof(float), as_stream(stream), K, vmin, vmax, logits_tm1, logits_t, R, D, gamma,
-                                                                             grad_scale, target, loss_ps, dlogits));
+    B200RL_CUDA_OK(launch_pdl_small(c51_loss_kernel<false>, dim3(B), dim3(threads), 3 * K * sizeof(float), as_stream(stream), K, vmin, vmax, logits_tm1, logits_t, R, D, gamma,
+                                                                             grad_scale, target, loss_ps, dlogits, IsWeighted{}));
   }
   B200RL_LAUNCH_OK();
   if (loss_mean) {
@@ -1271,12 +1362,66 @@ extern "C" int b200rl_c51_loss(int32_t B, int32_t K, float vmin, float vmax, con
 extern "C" int b200rl_td_learning(int32_t B, const float* v_tm1, const float* v_t, const float* R, const float* D, float gamma,
                                   float grad_scale, float* td, float* loss_ps, float* dv_tm1, float* loss_mean, void* stream) {
   B200RL_REQUIRE(v_tm1 && v_t && R && D && loss_ps && B >= 1, "bad argument");
-  B200RL_CUDA_OK(launch_pdl_small(td_learning_kernel, dim3(ceil_div(B, 128)), dim3(128), 0, as_stream(stream), B, v_tm1, v_t, R, D, gamma, grad_scale, td, loss_ps, dv_tm1));
+  B200RL_CUDA_OK(launch_pdl_small(td_learning_kernel<false>, dim3(ceil_div(B, 128)), dim3(128), 0, as_stream(stream), B, v_tm1, v_t, R, D, gamma, grad_scale, td, loss_ps, dv_tm1, IsWeighted{}));
   B200RL_LAUNCH_OK();
   if (loss_mean) {
     B200RL_CUDA_OK(launch_pdl_small(mean_kernel, dim3(1), dim3(256), 0, as_stream(stream), loss_ps, B, loss_mean));
     B200RL_LAUNCH_OK();
   }
+  return B200RL_OK;
+}
+
+// the importance-weight arguments shared by the two weighted critic losses; fills `iw` (ticket: the stream's slot)
+static int weighted_args(int32_t B, const float* prob, double beta, const double* wmax_dev, float* loss_ps, float* weight,
+                         float* priority, float* loss_mean, cudaStream_t st, IsWeighted* iw) {
+  B200RL_REQUIRE(prob && wmax_dev && loss_ps && weight && priority, "null argument");
+  B200RL_REQUIRE(B >= 1, "bad shape");
+  B200RL_REQUIRE(beta >= 0.0, "importance_sampling_exponent must be >= 0");
+  int ticket = 0;
+  if (loss_mean) {
+    ticket = ticket_for(st);
+    B200RL_REQUIRE(ticket >= 0, "weighted critic loss: more than 64 streams");
+  }
+  *iw = IsWeighted{prob, beta, wmax_dev, weight, priority, loss_mean, ticket, B};
+  return B200RL_OK;
+}
+
+extern "C" int b200rl_c51_loss_weighted(int32_t B, int32_t K, float vmin, float vmax, const float* logits_tm1,
+                                        const float* logits_t, const float* R, const float* D, float gamma,
+                                        const float* prob, double is_exponent, const double* wmax_dev, float grad_scale,
+                                        float* target, float* loss_ps, float* weight, float* priority,
+                                        float* dlogits, float* loss_mean, void* stream) {
+  B200RL_REQUIRE(logits_tm1 && logits_t && R && D, "null argument");
+  B200RL_REQUIRE(K >= 2 && K <= 1024, "bad shape");
+  cudaStream_t st = as_stream(stream);
+  IsWeighted iw;
+  const int rc = weighted_args(B, prob, is_exponent, wmax_dev, loss_ps, weight, priority, loss_mean, st, &iw);
+  if (rc != B200RL_OK) return rc;
+  static const int dense_env = getenv("B200RL_C51_DENSE") ? atoi(getenv("B200RL_C51_DENSE")) : 0;
+  if (K <= 64 && !dense_env) {
+    B200RL_CUDA_OK(launch_pdl_small(c51_loss_warp_kernel<true>, dim3((B + kC51WarpsPerCta - 1) / kC51WarpsPerCta), dim3(32 * kC51WarpsPerCta), 0, st,
+                                    B, K, vmin, vmax, logits_tm1, logits_t, R, D, gamma, grad_scale, target, loss_ps, dlogits, iw));
+  } else {
+    int threads = ((K + 31) / 32) * 32;
+    B200RL_CUDA_OK(launch_pdl_small(c51_loss_kernel<true>, dim3(B), dim3(threads), 3 * K * sizeof(float), st, K, vmin, vmax, logits_tm1, logits_t,
+                                    R, D, gamma, grad_scale, target, loss_ps, dlogits, iw));
+  }
+  B200RL_LAUNCH_OK();
+  return B200RL_OK;
+}
+
+extern "C" int b200rl_td_learning_weighted(int32_t B, const float* v_tm1, const float* v_t, const float* R, const float* D,
+                                           float gamma, const float* prob, double is_exponent, const double* wmax_dev,
+                                           float grad_scale, float* td, float* loss_ps, float* weight, float* priority,
+                                           float* dv_tm1, float* loss_mean, void* stream) {
+  B200RL_REQUIRE(v_tm1 && v_t && R && D, "null argument");
+  cudaStream_t st = as_stream(stream);
+  IsWeighted iw;
+  const int rc = weighted_args(B, prob, is_exponent, wmax_dev, loss_ps, weight, priority, loss_mean, st, &iw);
+  if (rc != B200RL_OK) return rc;
+  B200RL_CUDA_OK(launch_pdl_small(td_learning_kernel<true>, dim3(ceil_div(B, 128)), dim3(128), 0, st, B, v_tm1, v_t, R, D, gamma, grad_scale,
+                                  td, loss_ps, dv_tm1, iw));
+  B200RL_LAUNCH_OK();
   return B200RL_OK;
 }
 

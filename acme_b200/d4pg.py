@@ -6,7 +6,16 @@
   policy(o_t) -> critic(o_t, a) -> d mean / d a -> K(dpg) norm-clipped action gradient -> policy
   backward -> global-norm clip (40) of each gradient set -> two Adams.
 The reference's D4PG has no importance weights and never writes priorities (uniform table,
-`d4pg/agent.py:96-103`); neither does this one.
+`d4pg/agent.py:96-103`); by default neither does this one.
+
+Prioritized replay is an opt-in extension (the D4PG paper evaluates the agent both ways).  With
+`importance_sampling_exponent` (beta) the learner computes the batch's maximum importance weight right after K1 (on the
+target chain's stream), and the critic loss becomes the importance-weighted mean, with the DQN learner's f64 weights
+w = (1 / prob)^beta / max_b (1 / prob)^beta (`dqn/learning.py:138-143`): mean(w * CE) for D4PG, mean(w * 0.5 td^2) for
+DDPG.  With a `replay_client` as well, K2 writes the new priorities back for the sampled keys inside the same step: the
+unweighted per-sample cross-entropy (D4PG) or |td| (DDPG).  Only the critic loss is weighted; the DPG policy loss stays
+unweighted.  The agents take `priority_exponent` and `importance_sampling_exponent` together to build such a learner on a
+`Prioritized` table.
 """
 
 from __future__ import annotations
@@ -27,12 +36,23 @@ class D4PGLearner(core.Learner, core.Saveable):
                discount: float, target_update_period: int, dataset: replay.ReplayDataset,
                policy_lr: float = 1e-4, critic_lr: float = 1e-4, clipping: bool = True,
                counter: counting.Counter = None, logger: loggers.Logger = None, checkpoint: bool = True,
-               eps_mode: int = 0, use_cuda_graph: bool = True, process_group=None):
+               eps_mode: int = 0, use_cuda_graph: bool = True, process_group=None,
+               importance_sampling_exponent: Optional[float] = None, replay_client: Optional[replay.Client] = None):
     """`process_group`: data-parallel learner over per-rank replay shards -- both gradient sets are all-reduced (mean) over
     NCCL between the gradient half and the optimizer half of the step, then clipped and applied identically on every rank
-    (the ordering of the reference's only multi-replica learner, `crr/recurrent_learning.py:346-359`)."""
+    (the ordering of the reference's only multi-replica learner, `crr/recurrent_learning.py:346-359`).
+    `importance_sampling_exponent`: importance-weighted critic loss for a prioritized table (module docstring);
+    `replay_client`: also write the new priorities back.  Both None: the reference's uniform, unweighted step."""
+    if replay_client is not None and importance_sampling_exponent is None:
+      raise ValueError('replay_client writes priorities for prioritized replay: it needs importance_sampling_exponent')
+    if importance_sampling_exponent is not None and process_group is not None:
+      raise ValueError('prioritized replay (importance_sampling_exponent) is not supported by the data-parallel learner')
+    if importance_sampling_exponent is not None and importance_sampling_exponent < 0:
+      raise ValueError('importance_sampling_exponent must be >= 0')
     import torch
     self._torch = torch
+    self._beta = None if importance_sampling_exponent is None else float(importance_sampling_exponent)
+    self._replay_client = replay_client
     self._dp = parallel.DataParallel(process_group)
     self._policy, self._critic = policy_network, critic_network
     self._tpolicy, self._tcritic = target_policy_network, target_critic_network
@@ -65,6 +85,9 @@ class D4PGLearner(core.Learner, core.Saveable):
     self._pm, self._pv = torch.zeros_like(policy_network.params.flat), torch.zeros_like(policy_network.params.flat)
     self._cm, self._cv = torch.zeros_like(critic_network.params.flat), torch.zeros_like(critic_network.params.flat)
     self._num_steps = torch.zeros(1, dtype=torch.int64, device=dev)
+    if self._beta is not None:
+      self.weight, self.priority = f32(B), f32(B)
+      self._wmax = torch.zeros(1, dtype=torch.float64, device=dev)
     self._norm_ws, self._norm_ws2 = f32(1024), f32(1024)
     self._pscale, self._cscale, self.policy_norm, self.critic_norm = f32(1), f32(1), f32(1), f32(1)
     self._loss_host = torch.zeros(2, dtype=torch.float32).pin_memory()
@@ -128,6 +151,8 @@ class D4PGLearner(core.Learner, core.Saveable):
     else:
       s1 = s2 = main
     with torch.cuda.stream(s1):
+      if self._beta is not None:    # joined before the critic loss with the target chain
+        _capi.call('b200rl_is_weight_max', B, _capi.ptr(ds.prob), self._beta, _capi.ptr(self._wmax), 0, _capi.current_stream())
       a_targ = TP.lane(1).action(o1, self._p_tgt)
       logits_t = TC.lane(1).logits(o1, a_targ, self._c_tgt)
       if fork:
@@ -153,16 +178,35 @@ class D4PGLearner(core.Learner, core.Saveable):
     if fork:
       main.wait_event(tgt_done)
     self._critic_loss(logits_tm1, logits_t)
+    k2_done = None
+    if self._replay_client is not None:   # K2 (learning.py:151-154) beside the critic backward; the next K1 reads the tree
+      if fork:
+        ev = torch.cuda.Event()
+        ev.record(main)
+        s1.wait_event(ev)
+      with torch.cuda.stream(s1):
+        ds.table.update_priorities_device(ds.keys, self.priority)
+        if fork:
+          k2_done = torch.cuda.Event()
+          k2_done.record(s1)
     C.backward_flat(self._c_train['x'].data_ptr(), self._c_train, self._cg_train, self.dlogits.data_ptr(),
                     param_grads=True, input_grad=False)
     if fork:
       main.wait_event(pi_done)
+      if k2_done is not None:
+        main.wait_event(k2_done)
     for net in (P, C, TP, TC):
       net.lane(0)
 
   def _critic_loss(self, logits_tm1, logits_t):
     """K5: losses.categorical (distributional.py:22-37) and its gradient w.r.t. logits_tm1 (learning.py:202-203)."""
     C, ds, B = self._critic, self._dataset, self.B
+    if self._beta is not None:   # importance-weighted; priority = the unweighted per-sample cross-entropy
+      _capi.call('b200rl_c51_loss_weighted', B, C.K, C.vmin, C.vmax, _capi.ptr(logits_tm1), _capi.ptr(logits_t), _capi.ptr(ds.R),
+                 _capi.ptr(ds.D), self._discount, _capi.ptr(ds.prob), self._beta, _capi.ptr(self._wmax), 1.0 / B,
+                 _capi.ptr(self.target), _capi.ptr(self.critic_loss_ps), _capi.ptr(self.weight), _capi.ptr(self.priority),
+                 _capi.ptr(self.dlogits), _capi.ptr(self.critic_loss), _capi.current_stream())
+      return
     _capi.call('b200rl_c51_loss', B, C.K, C.vmin, C.vmax, _capi.ptr(logits_tm1), _capi.ptr(logits_t), _capi.ptr(ds.R),
                _capi.ptr(ds.D), self._discount, 1.0 / B, _capi.ptr(self.target), _capi.ptr(self.critic_loss_ps),
                _capi.ptr(self.dlogits), _capi.ptr(self.critic_loss), _capi.current_stream())
@@ -306,6 +350,12 @@ class DDPGLearner(D4PGLearner):
 
   def _critic_loss(self, q_tm1, q_t):
     ds, B = self._dataset, self.B
+    if self._beta is not None:   # importance-weighted; priority = |td|
+      _capi.call('b200rl_td_learning_weighted', B, _capi.ptr(q_tm1), _capi.ptr(q_t), _capi.ptr(ds.R), _capi.ptr(ds.D),
+                 self._discount, _capi.ptr(ds.prob), self._beta, _capi.ptr(self._wmax), 1.0 / B, _capi.ptr(self.td),
+                 _capi.ptr(self.critic_loss_ps), _capi.ptr(self.weight), _capi.ptr(self.priority), _capi.ptr(self.dlogits),
+                 _capi.ptr(self.critic_loss), _capi.current_stream())
+      return
     _capi.call('b200rl_td_learning', B, _capi.ptr(q_tm1), _capi.ptr(q_t), _capi.ptr(ds.R), _capi.ptr(ds.D), self._discount,
                1.0 / B, _capi.ptr(self.td), _capi.ptr(self.critic_loss_ps), _capi.ptr(self.dlogits), _capi.ptr(self.critic_loss),
                _capi.current_stream())
@@ -332,7 +382,10 @@ class GaussianNoisePolicy:
 
 
 class D4PG(agent.Agent):
-  """`acme/agents/tf/d4pg/agent.py:36-180`: uniform table, n-step adder, dataset, actor, learner."""
+  """`acme/agents/tf/d4pg/agent.py:36-180`: uniform table, n-step adder, dataset, actor, learner.  With
+  `priority_exponent` (alpha) and `importance_sampling_exponent` (beta), given together, the table is
+  `Prioritized(alpha)` and the learner weights its critic loss and writes priorities back (`D4PGLearner`); new items
+  enter with priority 1.0, as the reference adder's constant `priority_fns` gives them."""
 
   _learner_cls = D4PGLearner
 
@@ -344,10 +397,16 @@ class D4PG(agent.Agent):
                prefetch_size: int = 4, target_update_period: int = 100, min_replay_size: int = 1000,
                max_replay_size: int = 1000000, samples_per_insert: float = 32.0, n_step: int = 5,
                sigma: float = 0.3, clipping: bool = True, logger: loggers.Logger = None, checkpoint: bool = False,
-               seed: int = 0, use_cuda_graph: bool = True, num_envs: int = 1):
+               seed: int = 0, use_cuda_graph: bool = True, num_envs: int = 1,
+               priority_exponent: Optional[float] = None, importance_sampling_exponent: Optional[float] = None):
     """num_envs > 1: the agent is an `agent.BatchedAgent` acting for that many environments at once through
-    `actors.BatchedActor` (Gaussian exploration on the device), to be driven by `environment_loop.BatchedEnvironmentLoop`."""
-    table = replay.Table(name=replay.DEFAULT_PRIORITY_TABLE, sampler=replay.selectors.Uniform(),
+    `actors.BatchedActor` (Gaussian exploration on the device), to be driven by `environment_loop.BatchedEnvironmentLoop`.
+    priority_exponent / importance_sampling_exponent: prioritized replay (both or neither; the default is uniform)."""
+    if (priority_exponent is None) != (importance_sampling_exponent is None):
+      raise ValueError('prioritized replay needs both priority_exponent and importance_sampling_exponent')
+    prioritized = priority_exponent is not None
+    sampler = replay.selectors.Prioritized(priority_exponent) if prioritized else replay.selectors.Uniform()
+    table = replay.Table(name=replay.DEFAULT_PRIORITY_TABLE, sampler=sampler,
                          remover=replay.selectors.Fifo(), max_size=max_replay_size,
                          rate_limiter=replay.rate_limiters.MinSize(1),
                          signature=adders.NStepTransitionAdder.signature(environment_spec), max_window=n_step,
@@ -366,7 +425,8 @@ class D4PG(agent.Agent):
       actor = actors.FeedForwardActor(GaussianNoisePolicy(policy_network, sigma, aspec.minimum, aspec.maximum, seed), adder)
     learner = self._learner_cls(policy_network, critic_network, policy_network.clone(), critic_network.clone(), discount,
                                 target_update_period, dataset, clipping=clipping, logger=logger, checkpoint=checkpoint,
-                                use_cuda_graph=use_cuda_graph)
+                                use_cuda_graph=use_cuda_graph, importance_sampling_exponent=importance_sampling_exponent,
+                                replay_client=replay.TFClient(address) if prioritized else None)
     self._table = table
     super().__init__(actor=actor, learner=learner, min_observations=max(batch_size, min_replay_size),
                      observations_per_step=float(batch_size) / samples_per_insert)

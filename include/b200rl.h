@@ -243,6 +243,33 @@ int b200rl_c51_loss(int32_t B, int32_t K, float vmin, float vmax, const float* l
  * loss = 0.5 td^2, dv_tm1 = -td * grad_scale.  td, dv_tm1, loss_mean nullable. */
 int b200rl_td_learning(int32_t B, const float* v_tm1, const float* v_t, const float* R, const float* D, float gamma,
                        float grad_scale, float* td, float* loss_per_sample, float* dv_tm1, float* loss_mean, void* stream);
+/* The two critic losses above for prioritized replay (D4PG / DDPG with importance_sampling_exponent): only the critic loss
+ * is weighted; the DPG policy loss stays unweighted.  Per sample b, with w_b the importance weight of b200rl_dqn_td
+ * (flags 0), bit for bit:
+ *   w_b = (float)(pow(1.0 / (double)prob[b], is_exponent) / *wmax_dev)         (dqn/learning.py:138-143)
+ * wmax_dev is REQUIRED: the batch maximum of pow(1 / prob, is_exponent), written by b200rl_is_weight_max after sampling.
+ *   C51:  target and the unweighted cross-entropy ce_b with the arithmetic of b200rl_c51_loss (the same one-warp form for
+ *         K <= 64 and dense form above), then
+ *         loss_per_sample[b] = fl(ce_b * w_b),  priority[b] = ce_b,
+ *         dlogits[b][i] = (softmax(logits_tm1)_i * sum(target_b) - target_b,i) * fl(w_b * grad_scale)
+ *   TD:   td as b200rl_td_learning, then
+ *         loss_per_sample[b] = fl(fl(0.5 td^2) * w_b),  priority[b] = |td| (no epsilon, dqn/learning.py:152),
+ *         dv_tm1[b] = -td * fl(w_b * grad_scale)
+ * weight[b] = w_b.  With every w_b == 1 every output but loss_mean is bit-identical to the unweighted entry point's.
+ * loss_mean (nullable) = fl(sum_b loss_per_sample[b]) / B, summed in a fixed order inside the same launch (the warp that
+ * finishes last adds the per-sample losses in index order, found by a per-stream ticket that is reset on exit): ONE launch
+ * per call, bit-identical across launches, streams and CUDA-graph replay.  target, td, dlogits_tm1, dv_tm1 nullable.
+ * EINVAL without a launch: null prob, wmax_dev, loss_per_sample, weight or priority; B < 1; K outside [2, 1024];
+ * is_exponent < 0. */
+int b200rl_c51_loss_weighted(int32_t B, int32_t K, float vmin, float vmax, const float* logits_tm1,
+                             const float* logits_t, const float* R, const float* D, float gamma,
+                             const float* prob, double is_exponent, const double* wmax_dev, float grad_scale,
+                             float* target, float* loss_per_sample, float* weight, float* priority,
+                             float* dlogits_tm1, float* loss_mean, void* stream);
+int b200rl_td_learning_weighted(int32_t B, const float* v_tm1, const float* v_t, const float* R, const float* D,
+                                float gamma, const float* prob, double is_exponent, const double* wmax_dev,
+                                float grad_scale, float* td, float* loss_per_sample, float* weight, float* priority,
+                                float* dv_tm1, float* loss_mean, void* stream);
 /* mean of a discrete-valued distribution and its logit gradient (distributions.py:64-66):
  * q = sum softmax(l)_i z_i;  dlogits_i = p_i (z_i - q) * dq. */
 int b200rl_c51_mean_fwd(int32_t B, int32_t K, float vmin, float vmax, const float* logits, float* q,

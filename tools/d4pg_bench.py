@@ -1,12 +1,16 @@
 """D4PG learner updates/s on the control-suite-humanoid shape (67-d obs, 21-d act, C51 critic), batch 256, n=5
 (BASELINE.json configs[2]); device-resident timing with CUDA events, whole step as a CUDA graph.
 
-  python tools/d4pg_bench.py --precision tf32,bf16 --steps 300 --reps 3 [--out DIR]
+  python tools/d4pg_bench.py --precision tf32,bf16 [--replay uniform,prioritized] --steps 300 --reps 3 [--out DIR]
 
 Several precisions (fp32 = 0, tf32 = 1, bf16 = 2, the network `precision` modes) are timed in one process, alternating
 per repetition, so that they share the GPU's state.  Each line reports ms per step for every repetition, kernel launches
 per eager step (`b200rl_launch_count`), and the GPU's name and power limit read in the same run.  `bench.py --workload
-d4pg` keeps measuring precision 1."""
+d4pg` keeps measuring precision 1.
+
+`--replay prioritized` adds the opt-in prioritized learner (a Prioritized(0.6) table, importance_sampling_exponent 0.4,
+priorities written back every step) beside the uniform one; the two arms read separate tables with identical contents
+and alternate with the precisions.  Its results go to d4pg_bench_<precision>_prioritized.json."""
 import argparse
 import json
 import os
@@ -33,11 +37,14 @@ def gpu_info():
   return name, limit
 
 
-def fill_table(OBS, ACT, n, items):
+ALPHA, BETA = 0.6, 0.4
+
+
+def fill_table(OBS, ACT, n, items, sampler=None):
   rng = np.random.default_rng(0)
   spec = specs.EnvironmentSpec(specs.Array((OBS,), np.float32), specs.BoundedArray((ACT,), np.float32, -1., 1.),
                                specs.Array((), np.float32), specs.BoundedArray((), np.float32, 0., 1.))
-  table = replay.Table(replay.DEFAULT_PRIORITY_TABLE, replay.selectors.Uniform(), replay.selectors.Fifo(), max_size=items,
+  table = replay.Table(replay.DEFAULT_PRIORITY_TABLE, sampler or replay.selectors.Uniform(), replay.selectors.Fifo(), max_size=items,
                        rate_limiter=replay.rate_limiters.MinSize(1), signature=adders.NStepTransitionAdder.signature(spec),
                        max_window=n, discount=0.99, stage_slots=4096)
   server = replay.Server([table])
@@ -58,35 +65,46 @@ def fill_table(OBS, ACT, n, items):
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--precision', default='tf32', help='comma-separated subset of fp32, tf32, bf16')
+  ap.add_argument('--replay', default='uniform', help='comma-separated subset of uniform, prioritized')
   ap.add_argument('--steps', type=int, default=300, help='timed updates per repetition')
   ap.add_argument('--warmup', type=int, default=20)
   ap.add_argument('--reps', type=int, default=3)
   ap.add_argument('--out', default=None, help='directory for d4pg_bench_<precision>.json')
   args = ap.parse_args()
-  names = [p.strip() for p in args.precision.split(',') if p.strip()]
-  for p in names:
+  precisions = [p.strip() for p in args.precision.split(',') if p.strip()]
+  for p in precisions:
     if p not in PRECISIONS:
       ap.error(f'unknown precision {p!r} (fp32, tf32, bf16)')
+  arms = [r.strip() for r in args.replay.split(',') if r.strip()]
+  for r in arms:
+    if r not in ('uniform', 'prioritized'):
+      ap.error(f'unknown replay {r!r} (uniform, prioritized)')
+  # one run per (precision, replay); a uniform run keeps the name it always had
+  names = [p if r == 'uniform' else f'{p}_{r}' for p in precisions for r in arms]
   B, OBS, ACT, n = 256, 67, 21, 5
-  table, server = fill_table(OBS, ACT, n, 100_000)
+  tables = {r: fill_table(OBS, ACT, n, 100_000, replay.selectors.Prioritized(ALPHA) if r == 'prioritized' else None)
+            for r in arms}
   lib = _capi.load()
   learners, launches = {}, {}
-  for p in names:
+  for name in names:
+    p, prio = name.split('_')[0], name.endswith('_prioritized')
+    table, server = tables['prioritized' if prio else 'uniform']
     policy = networks.D4PGPolicy(OBS, ACT, seed=1, precision=PRECISIONS[p])
     critic = networks.D4PGCritic(OBS, ACT, seed=2, precision=PRECISIONS[p])
     ds = replay.ReplayDataset(table, B, seed=11, stratified=False)
+    extra = dict(importance_sampling_exponent=BETA, replay_client=replay.Client(server)) if prio else {}
     L = d4pg.D4PGLearner(policy, critic, policy.clone(), critic.clone(), 0.99, target_update_period=100, dataset=ds,
-                         logger=loggers.NoOpLogger())
+                         logger=loggers.NoOpLogger(), **extra)
     L.step(fetch_loss=False)
     torch.cuda.synchronize()
     n0 = lib.b200rl_launch_count()
     L.step(fetch_loss=False)          # the second update is still eager; the graph is captured at the third
     torch.cuda.synchronize()
-    launches[p] = int(lib.b200rl_launch_count() - n0)
+    launches[name] = int(lib.b200rl_launch_count() - n0)
     for _ in range(args.warmup):
       L.step(fetch_loss=False)
     torch.cuda.synchronize()
-    learners[p] = L
+    learners[name] = L
   ms = {p: [] for p in names}
   e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
   for _ in range(args.reps):
@@ -100,17 +118,24 @@ def main():
       torch.cuda.synchronize()
       ms[p].append(e0.elapsed_time(e1) / args.steps)
   gpu, power_limit = gpu_info()
-  for p in names:
-    med = float(np.median(ms[p]))
+  for name in names:
+    p = name.split('_')[0]
+    med = float(np.median(ms[name]))
     out = {'workload': 'D4PG humanoid-shaped 67/21, C51 (51 atoms), batch 256, n=5', 'precision': p,
-           'precision_mode': PRECISIONS[p], 'steps_per_rep': args.steps, 'ms_per_step_reps': ms[p], 'ms_per_step': med,
-           'updates_per_s': 1e3 / med, 'launches_per_eager_step': launches[p], 'gpu': gpu, 'power_limit': power_limit}
+           'precision_mode': PRECISIONS[p], 'steps_per_rep': args.steps, 'ms_per_step_reps': ms[name], 'ms_per_step': med,
+           'updates_per_s': 1e3 / med, 'launches_per_eager_step': launches[name], 'gpu': gpu, 'power_limit': power_limit}
+    if name.endswith('_prioritized'):
+      out.update(replay=f'prioritized (alpha {ALPHA}, importance_sampling_exponent {BETA}, priorities written back)',
+                 items=100_000)
+      if p in ms:   # the uniform arm of the same run
+        out.update(uniform_ms_per_step=float(np.median(ms[p])), uniform_launches_per_eager_step=launches[p])
     print(json.dumps(out))
     if args.out:
       os.makedirs(args.out, exist_ok=True)
-      with open(os.path.join(args.out, f'd4pg_bench_{p}.json'), 'w') as f:
+      with open(os.path.join(args.out, f'd4pg_bench_{name}.json'), 'w') as f:
         json.dump(out, f, indent=1)
-  server.stop()
+  for _, server in tables.values():
+    server.stop()
 
 
 if __name__ == '__main__':
