@@ -89,8 +89,6 @@ PROTOTYPES = {
     'b200rl_dpg_action_grad': (c_int, [c_i32, c_i32, c_vp, c_f32, c_int, c_f32, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_adam': (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_f32, c_f64, c_f64, c_f32, c_int,
                             c_vp, c_vp, c_vp]),
-    'b200rl_adam_throttled': (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_f32, c_f64, c_f64, c_f32, c_int,
-                                      c_vp, c_vp, c_i32, c_vp]),
     'b200rl_learner_tail': (c_int, [c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp]),
     'b200rl_global_norm_scale': (c_int, [c_i64, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_copy_if_period': (c_int, [c_i64, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp]),

@@ -476,13 +476,8 @@ __device__ __forceinline__ float adam_one(float& p, float g, float& m, float& v,
 }
 // 8 elements (two float4 per array = 8 independent 16-byte loads) per thread per iteration: enough bytes in
 // flight to run at HBM speed; p/m/v are read-modify-write, g is read once (streamed through the read-only path).
-// VPT = float4 vectors per array per thread per iteration: 2 for the full-occupancy launch, 4 for launches limited to a
-// few CTAs per SM (an update running beside other kernels): fewer threads, the same bytes in flight.
-// CS: p / g / m / v move with the cache-streaming policy (ld.global.cs / st.global.cs, evict-first): the update touches
-// 225 MB once per step, more than the L2 holds, so keeping its lines only evicts what the network kernels running beside
-// (or right after) it still want -- activations, the bf16 weight shadow (written with the default policy: the next
-// forward reads it).
-template <int VPT, bool CS>
+// Measured on B200: four float4 per array per thread is SLOWER (0.347 vs 0.318 ms per step at full occupancy, no gain
+// beside other kernels): the extra registers per thread cost more than the extra loads in flight bring.
 __global__ void __launch_bounds__(256)
 adam_kernel(long long n, float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
             float* __restrict__ v, const long long* __restrict__ step_dev, float lr, double b1,
@@ -503,7 +498,7 @@ adam_kernel(long long n, float* __restrict__ p, const float* __restrict__ g, flo
   c.b1f = (float)b1; c.b2f = (float)b2; c.omb1 = (float)(1.0 - b1); c.omb2 = (float)(1.0 - b2);
   c.gs = gscale_dev ? *gscale_dev : 1.f;
   c.k1 = sqrtf(c.bc2) / c.bc1; c.lr = lr; c.eps = eps; c.eps_mode = eps_mode;
-  constexpr int EPT = 4 * VPT;                       // elements per thread per iteration
+  constexpr int VPT = 2, EPT = 4 * VPT;              // float4 vectors / elements per array per thread per iteration
   const long long n8 = n - n % EPT;
   long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * EPT;
   const long long stride = (long long)gridDim.x * blockDim.x * EPT;
@@ -511,17 +506,10 @@ adam_kernel(long long n, float* __restrict__ p, const float* __restrict__ g, flo
     float4 pq[VPT], gq[VPT], mq[VPT], vq[VPT];
 #pragma unroll
     for (int h = 0; h < VPT; ++h) {
-      if (CS) {
-        pq[h] = __ldcs(reinterpret_cast<const float4*>(p + i + 4 * h));
-        gq[h] = __ldcs(reinterpret_cast<const float4*>(g + i + 4 * h));
-        mq[h] = __ldcs(reinterpret_cast<const float4*>(m + i + 4 * h));
-        vq[h] = __ldcs(reinterpret_cast<const float4*>(v + i + 4 * h));
-      } else {
-        pq[h] = *reinterpret_cast<const float4*>(p + i + 4 * h);
-        gq[h] = __ldg(reinterpret_cast<const float4*>(g + i + 4 * h));
-        mq[h] = *reinterpret_cast<const float4*>(m + i + 4 * h);
-        vq[h] = *reinterpret_cast<const float4*>(v + i + 4 * h);
-      }
+      pq[h] = *reinterpret_cast<const float4*>(p + i + 4 * h);
+      gq[h] = __ldg(reinterpret_cast<const float4*>(g + i + 4 * h));
+      mq[h] = *reinterpret_cast<const float4*>(m + i + 4 * h);
+      vq[h] = *reinterpret_cast<const float4*>(v + i + 4 * h);
     }
 #pragma unroll
     for (int h = 0; h < VPT; ++h) {
@@ -529,26 +517,17 @@ adam_kernel(long long n, float* __restrict__ p, const float* __restrict__ g, flo
       adam_one(pq[h].y, gq[h].y, mq[h].y, vq[h].y, c);
       adam_one(pq[h].z, gq[h].z, mq[h].z, vq[h].z, c);
       adam_one(pq[h].w, gq[h].w, mq[h].w, vq[h].w, c);
-      if (CS) {
-        __stcs(reinterpret_cast<float4*>(p + i + 4 * h), pq[h]);
-        __stcs(reinterpret_cast<float4*>(m + i + 4 * h), mq[h]);
-        __stcs(reinterpret_cast<float4*>(v + i + 4 * h), vq[h]);
-      } else {
-        *reinterpret_cast<float4*>(p + i + 4 * h) = pq[h];
-        *reinterpret_cast<float4*>(m + i + 4 * h) = mq[h];
-        *reinterpret_cast<float4*>(v + i + 4 * h) = vq[h];
-      }
+      *reinterpret_cast<float4*>(p + i + 4 * h) = pq[h];
+      *reinterpret_cast<float4*>(m + i + 4 * h) = mq[h];
+      *reinterpret_cast<float4*>(v + i + 4 * h) = vq[h];
     }
     if (shadow) {
-#pragma unroll
-      for (int h = 0; h < VPT; h += 2) {
-        uint4 pk;
-        __nv_bfloat162 t0 = __floats2bfloat162_rn(pq[h].x, pq[h].y), t1 = __floats2bfloat162_rn(pq[h].z, pq[h].w);
-        __nv_bfloat162 t2 = __floats2bfloat162_rn(pq[h + 1].x, pq[h + 1].y), t3 = __floats2bfloat162_rn(pq[h + 1].z, pq[h + 1].w);
-        pk.x = *reinterpret_cast<uint32_t*>(&t0); pk.y = *reinterpret_cast<uint32_t*>(&t1);
-        pk.z = *reinterpret_cast<uint32_t*>(&t2); pk.w = *reinterpret_cast<uint32_t*>(&t3);
-        *reinterpret_cast<uint4*>(shadow + i + 4 * h) = pk;
-      }
+      uint4 pk;
+      __nv_bfloat162 t0 = __floats2bfloat162_rn(pq[0].x, pq[0].y), t1 = __floats2bfloat162_rn(pq[0].z, pq[0].w);
+      __nv_bfloat162 t2 = __floats2bfloat162_rn(pq[1].x, pq[1].y), t3 = __floats2bfloat162_rn(pq[1].z, pq[1].w);
+      pk.x = *reinterpret_cast<uint32_t*>(&t0); pk.y = *reinterpret_cast<uint32_t*>(&t1);
+      pk.z = *reinterpret_cast<uint32_t*>(&t2); pk.w = *reinterpret_cast<uint32_t*>(&t3);
+      *reinterpret_cast<uint4*>(shadow + i) = pk;
     }
   }
   if (blockIdx.x == 0 && threadIdx.x < (int)(n - n8)) {   // ragged tail (< EPT elements)
@@ -1463,44 +1442,17 @@ extern "C" int b200rl_debug_stamp(unsigned long long* buf, int slot, void* strea
   return cudaGetLastError() == cudaSuccess ? 0 : -2;
 }
 
-extern "C" int b200rl_adam_throttled(int64_t n, float* param, const float* grad, float* m, float* v, const int64_t* step_dev,
-                                     float lr, double b1, double b2, float eps, int eps_mode, const float* grad_scale_dev,
-                                     void* bf16_shadow, int32_t ctas_per_sm, void* stream);
-#define ADAM_CS_DEFAULT 0   // 1 once measured faster on B200 (gpurun_out/c2_*)
 extern "C" int b200rl_adam(int64_t n, float* param, const float* grad, float* m, float* v, const int64_t* step_dev,
                            float lr, double b1, double b2, float eps, int eps_mode, const float* grad_scale_dev,
                            void* bf16_shadow, void* stream) {
-  return b200rl_adam_throttled(n, param, grad, m, v, step_dev, lr, b1, b2, eps, eps_mode, grad_scale_dev, bf16_shadow, 0, stream);
-}
-// ctas_per_sm > 0 limits the grid to that many CTAs per SM: an update that runs BESIDE other kernels (the fc1 + head
-// bucket under the convolution backward) must leave them SM slots; 0 = the default (8, or B200RL_ADAM_CTAS_PER_SM)
-extern "C" int b200rl_adam_throttled(int64_t n, float* param, const float* grad, float* m, float* v, const int64_t* step_dev,
-                                     float lr, double b1, double b2, float eps, int eps_mode, const float* grad_scale_dev,
-                                     void* bf16_shadow, int32_t ctas_per_sm, void* stream) {
   B200RL_REQUIRE(param && grad && m && v && step_dev, "null argument");
   B200RL_REQUIRE(n >= 0 && (eps_mode == 0 || eps_mode == 1), "bad argument");
   B200RL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)m | (uintptr_t)v) & 15) == 0, "buffers must be 16-byte aligned");
   if (n == 0) return B200RL_OK;
-  static const int per_sm_env = getenv("B200RL_ADAM_CTAS_PER_SM") ? atoi(getenv("B200RL_ADAM_CTAS_PER_SM")) : 8;   // 0 = one pass, no loop
-  const int per_sm = ctas_per_sm > 0 ? ctas_per_sm : per_sm_env;
-  static const int wide = getenv("B200RL_ADAM_WIDE") ? atoi(getenv("B200RL_ADAM_WIDE")) : -1;                 // -1 = by CTA count
-  // measured on B200: the 4-vector variant is SLOWER (0.347 vs 0.318 ms per step at full occupancy, no gain beside other
-  // kernels): more registers per thread cost more than the extra loads in flight bring.  Kept behind B200RL_ADAM_WIDE=1.
-  const bool use_wide = wide > 0;
-  static const int cs = getenv("B200RL_ADAM_CS") ? atoi(getenv("B200RL_ADAM_CS")) : ADAM_CS_DEFAULT;   // cache-streaming accesses
-  if (use_wide) {
-    int blocks = grid1d((n + 15) / 16, 256, per_sm > 0 ? kNumSMs * per_sm : (1 << 30));
-    adam_kernel<4, false><<<blocks, 256, 0, as_stream(stream)>>>(n, param, grad, m, v, (const long long*)step_dev, lr, b1, b2, eps,
-                                                                eps_mode, grad_scale_dev, (__nv_bfloat16*)bf16_shadow);
-  } else {
-    int blocks = grid1d((n + 7) / 8, 256, per_sm > 0 ? kNumSMs * per_sm : (1 << 30));
-    if (cs)
-      B200RL_CUDA_OK(launch_pdl(adam_kernel<2, true>, dim3(blocks), dim3(256), 0, as_stream(stream), n, param, grad, m, v, (const long long*)step_dev, lr, b1, b2, eps,
-                                                                 eps_mode, grad_scale_dev, (__nv_bfloat16*)bf16_shadow));
-    else
-      B200RL_CUDA_OK(launch_pdl(adam_kernel<2, false>, dim3(blocks), dim3(256), 0, as_stream(stream), n, param, grad, m, v, (const long long*)step_dev, lr, b1, b2, eps,
-                                                                  eps_mode, grad_scale_dev, (__nv_bfloat16*)bf16_shadow));
-  }
+  const int blocks = grid1d((n + 7) / 8, 256, kNumSMs * 8);   // 8 CTAs per SM, grid-stride loop beyond that
+  B200RL_CUDA_OK(launch_pdl(adam_kernel, dim3(blocks), dim3(256), 0, as_stream(stream), n, param, grad, m, v,
+                            (const long long*)step_dev, lr, b1, b2, eps, eps_mode, grad_scale_dev,
+                            (__nv_bfloat16*)bf16_shadow));
   B200RL_LAUNCH_OK();
   return B200RL_OK;
 }

@@ -23,8 +23,6 @@ from acme_b200 import _capi, actors, adders, agent, core, counting, loggers, net
 
 # Single-GPU pipelined update (see DQNLearner.__init__): '1' once measured faster than the one-graph serial step.
 PIPELINE_1GPU_DEFAULT = '0'
-STREAM_PRIO_DEFAULT = '0'
-K2_EARLY_DEFAULT = '1'      # measured: 0.298 -> 0.289 ms per step (gpurun_out/c3_bench_k2early.json)
 
 
 class DQNLearner(core.Learner, core.Saveable):
@@ -75,7 +73,7 @@ class DQNLearner(core.Learner, core.Saveable):
     # Fused path (networks with a duelling head and features(): DQNAtariNetwork): the two online forwards
     # (learning.py:123,125) run as ONE pass over the 2B frames [o_tm1; o_t] (fc1's weights are read once, half the
     # launches), and the three heads + K4 + the head's data gradient are one kernel (b200rl_dqn_head_td).
-    self._fused = (hasattr(network, 'features') and A <= 32 and os.environ.get('B200RL_FUSED_HEAD', '1') != '0')
+    self._fused = hasattr(network, 'features') and A <= 32
     if self._fused:
       self._bufs_on = network.make_buffers(2 * B)                 # rows [0, B) = o_tm1, rows [B, 2B) = o_t
       self._bufs_train = dict(self._bufs_on, B=B)                 # the same storage seen as the o_tm1 batch (backward)
@@ -104,32 +102,14 @@ class DQNLearner(core.Learner, core.Saveable):
     self._use_graph = bool(use_cuda_graph)
     # the three forward passes are independent, and so are a layer's weight- and data-gradient: run them on
     # parallel streams (fork/join with events, also inside the captured graph)
-    self._concurrent = bool(concurrent_streams) and hasattr(network, '_backward_two_streams')
-    # Adam on the fc1 + head bucket underneath the convolution backward: measured zero-sum on B200 (the update streams
-    # 200 MB and takes the SM slots the latency-bound conv kernels need), so it is off unless asked for
-    # With a peer exchange on >= 4 ranks the bucket's kernel is NVLink-bound (1/R of the Adam work) and does hide
-    # behind the convolution backward.
-    # Round 2, single GPU, fused path: the update of the fc1 + head bucket throttled to 2 CTAs per SM underneath the
-    # convolution backward (it must start after fc1's data gradient, the last reader of fc1's weights): 0.336 ms per step
-    # against 0.317 unsplit (3 CTAs per SM: 0.322; 1: 0.384) -- the throttled update is slow and still takes SM slots
-    # and L2 bandwidth from the latency-bound conv kernels.  (A first measurement of 0.300 ms started the update BEFORE
-    # fc1's data gradient had finished -- a race -- and is void.)  Data parallel, 8 GPUs (round 1): 0.540 split vs 0.522.
-    split_default = '0'
-    self._split_adam = (self._concurrent and hasattr(network, 'grad_buckets') and
-                        os.environ.get('B200RL_SPLIT_ADAM', split_default) == '1')
-    self._tail_ctas = int(os.environ.get('B200RL_TAIL_ADAM_CTAS', '2'))
+    self._concurrent = bool(concurrent_streams) and hasattr(network, 'grad_buckets')
     # one launch ends the step (target copy of parameters + shadow, both counters): single GPU only, where the whole step
     # is one graph and the counters are bumped in one place
-    self._fuse_tail = self._world == 1 and os.environ.get('B200RL_FUSE_TAIL', '1') != '0'
-    self._tail_done = None
+    self._fuse_tail = self._world == 1
     self._side = [torch.cuda.Stream(device=dev) for _ in range(6)] if self._concurrent else None
     self._wmax_done = None
     self._params_ready = None      # pipelined exchange: event the online forwards wait for
     self._k2_done = False          # K2 of this step was already issued beside the backward
-    self._pdl_scope_mode = os.environ.get('B200RL_PDL_SCOPE', 'all')
-    # single GPU: K2 right after K4 on the auxiliary stream (beside the backward) instead of beside Adam, which then has
-    # the HBM to itself
-    self._k2_early = self._world == 1 and os.environ.get('B200RL_K2_EARLY', K2_EARLY_DEFAULT) == '1'
     # data parallel: gradients and parameters live in a peer-mapped region and the exchange is fused with Adam
     # (parallel.PeerExchange); peer_exchange=False keeps the NCCL all-reduce + replicated Adam path
     if peer_exchange is None:
@@ -149,26 +129,17 @@ class DQNLearner(core.Learner, core.Saveable):
     # pass waits for the torso bucket before conv1 and for the fc1 + head bucket before fc1.  Same values as the serial
     # order (K1 of step t+1 still follows K2 of step t); `flush()` applies the update still in flight.
     self._pipeline1 = (self._px is None and self._world == 1 and self._concurrent and self._fused and bool(use_cuda_graph) and
-                       hasattr(network, 'grad_buckets') and os.environ.get('B200RL_PIPELINE_1GPU', PIPELINE_1GPU_DEFAULT) == '1')
+                       os.environ.get('B200RL_PIPELINE_1GPU', PIPELINE_1GPU_DEFAULT) == '1')
     self._cap_stream = None
     if self._pipeline1:
       self._pipeline = True
       self._fuse_tail = False          # the pipelined update ends with its own target copy + increment
       # The update's CTAs must not queue in front of the step's: the graph is captured on a high-priority stream (its
       # forks too) and only the update's side stream keeps the default (lowest) priority, so K1 / K3 / the forwards take
-      # every SM slot the streaming Adam kernel frees (B200RL_PIPE_PRIO=0: all streams equal -- measured 0.281 ms per
-      # step, K1 finishing 40 us into the step behind Adam's 1,184 CTAs).
-      if os.environ.get('B200RL_PIPE_PRIO', '1') == '1':
-        self._cap_stream = torch.cuda.Stream(device=dev, priority=-1)
-        self._side = [torch.cuda.Stream(device=dev, priority=(0 if i == 3 else -1)) for i in range(6)]
-    elif self._world == 1 and self._concurrent and os.environ.get('B200RL_STREAM_PRIO', STREAM_PRIO_DEFAULT) == '1':
-      # the step's critical chain (K1, K3, online pass, head, data gradients) is captured on a high-priority stream; the
-      # forks (target pass, weight gradients, bias gradients, K2) keep the default priority and fill the slots left over
+      # every SM slot the streaming Adam kernel frees (all streams equal: measured 0.281 ms per step, K1 finishing 40 us
+      # into the step behind Adam's 1,184 CTAs).
       self._cap_stream = torch.cuda.Stream(device=dev, priority=-1)
-    self._pipe_adam_ctas = int(os.environ.get('B200RL_PIPE_ADAM_CTAS', '0'))
-    # 1 = the update is forked AFTER K1 / K3 have been issued (they are short and latency-bound; the update then runs
-    # beside the forwards only); 0 = at the very start of the graph
-    self._pipe_order = int(os.environ.get('B200RL_PIPE_ORDER', '0'))   # measured: 0.282 (0) vs 0.291 (1)
+      self._side = [torch.cuda.Stream(device=dev, priority=(0 if i == 3 else -1)) for i in range(6)]
     # Early tail (>= 4 ranks, where the exchange is NVLink-bound rather than HBM-bound): the fc1 + head bucket of step
     # t is exchanged as soon as step t's dense backward has produced it, underneath the convolution backward, without
     # waiting for the peers' stores; the torso bucket's exchange at the start of step t+1 ends with the barrier that
@@ -237,18 +208,18 @@ class DQNLearner(core.Learner, core.Saveable):
     # bf16 dataflow on uint8 frames: K3 writes the first conv layer's row image itself (no conversion pass)
     self._gather_rows = None
     if (self._fused and getattr(network, 'flow', False) and self._obs_dtype == np.uint8 and
-        getattr(dataset, 'supports_gather_rows', True) and os.environ.get('B200RL_GATHER_ROWS', '1') != '0'):
+        getattr(dataset, 'supports_gather_rows', True)):
       buf = network.rows_buffer(2 * B, 'all')
       fb = network.rows_frame_bytes()
       if buf is not None and fb:
         self._gather_rows = (buf.data_ptr(), buf.data_ptr() + B * fb, network.geom(0, 1))
 
   # ------------------------------------------------------------------ one update on the device
-  def _obs_view(self, rows):
+  def _obs_view_n(self, rows, n):
     torch = self._torch
     if self._obs_dtype == np.uint8:
-      return rows.view((self.B,) + self._obs_shape)
-    return rows.view(getattr(torch, self._obs_dtype.name)).view((self.B,) + self._obs_shape)
+      return rows.view((n,) + self._obs_shape)
+    return rows.view(getattr(torch, self._obs_dtype.name)).view((n,) + self._obs_shape)
 
   def _actions_i32(self):
     torch = self._torch
@@ -276,7 +247,7 @@ class DQNLearner(core.Learner, core.Saveable):
       self._forwards_fused()
       self._stamp(2)
       return
-    o_tm1, o_t = self._obs_view(ds.o_tm1), self._obs_view(ds.o_t)
+    o_tm1, o_t = self._obs_view_n(ds.o_tm1, self.B), self._obs_view_n(ds.o_t, self.B)
     if self._concurrent:
       torch = self._torch
       main = torch.cuda.current_stream()
@@ -286,7 +257,7 @@ class DQNLearner(core.Learner, core.Saveable):
         s.wait_event(start)
       # uint8 frames in tensor-core mode: one fp32 row image per observation batch serves every pass over it
       # (o_t: target + online forward; o_tm1: online forward + conv1's weight gradient)
-      shared = hasattr(net, 'prepare_frames') and os.environ.get('B200RL_SHARED_ROWS', '1') == '1'
+      shared = hasattr(net, 'prepare_frames')
       rows_t = None
       self._rows_tm1 = None
       with torch.cuda.stream(self._side[0]):
@@ -327,28 +298,12 @@ class DQNLearner(core.Learner, core.Saveable):
       net.forward(o_t, self._bufs_sel)                           # learning.py:125
     self._stamp(2)
 
-  def _pdl_scope(self, what):
-    """Programmatic dependent launch per phase (B200RL_PDL_SCOPE = all | bwd | noft: everything but the target forward):
-    a dependent grid scheduled early holds SM slots while it waits, which the OTHER forward pass running beside it
-    could have used."""
-    scope = self._pdl_scope_mode
-    if scope == 'all':
-      return
-    off = what is not None and (scope == 'bwd' or (scope == 'noft' and what == 'tgt'))
-    _capi.load().b200rl_debug_set_pdl(0 if off else -1)
-
-  def _obs_view_n(self, rows, n):
-    torch = self._torch
-    if self._obs_dtype == np.uint8:
-      return rows.view((n,) + self._obs_shape)
-    return rows.view(getattr(torch, self._obs_dtype.name)).view((n,) + self._obs_shape)
-
   def _forwards_fused(self):
     """Target features on o_t (side stream) beside ONE online pass over the 2B frames [o_tm1; o_t]."""
     torch = self._torch
     ds, net, tgt, B = self._dataset, self._net, self._tgt, self.B
     o_all = self._obs_view_n(ds.o_both, 2 * B)
-    o_t = self._obs_view(ds.o_t)
+    o_t = self._obs_view_n(ds.o_t, B)
     main = torch.cuda.current_stream()
     rows_all = rows_t = None
     self._rows_tm1 = None
@@ -377,11 +332,9 @@ class DQNLearner(core.Learner, core.Saveable):
       with torch.cuda.stream(side):
         if rows_all is not None and rows_t is None:
           rows_t = tgt.prepare_frames(o_t, 't')              # precision 1: the row image cannot be sliced
-        self._pdl_scope('tgt')
         tgt.lane(1).features(o_t, self._bufs_tgt, **(dict(rows=rows_t) if rows_t is not None else {}))   # learning.py:124
         done = torch.cuda.Event()
         done.record(side)
-      self._pdl_scope('on')
       tgt.lane(0)
       if ev_conv is not None:
         # pipelined exchange: the torso's parameters (a 0.3 MB bucket, exchanged first) must have landed before the
@@ -392,7 +345,6 @@ class DQNLearner(core.Learner, core.Saveable):
       if rows_all is not None:
         kw['rows'] = rows_all
       net.lane(0).features(o_all, self._bufs_on, **kw)       # learning.py:123 and :125 in one pass
-      self._pdl_scope(None)
       main.wait_event(done)
     else:
       if rows_all is not None and rows_t is None:
@@ -435,12 +387,11 @@ class DQNLearner(core.Learner, core.Saveable):
     step cut the backward in two ('dense' = loss + head + fc1, 'conv' = the torso) so that the all-reduce
     of the fc1/head gradients (99% of the bytes) overlaps the convolution backward."""
     ds, net = self._dataset, self._net
+    o_tm1 = self._obs_view_n(ds.o_tm1, self.B)
     if part == 'conv':
-      net.backward_conv_part(self._obs_view(ds.o_tm1), self._bufs_train, self._gbufs, self._side[0],
-                             **self._rows_kw())
+      net.backward_conv_part(o_tm1, self._bufs_train, self._gbufs, self._side[0], **self._rows_kw())
       return
     st = _capi.current_stream()
-    o_tm1 = self._obs_view(ds.o_tm1)
     if self._wmax_done is not None:
       self._torch.cuda.current_stream().wait_event(self._wmax_done)
       self._wmax_done = None
@@ -456,29 +407,22 @@ class DQNLearner(core.Learner, core.Saveable):
     self._stamp(3)
     if part == 'dense':
       net.backward_dense_part(self._bufs_train, self._gbufs, self.dq, self._side[0])
-    elif self._concurrent and self._split_adam and (self._world == 1 or self._px is not None):
-      # fc1 + heads (99% of the parameters) are final after the dense part: their Adam update streams 200 MB and
-      # runs on a third stream underneath the latency-bound convolution backward
-      net.backward_dense_part(self._bufs_train, self._gbufs, self.dq, self._side[0])
-      self._adam_tail_async()
-      net.backward_conv_part(o_tm1, self._bufs_train, self._gbufs, self._side[0], **self._rows_kw())
-    elif self._concurrent and self._early_tail_now:
-      torch = self._torch
-      net.backward_dense_part(self._bufs_train, self._gbufs, self.dq, self._side[0])
-      main, side = torch.cuda.current_stream(), self._side[4]
-      ev = torch.cuda.Event()
-      ev.record(main)
-      side.wait_event(ev)
-      if self._inc_done is not None:
-        side.wait_event(self._inc_done)
-        self._inc_done = None
-      with torch.cuda.stream(side):
-        self._early_tail_exchange()
-        self._early_done = torch.cuda.Event()
-        self._early_done.record(side)
-      net.backward_conv_part(o_tm1, self._bufs_train, self._gbufs, self._side[0], **self._rows_kw())
     elif self._concurrent:
-      net.backward(o_tm1, self._bufs_train, self._gbufs, self.dq, side_stream=self._side[0], **self._rows_kw())
+      net.backward_dense_part(self._bufs_train, self._gbufs, self.dq, self._side[0])
+      if self._early_tail_now:
+        torch = self._torch
+        main, side = torch.cuda.current_stream(), self._side[4]
+        ev = torch.cuda.Event()
+        ev.record(main)
+        side.wait_event(ev)
+        if self._inc_done is not None:
+          side.wait_event(self._inc_done)
+          self._inc_done = None
+        with torch.cuda.stream(side):
+          self._early_tail_exchange()
+          self._early_done = torch.cuda.Event()
+          self._early_done.record(side)
+      net.backward_conv_part(o_tm1, self._bufs_train, self._gbufs, self._side[0], **self._rows_kw())
     else:
       net.backward(o_tm1, self._bufs_train, self._gbufs, self.dq)
 
@@ -507,15 +451,16 @@ class DQNLearner(core.Learner, core.Saveable):
       aux.wait_event(ev)
       with torch.cuda.stream(aux):
         _capi.call('b200rl_mean', B, _capi.ptr(self.loss_ps), _capi.ptr(self.loss), _capi.current_stream())
-        if (self._pipeline1 or self._k2_early) and self._replay_client is not None:
-          # K2 (learning.py:151-154) only needs K4's priorities: beside the backward instead of after it
+        if self._world == 1 and self._replay_client is not None:
+          # K2 (learning.py:151-154) only needs K4's priorities: on one GPU it runs beside the backward instead of beside
+          # Adam, which then has the HBM to itself
           ds.table.update_priorities_device(ds.keys, self.priority)
           self._k2_done = True
         self._loss_done = torch.cuda.Event()
         self._loss_done.record(aux)
     else:
       _capi.call('b200rl_mean', B, _capi.ptr(self.loss_ps), _capi.ptr(self.loss), _capi.current_stream())
-    o_tm1 = self._obs_view(ds.o_tm1)
+    o_tm1 = self._obs_view_n(ds.o_tm1, B)
     bt = self._bufs_train
     if part == 'dense':
       net.backward_dense_part(bt, gb, None, self._side[0])
@@ -535,27 +480,10 @@ class DQNLearner(core.Learner, core.Saveable):
             self._early_tail_exchange()
             self._early_done = torch.cuda.Event()
             self._early_done.record(side)
-      elif self._split_adam and (self._world == 1 or self._px is not None):
-        # fc1 + heads are 99% of the parameters and final long before the torso's gradients: their optimizer update can
-        # run underneath the convolution backward (B200RL_SPLIT_ADAM=1; `_apply` then only updates the torso bucket)
-        def hook(events):
-          side = self._side[3]
-          for ev in events:
-            side.wait_event(ev)
-          with torch.cuda.stream(side):
-            (o1, n1), _ = net.grad_buckets()
-            self._adam(o1, n1, bucket=0)
-            self._tail_done = torch.cuda.Event()
-            self._tail_done.record(side)
       net.backward_after_head(o_tm1, bt, gb, self._side[0], self._side[1], on_dense_done=hook, **self._rows_kw())
     else:
       net.head_wgrad(bt, gb)
-      net._fc1_wgrad(bt, gb)
-      net._fc1_dgrad(bt, gb)
-      for i in (2, 1, 0):
-        net._conv_wgrad(i, o_tm1, bt, gb, self._rows_kw().get('rows'))
-        if i > 0:
-          net._conv_dgrad(i, bt, gb)
+      net.backward_from_dh(o_tm1, bt, gb, **self._rows_kw())
     if getattr(self, '_loss_done', None) is not None:
       torch.cuda.current_stream().wait_event(self._loss_done)
       self._loss_done = None
@@ -589,46 +517,23 @@ class DQNLearner(core.Learner, core.Saveable):
     else:
       self._px.adam(o1, n1, *args, 0, final_barrier=False)
 
-  def _adam(self, off: int, n: int, bucket: int = 0):
+  def _adam(self, off: int, n: int):
     """K7 over params[off : off + n] (snt.optimizers.Adam.apply, dqn/learning.py:147-149); with a peer exchange the
     gradient mean over the ranks, Adam on the owned shard and the parameter broadcast are one kernel."""
     if self._px is not None:
-      # the fc1 + head bucket (0) of a split update is followed by the conv bucket (1), whose barrier covers both
-      final = not (self._split_adam and bucket == 0)
-      self._px.adam(off, n, self._m, self._v, self._num_steps, self._lr, 0.9, 0.999, self._adam_eps, self._eps_mode, bucket,
-                    final_barrier=final)
+      self._px.adam(off, n, self._m, self._v, self._num_steps, self._lr, 0.9, 0.999, self._adam_eps, self._eps_mode, 0)
       self._net.params.refresh_shadow(off, n)
       return
     P, b = self._net.params, 4 * off
     shadow = (P.shadow.data_ptr() + 2 * off) if P.shadow is not None else None      # bf16 dataflow: weights' bf16 copy
-    throttle = self._tail_ctas if (self._split_adam and bucket == 0 and n < P.size) else 0   # beside the conv backward
-    if self._pipeline1 and bucket == 0 and n < P.size:
-      throttle = self._pipe_adam_ctas                                                       # beside the next step's torso
-    _capi.call('b200rl_adam_throttled', n, _capi.ptr(P.flat) + b, _capi.ptr(P.grad) + b, _capi.ptr(self._m) + b,
+    _capi.call('b200rl_adam', n, _capi.ptr(P.flat) + b, _capi.ptr(P.grad) + b, _capi.ptr(self._m) + b,
                _capi.ptr(self._v) + b, _capi.ptr(self._num_steps), self._lr, 0.9, 0.999, self._adam_eps, self._eps_mode,
-               _capi.ptr(self._gscale) if self._world > 1 else None, shadow, throttle, _capi.current_stream())
+               _capi.ptr(self._gscale) if self._world > 1 else None, shadow, _capi.current_stream())
 
-  def _adam_tail_async(self):
-    """Adam on the fc1 + head bucket on side stream 1 (B200RL_SPLIT_ADAM=1)."""
-    torch = self._torch
-    (o1, n1), _ = self._net.grad_buckets()
-    main, side = torch.cuda.current_stream(), self._side[1]
-    ev = torch.cuda.Event()
-    ev.record(main)
-    side.wait_event(ev)
-    with torch.cuda.stream(side):
-      self._adam(o1, n1, bucket=0)
-      self._tail_done = torch.cuda.Event()
-      self._tail_done.record(side)
-
-  def _apply(self, adam: str = 'auto'):
-    """Adam, priority update, periodic target copy, step counter.  adam = 'all' | 'conv+join' (the fc1 + head bucket
-    was updated by _adam_tail_async inside this capture: join it) | 'conv' (the caller has joined it)."""
+  def _apply(self):
+    """Adam, priority update, periodic target copy, step counter."""
     net, tgt, st = self._net, self._tgt, _capi.current_stream()
     P = net.params
-    if adam == 'auto':
-      split = self._concurrent and self._split_adam and (self._world == 1 or self._px is not None)
-      adam = 'conv+join' if split else 'all'
     prio_done = None
     k2_done, self._k2_done = self._k2_done, False
     if self._replay_client is not None and self._concurrent and not k2_done:
@@ -641,13 +546,7 @@ class DQNLearner(core.Learner, core.Saveable):
         self._dataset.table.update_priorities_device(self._dataset.keys, self.priority)   # learning.py:151-154
         prio_done = torch.cuda.Event()
         prio_done.record(self._side[2])
-    if adam == 'all':
-      self._adam(0, P.size)
-    else:
-      if adam == 'conv+join':
-        self._torch.cuda.current_stream().wait_event(self._tail_done)
-      _, (o0, n0) = net.grad_buckets()
-      self._adam(o0, n0, bucket=1)
+    self._adam(0, P.size)
     self._stamp(5)
     if prio_done is not None:
       self._torch.cuda.current_stream().wait_event(prio_done)
@@ -731,10 +630,10 @@ class DQNLearner(core.Learner, core.Saveable):
     elif self._pipeline1:
       torch = self._torch
       (o1, n1), (o0, n0) = self._net.grad_buckets()
-      self._adam(o0, n0, bucket=1)       # torso: 0.3 MB, what conv1 of the next online pass waits for
+      self._adam(o0, n0)                 # torso: 0.3 MB, what conv1 of the next online pass waits for
       ev_conv = torch.cuda.Event()
       ev_conv.record(torch.cuda.current_stream())
-      self._adam(o1, n1, bucket=0)       # fc1 + heads: 99% of the bytes, needed only before fc1
+      self._adam(o1, n1)                 # fc1 + heads: 99% of the bytes, needed only before fc1
       ev_tail = torch.cuda.Event()
       ev_tail.record(torch.cuda.current_stream())
       events = (ev_conv, ev_tail)
@@ -749,19 +648,14 @@ class DQNLearner(core.Learner, core.Saveable):
       self._inc_done.record(self._torch.cuda.current_stream())
     return events
 
-  def _compute_head(self, uniforms=None):
-    """K1 + K3 of a step."""
+  def _compute(self, uniforms=None):
+    """The gradient half of a step: K1, K3, forwards, K4, backward, K2."""
     self._stamp(0)
     self._mk('start')
     self._sample(uniforms)
     self._mk('k1')
     self._dataset.gather_only(self._gather_rows)
     self._mk('k3')
-
-  def _compute(self, uniforms=None, head_done: bool = False):
-    """The gradient half of a step: K1, K3, forwards, K4, backward, K2."""
-    if not head_done:
-      self._compute_head(uniforms)
     self._forwards()
     self._loss_backward()
     self._stamp(4)
@@ -780,13 +674,9 @@ class DQNLearner(core.Learner, core.Saveable):
     def body():
       self._early_tail_now = self._early_tail
       self._inc_done = None
-      head_done = False
       if variant == 'copy':          # the target network changes in this update: strict order
         self._apply_update(copy=True, tail_done=self._early_tail)
       elif variant == 'norm':        # update on a side stream; only the online forwards wait for it
-        if self._pipeline1 and self._pipe_order == 1:
-          self._compute_head()
-          head_done = True
         main, side = torch.cuda.current_stream(), self._side[3]
         ev = torch.cuda.Event()
         ev.record(main)
@@ -799,7 +689,7 @@ class DQNLearner(core.Learner, core.Saveable):
             self._params_ready = (ev, ev)
           self._update_done = torch.cuda.Event()     # the side stream must rejoin the capture's origin stream
           self._update_done.record(side)
-      self._compute(head_done=head_done)
+      self._compute()
       if variant == 'norm':
         torch.cuda.current_stream().wait_event(self._update_done)
       self._early_tail_now = False
@@ -894,13 +784,13 @@ class DQNLearner(core.Learner, core.Saveable):
         def second():
           self._dataset.gather_only(self._gather_rows)
           self._forwards()
-        if self._concurrent and hasattr(self._net, 'grad_buckets'):
+        if self._concurrent:
           self._graphs = [self._capture(self._sample), self._capture(second),
                           self._capture(lambda: self._loss_backward('dense')),
-                          self._capture(lambda: self._loss_backward('conv')), self._capture(lambda: self._apply('all'))]
+                          self._capture(lambda: self._loss_backward('conv')), self._capture(self._apply)]
         else:
           self._graphs = [self._capture(self._sample), self._capture(second), self._capture(self._loss_backward),
-                          self._capture(lambda: self._apply('all'))]
+                          self._capture(self._apply)]
     if self._world == 1 or self._px is not None:
       self._graphs[0].replay()
       return

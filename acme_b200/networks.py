@@ -573,26 +573,25 @@ class DQNAtariNetwork(Network):
     else:
       _conv_dgrad(dy, P.p(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), g, bufs[f'y{i}'].data_ptr(), ACT_RELU, self)
 
-  def backward(self, obs, bufs, gbufs, dq, side_stream=None, rows=None):
+  def backward(self, obs, bufs, gbufs, dq, rows=None):
     """Accumulates nothing: overwrites params.grad with d(loss)/d(params) given dq [B, A].  `rows`: the row image of
     `obs` from prepare_frames(), if the caller has one.
 
-    With `side_stream`, the weight-gradient GEMMs of fc1 / conv3 / conv2 run on it (workspace lane 1)
-    concurrently with the data-gradient chain on the current stream: the two are independent once a
+    All on the current stream.  backward_dense_part followed by backward_conv_part is the same computation with the
+    weight-gradient GEMMs on a side stream, concurrent with the data-gradient chain: the two are independent once a
     layer's dy exists, and each kernel alone is too latency-bound to fill the machine."""
-    if side_stream is not None:
-      return self._backward_two_streams(obs, bufs, gbufs, dq, side_stream, rows)
     self._head_backward(bufs, gbufs, dq)
+    self.backward_from_dh(obs, bufs, gbufs, rows)
+
+  def backward_from_dh(self, obs, bufs, gbufs, rows=None):
+    """fc1's and the torso's gradients from gbufs['dh'] (written by _head_backward or the fused head + TD kernel), on
+    the current stream."""
     self._fc1_wgrad(bufs, gbufs)
     self._fc1_dgrad(bufs, gbufs)
     for i in (2, 1, 0):
       self._conv_wgrad(i, obs, bufs, gbufs, rows)
       if i > 0:
         self._conv_dgrad(i, bufs, gbufs)
-
-  def _backward_two_streams(self, obs, bufs, gbufs, dq, side, rows=None):
-    self.backward_dense_part(bufs, gbufs, dq, side)
-    self.backward_conv_part(obs, bufs, gbufs, side, rows)
 
   def backward_after_head(self, obs, bufs, gbufs, s1, s2, rows=None, on_dense_done=None):
     """Everything behind the fused head + TD kernel (which has produced gbufs['dh'] / ['dval'] / ['dadv']), scheduled on

@@ -288,10 +288,6 @@ int b200rl_dpg_action_grad(int32_t B, int32_t A, const float* dqda, float clip, 
 int b200rl_adam(int64_t n, float* param, const float* grad, float* m, float* v,
                 const int64_t* step_dev, float lr, double b1, double b2, float eps, int eps_mode,
                 const float* grad_scale_dev, void* bf16_shadow, void* stream);
-/* b200rl_adam on a grid limited to ctas_per_sm CTAs per SM (0 = default): for an update issued BESIDE other kernels */
-int b200rl_adam_throttled(int64_t n, float* param, const float* grad, float* m, float* v, const int64_t* step_dev,
-                          float lr, double b1, double b2, float eps, int eps_mode, const float* grad_scale_dev,
-                          void* bf16_shadow, int32_t ctas_per_sm, void* stream);
 /* tf.clip_by_global_norm (d4pg/learning.py:235-237): *scale_out = clip / max(||g||, clip). */
 int b200rl_global_norm_scale(int64_t n, const float* grad, float clip, float* partial_ws,
                              float* scale_out_dev, float* norm_out_dev, void* stream);

@@ -1,5 +1,5 @@
 """K7 micro-benchmark: the Adam kernel on 8,018,624 parameters with random and with 'trained-network-like' data (many
-tiny gradients), with / without the bf16 shadow.  Env: B200RL_ADAM_FAST, B200RL_ADAM_CTAS_PER_SM."""
+tiny gradients), with / without the bf16 shadow."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
