@@ -132,6 +132,10 @@ PROTOTYPES = {
                                            c_vp, c_vp, c_i64, c_vp]),
     'b200rl_layernorm_tanh_fwd': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_layernorm_tanh_bwd': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'b200rl_feature_layer_fwd': (c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp,
+                                         c_vp]),
+    'b200rl_feature_layer_bwd': (c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                         c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
     'b200rl_tanh_to_spec_fwd': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_tanh_to_spec_bwd': (c_int, [c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'b200rl_concat2': (c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp]),

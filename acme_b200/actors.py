@@ -85,8 +85,11 @@ class BatchedGaussianNoise:
 
   _SEED_SALT = BatchedEpsilonGreedy._SEED_SALT
 
-  def __init__(self, policy, sigma: float, act_min, act_max, seed: int = 0):
+  def __init__(self, policy, sigma: float, act_min, act_max, seed: int = 0, observation_network=None):
+    """observation_network (networks.AtariTorso): the policy reads its features (conv1's row image in its own 'act'
+    slot)."""
     self.network, self.sigma, self.seed = policy, float(np.float32(sigma)), int(seed) ^ self._SEED_SALT
+    self.torso = observation_network
     A = policy.act_dim
     self._lo = np.ascontiguousarray(np.broadcast_to(np.asarray(act_min, np.float32), (A,)))
     self._hi = np.ascontiguousarray(np.broadcast_to(np.asarray(act_max, np.float32), (A,)))
@@ -96,6 +99,8 @@ class BatchedGaussianNoise:
     import torch
     dev = torch.device('cuda', self.network.device)
     self.bufs = self.network.make_buffers(N)
+    if self.torso is not None:
+      self.torso_bufs = self.torso.make_buffers(N)
     self.counter = torch.zeros(1, dtype=torch.int64, device=dev)
     self.lo, self.hi = torch.as_tensor(self._lo).to(dev), torch.as_tensor(self._hi).to(dev)
     self.actions = torch.empty((N, self.network.act_dim), dtype=torch.float32, device=dev)
@@ -103,7 +108,11 @@ class BatchedGaussianNoise:
 
   def act(self, obs):
     N, A = obs.shape[0], self.network.act_dim
-    a = self.network.action(obs, self.bufs)
+    if self.torso is not None:
+      feat = self.torso.forward(obs, self.torso_bufs, rows=self.torso.prepare_frames(obs, 'act'))
+      a = self.network.action_features(feat.data_ptr(), self.bufs)
+    else:
+      a = self.network.action(obs, self.bufs)
     _capi.call('b200rl_gaussian_explore', N, A, _capi.ptr(a), self.sigma, _capi.ptr(self.lo), _capi.ptr(self.hi), self.seed,
                _capi.ptr(self.counter), _capi.ptr(self.actions), None, _capi.current_stream())
     return self.actions

@@ -1179,6 +1179,149 @@ __global__ void layernorm_param_grad_kernel(int B, int N, const float* __restric
   doffset[i] = dof;
 }
 
+// The first LayerNormMLP layer over observation-network features: z0 = z_f + a @ w_a^T + b (z_f = features @ w_f^T, a
+// GEMM with an fp32 output), then LayerNorm + tanh with the arithmetic of layernorm_tanh_fwd_kernel.  CTA per row.
+constexpr int kFeatMaxN = 1024, kFeatMaxA = 64, kFeatRows = 8;
+__device__ unsigned int g_feature_tickets[64];
+
+__global__ void __launch_bounds__(256)
+feature_layer_fwd_kernel(int N, int A, const float* __restrict__ zf, const float* __restrict__ act,
+                         const float* __restrict__ w_a, const float* __restrict__ bias, const float* __restrict__ scale,
+                         const float* __restrict__ offset, float eps, float* __restrict__ y,
+                         __nv_bfloat16* __restrict__ y_bf16, float* __restrict__ xhat, float* __restrict__ rstd) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ float scratch[32];
+  __shared__ float z[kFeatMaxN];
+  __shared__ float a_s[kFeatMaxA];
+  const int b = blockIdx.x;
+  if (threadIdx.x < A) a_s[threadIdx.x] = act[(size_t)b * A + threadIdx.x];
+  __syncthreads();
+  float s = 0.f;
+  for (int i = threadIdx.x; i < N; i += blockDim.x) {
+    float v = zf[(size_t)b * N + i];
+    for (int k = 0; k < A; ++k) v = fmaf(a_s[k], w_a[(size_t)i * A + k], v);
+    v = v + bias[i];
+    z[i] = v;
+    s += v;
+  }
+  const float mean = block_reduce(s, SumF(), 0.f, scratch) / (float)N;
+  float vs = 0.f;
+  for (int i = threadIdx.x; i < N; i += blockDim.x) { float d = z[i] - mean; vs += d * d; }
+  const float var = block_reduce(vs, SumF(), 0.f, scratch) / (float)N;
+  const float rs = rsqrtf(var + eps);
+  for (int i = threadIdx.x; i < N; i += blockDim.x) {
+    float xh = (z[i] - mean) * rs;
+    xhat[(size_t)b * N + i] = xh;
+    const float yv = tanhf(xh * scale[i] + offset[i]);
+    y[(size_t)b * N + i] = yv;
+    if (y_bf16) y_bf16[(size_t)b * N + i] = __float2bfloat16_rn(yv);
+  }
+  if (threadIdx.x == 0) rstd[b] = rs;
+}
+
+// Its backward.  CTA s owns rows [s * rows_per_cta, ...) (at most kFeatRows): per row the LayerNorm + tanh backward of
+// layernorm_tanh_bwd_kernel gives dz (fp32, and RN-bf16(dz) when asked) and, when asked, da = dz @ w_a (one warp per
+// action column, lanes in a fixed stride, then a fixed butterfly).  The parameter gradients are sums over the batch in
+// ascending row order: d scale = sum dt * xhat, d offset = sum dt (dt = dy * (1 - y^2)), db = sum dz, dw_a = dz^T a.
+// With one slice the CTA writes them; with several each writes a partial slab to `partial` and the CTA that finishes last
+// (per-stream ticket, reset on exit: CUDA-graph safe) adds the slabs in slice order.
+__global__ void __launch_bounds__(256)
+feature_layer_bwd_kernel(int B, int N, int A, const float* __restrict__ dy, const float* __restrict__ y,
+                         const float* __restrict__ xhat, const float* __restrict__ rstd, const float* __restrict__ scale,
+                         const float* __restrict__ act, const float* __restrict__ w_a, float* __restrict__ dz,
+                         __nv_bfloat16* __restrict__ dz_bf16, float* __restrict__ dscale, float* __restrict__ doffset,
+                         float* __restrict__ db, float* __restrict__ dw_a, float* __restrict__ da, int rows_per_cta,
+                         float* __restrict__ partial, int ticket) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ float scratch[32];
+  __shared__ float dz_s[kFeatRows][kFeatMaxN];
+  __shared__ float a_s[kFeatRows][kFeatMaxA];
+  __shared__ bool last;
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const int m0 = blockIdx.x * rows_per_cta, rows = min(rows_per_cta, B - m0);
+  const bool grads = dscale != nullptr;
+  float acc_s[kFeatMaxN / 256], acc_o[kFeatMaxN / 256];
+#pragma unroll
+  for (int q = 0; q < kFeatMaxN / 256; ++q) acc_s[q] = acc_o[q] = 0.f;
+  for (int r = 0; r < rows; ++r) {
+    const size_t o = (size_t)(m0 + r) * N;
+    float s1 = 0.f, s2 = 0.f;
+    for (int i = t; i < N; i += blockDim.x) {
+      float dt = dy[o + i] * (1.f - y[o + i] * y[o + i]);
+      float dxh = dt * scale[i];
+      s1 += dxh;
+      s2 += dxh * xhat[o + i];
+    }
+    const float m1 = block_reduce(s1, SumF(), 0.f, scratch) / (float)N;
+    const float m2 = block_reduce(s2, SumF(), 0.f, scratch) / (float)N;
+    const float rs = rstd[m0 + r];
+#pragma unroll
+    for (int q = 0; q < kFeatMaxN / 256; ++q) {
+      const int i = t + 256 * q;
+      if (i < N) {
+        float dt = dy[o + i] * (1.f - y[o + i] * y[o + i]);
+        float dxh = dt * scale[i];
+        const float v = rs * (dxh - m1 - xhat[o + i] * m2);
+        dz[o + i] = v;
+        if (dz_bf16) dz_bf16[o + i] = __float2bfloat16_rn(v);
+        dz_s[r][i] = v;
+        acc_s[q] = acc_s[q] + dt * xhat[o + i];
+        acc_o[q] = acc_o[q] + dt;
+      }
+    }
+    if (act && t < A) a_s[r][t] = act[(size_t)(m0 + r) * A + t];
+  }
+  __syncthreads();
+  if (da)
+    for (int p = warp; p < rows * A; p += 8) {
+      const int r = p / A, k = p % A;
+      float s = 0.f;
+      for (int i = lane; i < N; i += 32) s = fmaf(dz_s[r][i], w_a[(size_t)i * A + k], s);
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) s = s + __shfl_xor_sync(0xffffffffu, s, off);
+      if (lane == 0) da[(size_t)(m0 + r) * A + k] = s;
+    }
+  if (!grads) return;
+  // this slice's sums: [d scale | d offset | db] (3N) then dw_a (N x A)
+  const int per = N * (3 + A);
+  float* out = gridDim.x == 1 ? nullptr : partial + (size_t)blockIdx.x * per;
+#pragma unroll
+  for (int q = 0; q < kFeatMaxN / 256; ++q) {
+    const int i = t + 256 * q;
+    if (i < N) {
+      float sb = 0.f;
+      for (int r = 0; r < rows; ++r) sb = sb + dz_s[r][i];
+      if (out) { out[i] = acc_s[q]; out[N + i] = acc_o[q]; out[2 * N + i] = sb; }
+      else { dscale[i] = acc_s[q]; doffset[i] = acc_o[q]; db[i] = sb; }
+    }
+  }
+  for (int e = t; e < N * A; e += blockDim.x) {
+    const int i = e / A, k = e % A;
+    float s = 0.f;
+    for (int r = 0; r < rows; ++r) s = fmaf(dz_s[r][i], a_s[r][k], s);
+    if (out) out[3 * N + e] = s;
+    else dw_a[e] = s;
+  }
+  if (!out) return;
+  __threadfence();
+  __syncthreads();
+  if (t == 0) last = atomicAdd(&g_feature_tickets[ticket], 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  for (int e = t; e < per; e += blockDim.x) {
+    float s = 0.f;
+    for (int q = 0; q < (int)gridDim.x; ++q) s = s + __ldcg(partial + (size_t)q * per + e);
+    if (e < N) dscale[e] = s;
+    else if (e < 2 * N) doffset[e - N] = s;
+    else if (e < 3 * N) db[e - 2 * N] = s;
+    else dw_a[e - 3 * N] = s;
+  }
+  if (t == 0) g_feature_tickets[ticket] = 0u;
+}
+
 // acme/tf/networks/rescaling.py:63-74
 __global__ void tanh_to_spec_fwd_kernel(long long n, int A, const float* __restrict__ x, const float* __restrict__ scale,
                                         const float* __restrict__ offset, float* __restrict__ a) {
@@ -1709,6 +1852,52 @@ extern "C" int b200rl_layernorm_tanh_bwd(int32_t B, int32_t N, const float* dy, 
     B200RL_CUDA_OK(launch_pdl_small(layernorm_param_grad_kernel, dim3(ceil_div(N, 128)), dim3(128), 0, as_stream(stream), B, N, dy, y, xhat, dscale, doffset));
     B200RL_LAUNCH_OK();
   }
+  return B200RL_OK;
+}
+
+extern "C" int b200rl_feature_layer_fwd(int32_t B, int32_t N, int32_t A, const float* zf, const float* a, const float* w_a,
+                                        const float* bias, const float* scale, const float* offset, float eps, float* y,
+                                        void* y_bf16, float* xhat, float* rstd, void* stream) {
+  B200RL_REQUIRE(zf && bias && scale && offset && y && xhat && rstd && (A == 0 || (a && w_a)), "feature layer: null argument");
+  B200RL_REQUIRE(B >= 1 && N >= 1 && N <= kFeatMaxN && A >= 0 && A <= kFeatMaxA,
+                 "feature layer: N = %d must be in [1, %d] and A = %d in [0, %d]", N, kFeatMaxN, A, kFeatMaxA);
+  B200RL_CUDA_OK(launch_pdl_small(feature_layer_fwd_kernel, dim3(B), dim3(256), 0, as_stream(stream), N, A, zf, a, w_a, bias,
+                                  scale, offset, eps, y, (__nv_bfloat16*)y_bf16, xhat, rstd));
+  B200RL_LAUNCH_OK();
+  return B200RL_OK;
+}
+
+extern "C" int b200rl_feature_layer_bwd(int32_t B, int32_t N, int32_t A, const float* dy, const float* y, const float* xhat,
+                                        const float* rstd, const float* scale, const float* a, const float* w_a, float* dz,
+                                        void* dz_bf16, float* dscale, float* doffset, float* db, float* dw_a, float* da,
+                                        void* ws, int64_t ws_bytes, void* stream) {
+  const bool grads = dscale || doffset || db || dw_a;
+  B200RL_REQUIRE(dy && y && xhat && rstd && scale && dz, "feature layer backward: null argument");
+  B200RL_REQUIRE(B >= 1 && N >= 1 && N <= kFeatMaxN && A >= 0 && A <= kFeatMaxA,
+                 "feature layer backward: N = %d must be in [1, %d] and A = %d in [0, %d]", N, kFeatMaxN, A, kFeatMaxA);
+  B200RL_REQUIRE(!grads || (dscale && doffset && db && (A == 0 || dw_a)),
+                 "feature layer backward: d scale, d offset, db and dw_a are requested together");
+  B200RL_REQUIRE(!(grads && A > 0) || a, "feature layer backward: dw_a needs the actions");
+  B200RL_REQUIRE(!da || (A > 0 && w_a), "feature layer backward: da needs A >= 1 and w_a");
+  cudaStream_t st = as_stream(stream);
+  int slices = ceil_div(B, kFeatRows);
+  int ticket = -1;
+  if (grads && slices > 1) {
+    const int64_t per = (int64_t)N * (3 + A) * 4;
+    slices = ws ? (int)std::min<int64_t>(slices, ws_bytes / per) : 1;
+    if (slices > 1) ticket = ticket_for(st);
+    if (ticket < 0) slices = 1;
+  }
+  slices = std::max(slices, 1);
+  const int rpc = ceil_div(B, slices);
+  // a slice holds at most kFeatRows rows in shared memory: with too little workspace for the slabs, refuse
+  B200RL_REQUIRE(rpc <= kFeatRows, "feature layer backward: workspace of %lld bytes is too small for B = %d",
+                 (long long)ws_bytes, B);
+  slices = ceil_div(B, rpc);
+  B200RL_CUDA_OK(launch_pdl_small(feature_layer_bwd_kernel, dim3(slices), dim3(256), 0, st, B, N, A, dy, y, xhat, rstd, scale,
+                                  a, w_a, dz, (__nv_bfloat16*)dz_bf16, dscale, doffset, db, A > 0 ? dw_a : nullptr, da, rpc,
+                                  (float*)ws, ticket < 0 ? 0 : ticket));
+  B200RL_LAUNCH_OK();
   return B200RL_OK;
 }
 

@@ -232,6 +232,8 @@ class Network:
         a = a.T
       elif isinstance(kind, tuple) and kind[0] == 'rows':   # rows [lo:hi] of a stacked [out, in]
         a = a[kind[1]:kind[2]].T if a.ndim == 2 else a[kind[1]:kind[2]]
+      elif isinstance(kind, tuple) and kind[0] == 'cat':    # [out, in0] and [out, in1] stored apart: one [in0 + in1, out]
+        a = np.concatenate([a, self.params.get(kind[1], grad)], axis=1).T
       out[sonnet_name] = np.ascontiguousarray(a)
     return out
 
@@ -249,6 +251,9 @@ class Network:
           full = self.params.get(name)
         full[kind[1]:kind[2]] = v.T if full.ndim == 2 else v
         staged[name] = full
+      elif isinstance(kind, tuple) and kind[0] == 'cat':
+        n0 = self.params.entries[name][1][1]
+        staged[name], staged[kind[1]] = v.T[:, :n0], v.T[:, n0:]
       else:
         staged[name] = v
     for name, v in staged.items():
@@ -302,14 +307,12 @@ def _conv_dgrad(dy, w, dx, g, mask, mask_act, net: Network):
   _capi.call('b200rl_conv2d_dgrad', dy, w, dx, g, mask, mask_act, net.precision, ws, wsb, _capi.current_stream())
 
 
-# =============================================================================== DQN Atari network
-class DQNAtariNetwork(Network):
-  """AtariTorso (3 SAME-padded convs + ReLU, NHWC) -> DuellingMLP([512]) (atari.py:36-69)."""
+# =============================================================================== AtariTorso convolutions
+class _ConvTorso(Network):
+  """The AtariTorso convolutions (atari.py:36-52: three SAME-padded convs + ReLU, NHWC): geometry, parameters, row
+  images and the layer calls of their forward and backward passes, shared by AtariTorso and DQNAtariNetwork."""
 
-  def __init__(self, num_actions: int, device: int = 0, precision: int = _capi.PRECISION_FP32,
-               seed: int = 0, input_hw: int = 84, input_channels: int = 4):
-    super().__init__(device, precision)
-    self.A = int(num_actions)
+  def _declare_convs(self, input_hw: int, input_channels: int):
     self.in_hw, self.in_c = input_hw, input_channels
     self.convs = []  # (k, stride, cin, cout, in_hw, out_hw, pad)
     h, c = input_hw, input_channels
@@ -318,60 +321,22 @@ class DQNAtariNetwork(Network):
       self.convs.append((k, s, c, co, h, oh, pad))
       h, c = oh, co
     self.flat_dim = h * h * c
-    P = self.params
     for i, (k, s, ci, co, _, _, _) in enumerate(self.convs, 1):
-      P.declare(f'conv{i}.w', (co, k, k, ci))
-      P.declare(f'conv{i}.b', (co,))
-    P.declare('fc1.w', (1024, self.flat_dim))   # rows 0..511 value stream, 512..1023 advantage stream
-    P.declare('fc1.b', (1024,))
-    P.declare('v2.w', (1, 512))
-    P.declare('v2.b', (1,))
-    P.declare('a2.w', (self.A, 512))
-    P.declare('a2.b', (self.A,))
-    self._export = {
-        'conv1/w': ('conv1.w', 'conv'), 'conv1/b': ('conv1.b', None),
-        'conv2/w': ('conv2.w', 'conv'), 'conv2/b': ('conv2.b', None),
-        'conv3/w': ('conv3.w', 'conv'), 'conv3/b': ('conv3.b', None),
-        'value/l0/w': ('fc1.w', ('rows', 0, 512)), 'value/l0/b': ('fc1.b', ('rows', 0, 512)),
-        'value/l1/w': ('v2.w', 'linear'), 'value/l1/b': ('v2.b', None),
-        'adv/l0/w': ('fc1.w', ('rows', 512, 1024)), 'adv/l0/b': ('fc1.b', ('rows', 512, 1024)),
-        'adv/l1/w': ('a2.w', 'linear'), 'adv/l1/b': ('a2.b', None),
-    }
-    self._finalize()
-    self.init(seed)
+      self.params.declare(f'conv{i}.w', (co, k, k, ci))
+      self.params.declare(f'conv{i}.b', (co,))
 
-  def init(self, seed: int):
+  def _init_convs(self, rng):
     """Sonnet defaults: TruncatedNormal(stddev=1/sqrt(fan_in)) weights, zero biases."""
-    rng = np.random.default_rng(seed)
-    P = self.params
     for i, (k, s, ci, co, _, _, _) in enumerate(self.convs, 1):
-      P.set(f'conv{i}.w', _truncated_normal(rng, (co, k, k, ci), 1 / math.sqrt(k * k * ci)))
-    P.set('fc1.w', _truncated_normal(rng, (1024, self.flat_dim), 1 / math.sqrt(self.flat_dim)))
-    P.set('v2.w', _truncated_normal(rng, (1, 512), 1 / math.sqrt(512)))
-    P.set('a2.w', _truncated_normal(rng, (self.A, 512), 1 / math.sqrt(512)))
+      self.params.set(f'conv{i}.w', _truncated_normal(rng, (co, k, k, ci), 1 / math.sqrt(k * k * ci)))
 
   def geom(self, i: int, B: int) -> ConvGeom:
     k, s, ci, co, h, oh, pad = self.convs[i]
     return ConvGeom(B=B, H=h, W=h, C=ci, kh=k, kw=k, stride=s, pad_top=pad, pad_left=pad, OH=oh, OW=oh, Cout=co)
 
-  # ---- buffers.  In the bf16 dataflow (precision 2) activations y1..y3 and the back-propagated gradients dh, dy1..dy3
-  # are bf16; the hidden row h (consumed by the duelling head in fp32), q, value / advantage and everything the loss
-  # touches stay fp32.
-  def make_buffers(self, B: int):
-    import torch
-    dev = torch.device('cuda', self.device)
-    f = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
-    a = (lambda *shape: torch.empty(shape, dtype=torch.bfloat16, device=dev)) if self.flow else f
-    bufs = dict(B=B, q=f(B, self.A), h=f(B, 1024), val=f(B, 1), adv=f(B, self.A))
-    for i, (k, s, ci, co, h, oh, pad) in enumerate(self.convs, 1):
-      bufs[f'y{i}'] = a(B, oh, oh, co)
-    self._size_lanes(B)
-    return bufs
-
-  def _x3_calls(self, B: int):
+  def _conv_x3_calls(self, B: int):
     X = _capi
-    calls = [(X.X3_LINEAR_FWD, B, 1024, self.flat_dim, None, 0), (X.X3_LINEAR_DGRAD, B, 1024, self.flat_dim, None, 0),
-             (X.X3_LINEAR_WGRAD, B, 1024, self.flat_dim, None, 0)]
+    calls = []
     for i in range(3):
       g = self.geom(i, B)
       x_u8s = (1, 2) if i == 0 else (0,)     # conv1 on uint8 frames or on their row image
@@ -380,17 +345,36 @@ class DQNAtariNetwork(Network):
         calls.append((X.X3_CONV_DGRAD, 0, 0, 0, g, 0))
     return calls
 
-  def make_grad_buffers(self, B: int):
+  def _torso_forward(self, obs, bufs, rows=None) -> int:
+    """The three convolutions: obs -> bufs['y1'..'y3']; returns the address of y3 (post-ReLU, bf16 in the bf16 dataflow).
+    obs: uint8 or float32 [B, H, W, C] (NHWC); uint8 is read as float32(x)/255.  `rows`: the frames' row image from
+    prepare_frames() (required in the bf16 dataflow; built here if absent)."""
     import torch
-    dev = torch.device('cuda', self.device)
-    f = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
-    a = (lambda *shape: torch.empty(shape, dtype=torch.bfloat16, device=dev)) if self.flow else f
-    g = dict(dh=a(B, 1024), dval=f(B, 1), dadv=f(B, self.A))
+    B, P, st = bufs['B'], self.params, _capi.current_stream()
+    ws, wsb = self.ws
     if self.flow:
-      g['dh32'] = f(B, 1024)           # the unfused head backward writes fp32; converted for the bf16 GEMMs
-    for i, (k, s, ci, co, h, oh, pad) in enumerate(self.convs, 1):
-      g[f'dy{i}'] = a(B, oh, oh, co)
-    return g
+      P.ensure_shadow()
+      if rows is None:
+        if obs.dtype != torch.uint8:
+          raise ValueError('the bf16 dataflow reads uint8 frames')
+        rows = self.prepare_frames(obs, 'fwd')
+      x, x_rows = rows.data_ptr(), 1
+      self._mark(f'fwd{B}.start')
+      for i in range(3):
+        y = bufs[f'y{i + 1}']
+        _capi.call('b200rl_conv2d_fwd_bf16', x, x_rows, P.sp(f'conv{i + 1}.w'), P.p(f'conv{i + 1}.b'), y.data_ptr(), 1,
+                   self.geom(i, B), ACT_RELU, ws, wsb, st)
+        self._mark(f'fwd{B}.conv{i + 1}')
+        x, x_rows = y.data_ptr(), 0
+      return x
+    x, x_u8 = obs.data_ptr(), int(obs.dtype == torch.uint8)
+    if rows is not None:              # the frames' row image from prepare_frames()
+      x, x_u8 = rows.data_ptr(), 2
+    for i in range(3):
+      y = bufs[f'y{i + 1}']
+      _conv_fwd(x, x_u8, P.p(f'conv{i + 1}.w'), P.p(f'conv{i + 1}.b'), y.data_ptr(), self.geom(i, B), ACT_RELU, self)
+      x, x_u8 = y.data_ptr(), 0
+    return x
 
   def rows_frame_bytes(self) -> int:
     """Bytes of ONE frame in the bf16 row image (precisions 2 and 3): a batched image can be sliced per sample range."""
@@ -430,42 +414,134 @@ class DQNAtariNetwork(Network):
     _capi.call(name, obs.data_ptr(), self.geom(0, B), buf.data_ptr(), buf.numel(), _capi.current_stream())
     return buf
 
+  def _conv_bias_grad(self, i, bufs, gbufs):
+    """bf16 dataflow: db of conv layer i+1 = column sums of dy, as its own launch (so it can sit on another stream)."""
+    B, P = bufs['B'], self.params
+    ws, wsb = self.ws
+    _, _, _, co, _, oh, _ = self.convs[i]
+    _capi.call('b200rl_colsum_bf16', B * oh * oh, co, gbufs[f'dy{i + 1}'].data_ptr(), co, P.g(f'conv{i + 1}.b'), ws, wsb,
+               _capi.current_stream())
+
+  def _conv_wgrad(self, i, obs, bufs, gbufs, rows, bias: bool = True):
+    import torch
+    B, P = bufs['B'], self.params
+    ws, wsb = self.ws
+    g = self.geom(i, B)
+    dy = gbufs[f'dy{i + 1}'].data_ptr()
+    if self.flow:
+      if i > 0:
+        x, x_rows = bufs[f'y{i}'].data_ptr(), 0
+      else:
+        if rows is None:
+          rows = self.prepare_frames(obs, 'bwd')
+        x, x_rows = rows.data_ptr(), 1
+      _capi.call('b200rl_conv2d_wgrad_bf16', x, x_rows, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b') if bias else None, g,
+                 ws, wsb, _capi.current_stream())
+      return
+    if i > 0:
+      x, x_u8 = bufs[f'y{i}'].data_ptr(), 0
+    elif rows is not None:
+      x, x_u8 = rows.data_ptr(), 2
+    else:
+      x, x_u8 = obs.data_ptr(), int(obs.dtype == torch.uint8)
+    _conv_wgrad(x, x_u8, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b'), g, self)
+
+  def _conv_dgrad(self, i, bufs, gbufs):
+    B, P = bufs['B'], self.params
+    ws, wsb = self.ws
+    g = self.geom(i, B)
+    dy = gbufs[f'dy{i + 1}'].data_ptr()
+    if self.flow:
+      _capi.call('b200rl_conv2d_dgrad_bf16', dy, P.sp(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), 1, g,
+                 bufs[f'y{i}'].data_ptr(), 1, ACT_RELU, _capi.current_stream())
+    else:
+      _conv_dgrad(dy, P.p(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), g, bufs[f'y{i}'].data_ptr(), ACT_RELU, self)
+
+
+# =============================================================================== DQN Atari network
+class DQNAtariNetwork(_ConvTorso):
+  """AtariTorso (3 SAME-padded convs + ReLU, NHWC) -> DuellingMLP([512]) (atari.py:36-69)."""
+
+  def __init__(self, num_actions: int, device: int = 0, precision: int = _capi.PRECISION_FP32,
+               seed: int = 0, input_hw: int = 84, input_channels: int = 4):
+    super().__init__(device, precision)
+    self.A = int(num_actions)
+    self._declare_convs(input_hw, input_channels)
+    P = self.params
+    P.declare('fc1.w', (1024, self.flat_dim))   # rows 0..511 value stream, 512..1023 advantage stream
+    P.declare('fc1.b', (1024,))
+    P.declare('v2.w', (1, 512))
+    P.declare('v2.b', (1,))
+    P.declare('a2.w', (self.A, 512))
+    P.declare('a2.b', (self.A,))
+    self._export = {
+        'conv1/w': ('conv1.w', 'conv'), 'conv1/b': ('conv1.b', None),
+        'conv2/w': ('conv2.w', 'conv'), 'conv2/b': ('conv2.b', None),
+        'conv3/w': ('conv3.w', 'conv'), 'conv3/b': ('conv3.b', None),
+        'value/l0/w': ('fc1.w', ('rows', 0, 512)), 'value/l0/b': ('fc1.b', ('rows', 0, 512)),
+        'value/l1/w': ('v2.w', 'linear'), 'value/l1/b': ('v2.b', None),
+        'adv/l0/w': ('fc1.w', ('rows', 512, 1024)), 'adv/l0/b': ('fc1.b', ('rows', 512, 1024)),
+        'adv/l1/w': ('a2.w', 'linear'), 'adv/l1/b': ('a2.b', None),
+    }
+    self._finalize()
+    self.init(seed)
+
+  def init(self, seed: int):
+    """Sonnet defaults: TruncatedNormal(stddev=1/sqrt(fan_in)) weights, zero biases."""
+    rng = np.random.default_rng(seed)
+    P = self.params
+    self._init_convs(rng)
+    P.set('fc1.w', _truncated_normal(rng, (1024, self.flat_dim), 1 / math.sqrt(self.flat_dim)))
+    P.set('v2.w', _truncated_normal(rng, (1, 512), 1 / math.sqrt(512)))
+    P.set('a2.w', _truncated_normal(rng, (self.A, 512), 1 / math.sqrt(512)))
+
+  # ---- buffers.  In the bf16 dataflow (precision 2) activations y1..y3 and the back-propagated gradients dh, dy1..dy3
+  # are bf16; the hidden row h (consumed by the duelling head in fp32), q, value / advantage and everything the loss
+  # touches stay fp32.
+  def make_buffers(self, B: int):
+    import torch
+    dev = torch.device('cuda', self.device)
+    f = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
+    a = (lambda *shape: torch.empty(shape, dtype=torch.bfloat16, device=dev)) if self.flow else f
+    bufs = dict(B=B, q=f(B, self.A), h=f(B, 1024), val=f(B, 1), adv=f(B, self.A))
+    for i, (k, s, ci, co, h, oh, pad) in enumerate(self.convs, 1):
+      bufs[f'y{i}'] = a(B, oh, oh, co)
+    self._size_lanes(B)
+    return bufs
+
+  def _x3_calls(self, B: int):
+    X = _capi
+    return [(X.X3_LINEAR_FWD, B, 1024, self.flat_dim, None, 0), (X.X3_LINEAR_DGRAD, B, 1024, self.flat_dim, None, 0),
+            (X.X3_LINEAR_WGRAD, B, 1024, self.flat_dim, None, 0)] + self._conv_x3_calls(B)
+
+  def make_grad_buffers(self, B: int):
+    import torch
+    dev = torch.device('cuda', self.device)
+    f = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
+    a = (lambda *shape: torch.empty(shape, dtype=torch.bfloat16, device=dev)) if self.flow else f
+    g = dict(dh=a(B, 1024), dval=f(B, 1), dadv=f(B, self.A))
+    if self.flow:
+      g['dh32'] = f(B, 1024)           # the unfused head backward writes fp32; converted for the bf16 GEMMs
+    for i, (k, s, ci, co, h, oh, pad) in enumerate(self.convs, 1):
+      g[f'dy{i}'] = a(B, oh, oh, co)
+    return g
+
   def features(self, obs, bufs, before_fc1=None, rows=None):
     """The torso and the first dense layer of both streams: obs -> bufs['h'] (post-ReLU, fp32 [B, 1024]).
     obs: uint8 or float32 [B, H, W, C] (NHWC); uint8 is read as float32(x)/255.  `rows`: the frames' row image from
     prepare_frames() (required in the bf16 dataflow; built here if absent).  `before_fc1` (optional callable) runs after
     the torso has been issued and before the dense layer: the pipelined data-parallel learner makes the stream wait there
     for the fc1 + head parameters, which arrive while the convolutions run."""
-    import torch
     B, P, st = bufs['B'], self.params, _capi.current_stream()
     ws, wsb = self.ws
+    x = self._torso_forward(obs, bufs, rows)
     if self.flow:
-      P.ensure_shadow()
-      if rows is None:
-        if obs.dtype != torch.uint8:
-          raise ValueError('the bf16 dataflow reads uint8 frames')
-        rows = self.prepare_frames(obs, 'fwd')
-      x, x_rows = rows.data_ptr(), 1
-      self._mark(f'fwd{B}.start')
-      for i in range(3):
-        y = bufs[f'y{i + 1}']
-        _capi.call('b200rl_conv2d_fwd_bf16', x, x_rows, P.sp(f'conv{i + 1}.w'), P.p(f'conv{i + 1}.b'), y.data_ptr(), 1,
-                   self.geom(i, B), ACT_RELU, ws, wsb, st)
-        self._mark(f'fwd{B}.conv{i + 1}')
-        x, x_rows = y.data_ptr(), 0
       if before_fc1 is not None:
         before_fc1()
       _capi.call('b200rl_linear_fwd_bf16', B, 1024, self.flat_dim, x, self.flat_dim, P.sp('fc1.w'), P.p('fc1.b'),
                  bufs['h'].data_ptr(), 1024, 0, ACT_RELU, ws, wsb, st)
       self._mark(f'fwd{B}.fc1')
       return bufs['h']
-    x, x_u8 = obs.data_ptr(), int(obs.dtype == torch.uint8)
-    if rows is not None:              # the frames' row image from prepare_frames()
-      x, x_u8 = rows.data_ptr(), 2
-    for i in range(3):
-      y = bufs[f'y{i + 1}']
-      _conv_fwd(x, x_u8, P.p(f'conv{i + 1}.w'), P.p(f'conv{i + 1}.b'), y.data_ptr(), self.geom(i, B), ACT_RELU, self)
-      x, x_u8 = y.data_ptr(), 0
     if before_fc1 is not None:
       before_fc1()
     h = bufs['h']
@@ -529,49 +605,6 @@ class DQNAtariNetwork(Network):
     else:
       _linear_dgrad(B, 1024, self.flat_dim, gbufs['dh'].data_ptr(), 1024, P.p('fc1.w'), gbufs['dy3'].data_ptr(), self.flat_dim,
                     bufs['y3'].data_ptr(), ACT_RELU, self)
-
-  def _conv_bias_grad(self, i, bufs, gbufs):
-    """bf16 dataflow: db of conv layer i+1 = column sums of dy, as its own launch (so it can sit on another stream)."""
-    B, P = bufs['B'], self.params
-    ws, wsb = self.ws
-    _, _, _, co, _, oh, _ = self.convs[i]
-    _capi.call('b200rl_colsum_bf16', B * oh * oh, co, gbufs[f'dy{i + 1}'].data_ptr(), co, P.g(f'conv{i + 1}.b'), ws, wsb,
-               _capi.current_stream())
-
-  def _conv_wgrad(self, i, obs, bufs, gbufs, rows, bias: bool = True):
-    import torch
-    B, P = bufs['B'], self.params
-    ws, wsb = self.ws
-    g = self.geom(i, B)
-    dy = gbufs[f'dy{i + 1}'].data_ptr()
-    if self.flow:
-      if i > 0:
-        x, x_rows = bufs[f'y{i}'].data_ptr(), 0
-      else:
-        if rows is None:
-          rows = self.prepare_frames(obs, 'bwd')
-        x, x_rows = rows.data_ptr(), 1
-      _capi.call('b200rl_conv2d_wgrad_bf16', x, x_rows, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b') if bias else None, g,
-                 ws, wsb, _capi.current_stream())
-      return
-    if i > 0:
-      x, x_u8 = bufs[f'y{i}'].data_ptr(), 0
-    elif rows is not None:
-      x, x_u8 = rows.data_ptr(), 2
-    else:
-      x, x_u8 = obs.data_ptr(), int(obs.dtype == torch.uint8)
-    _conv_wgrad(x, x_u8, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b'), g, self)
-
-  def _conv_dgrad(self, i, bufs, gbufs):
-    B, P = bufs['B'], self.params
-    ws, wsb = self.ws
-    g = self.geom(i, B)
-    dy = gbufs[f'dy{i + 1}'].data_ptr()
-    if self.flow:
-      _capi.call('b200rl_conv2d_dgrad_bf16', dy, P.sp(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), 1, g,
-                 bufs[f'y{i}'].data_ptr(), 1, ACT_RELU, _capi.current_stream())
-    else:
-      _conv_dgrad(dy, P.p(f'conv{i + 1}.w'), gbufs[f'dy{i}'].data_ptr(), g, bufs[f'y{i}'].data_ptr(), ACT_RELU, self)
 
   def backward(self, obs, bufs, gbufs, dq, rows=None):
     """Accumulates nothing: overwrites params.grad with d(loss)/d(params) given dq [B, A].  `rows`: the row image of
@@ -719,6 +752,60 @@ class DQNAtariNetwork(Network):
     self.lane(0)
 
 
+# =============================================================================== AtariTorso as an observation network
+class AtariTorso(_ConvTorso):
+  """AtariTorso (atari.py:36-52): three SAME-padded convolutions with ReLU, flattened in (H, W, C) order to `flat_dim`
+  (7744 at 84 x 84) features.  The observation network of D4PG / DDPG from pixels (d4pg/learning.py:189-195): its
+  output feeds the policy and the critic, whose first layers read it directly.  Features are fp32 at precisions 0, 1 and
+  3, bf16 at precision 2 (the bf16 dataflow, which reads uint8 frames)."""
+
+  def __init__(self, device: int = 0, precision: int = _capi.PRECISION_FP32, seed: int = 0, input_hw: int = 84,
+               input_channels: int = 4):
+    super().__init__(device, precision)
+    self._declare_convs(input_hw, input_channels)
+    self._export = {}
+    for i in range(1, 4):
+      self._export[f'conv{i}/w'] = (f'conv{i}.w', 'conv')
+      self._export[f'conv{i}/b'] = (f'conv{i}.b', None)
+    self._finalize()
+    self._init_convs(np.random.default_rng(seed))
+    if self.flow:
+      self.params.ensure_shadow()
+
+  def make_buffers(self, B: int):
+    import torch
+    dev = torch.device('cuda', self.device)
+    dt = torch.bfloat16 if self.flow else torch.float32
+    bufs = dict(B=B)
+    for i, (k, s, ci, co, h, oh, pad) in enumerate(self.convs, 1):
+      bufs[f'y{i}'] = torch.empty((B, oh, oh, co), dtype=dt, device=dev)
+    self._size_lanes(B)
+    return bufs
+
+  def make_grad_buffers(self, B: int):
+    import torch
+    dev = torch.device('cuda', self.device)
+    dt = torch.bfloat16 if self.flow else torch.float32
+    return {f'dy{i}': torch.empty((B, oh, oh, co), dtype=dt, device=dev)
+            for i, (k, s, ci, co, h, oh, pad) in enumerate(self.convs, 1)}
+
+  def _x3_calls(self, B: int):
+    return self._conv_x3_calls(B)
+
+  def forward(self, obs, bufs, rows=None):
+    """obs [B, H, W, C] -> the features bufs['y3'] [B, OH, OW, 64] (read as [B, flat_dim])."""
+    self._torso_forward(obs, bufs, rows)
+    return bufs['y3']
+
+  def backward(self, obs, bufs, gbufs, rows=None):
+    """Overwrites params.grad from gbufs['dy3'], the gradient w.r.t. conv3's pre-activation (the caller's data gradient
+    of the features, already masked by conv3's ReLU): conv3 and conv2 data gradients and the three weight gradients."""
+    for i in (2, 1, 0):
+      self._conv_wgrad(i, obs, bufs, gbufs, rows)
+      if i > 0:
+        self._conv_dgrad(i, bufs, gbufs)
+
+
 # =============================================================================== plain MLP Q-net
 class MLPQNetwork(Network):
   """snt.Sequential([snt.Flatten(), snt.nets.MLP(sizes)]) with ReLU between layers."""
@@ -801,6 +888,7 @@ class LayerNormMLP(Network):
   bf16 weight shadow and pass bf16 gradients back (tcgen05 kind::f16); the head's forward is a bf16 GEMM with an fp32
   output, its backward one `b200rl_dense_head_bwd_bf16` launch.  Weight gradients, biases and the master weights are fp32.
   """
+  act_in = 0     # width of the first layer's separate action block (split_action_input), 0: none
 
   def __init__(self, input_dim: int, sizes, head_dim: int, head_name: str, head_scale: Optional[float],
                device: int, precision: int, seed: int):
@@ -879,9 +967,80 @@ class LayerNormMLP(Network):
     f = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
     a = (lambda *shape: torch.empty(shape, dtype=torch.bfloat16, device=dev)) if self.flow else f
     g = dict(dz0=f(B, self.sizes[0]), dx=f(B, self.in_dim))
+    if self.act_in:
+      g['da'] = f(B, self.act_in)
+    if self.flow:
+      g['dz0_bf16'] = a(B, self.sizes[0])
     for i in range(len(self.sizes)):
       g[f'dy{i}'] = a(B, self.sizes[i]) if i > 0 else f(B, self.sizes[i])   # dy0 feeds the fp32 LayerNorm backward
     return g
+
+  def _hidden_forward(self, bufs):
+    """The layers after the first one's LayerNorm + tanh (bufs['y0'], or ['y0_bf16'] in the bf16 dataflow): the ELU
+    layers and the head -> bufs['out']."""
+    B, P, st = bufs['B'], self.params, _capi.current_stream()
+    ws, wsb = self.ws
+    h0 = self.sizes[0]
+    if self.flow:
+      x, d = bufs['y0_bf16'].data_ptr(), h0
+      for i in range(1, len(self.sizes)):
+        y = bufs[f'y{i}']
+        _capi.call('b200rl_linear_fwd_bf16', B, self.sizes[i], d, x, d, P.sp(f'l{i}.w'), P.p(f'l{i}.b'), y.data_ptr(),
+                   self.sizes[i], 1, ACT_ELU, ws, wsb, st)
+        x, d = y.data_ptr(), self.sizes[i]
+      _capi.call('b200rl_linear_fwd_bf16', B, self.head_dim, d, x, d, P.sp(f'{self.head}.w'), P.p(f'{self.head}.b'),
+                 bufs['out'].data_ptr(), self.head_dim, 0, ACT_NONE, ws, wsb, st)
+      return bufs['out']
+    x, d = bufs['y0'].data_ptr(), h0
+    for i in range(1, len(self.sizes)):
+      y = bufs[f'y{i}']
+      _linear(B, self.sizes[i], d, x, d, P.p(f'l{i}.w'), P.p(f'l{i}.b'), y.data_ptr(), self.sizes[i], ACT_ELU, self)
+      x, d = y.data_ptr(), self.sizes[i]
+    _linear(B, self.head_dim, d, x, d, P.p(f'{self.head}.w'), P.p(f'{self.head}.b'), bufs['out'].data_ptr(),
+            self.head_dim, ACT_NONE, self)
+    return bufs['out']
+
+  def _hidden_backward(self, bufs, gbufs, dout_ptr: int, param_grads: bool) -> int:
+    """Backward through the head and the ELU layers: returns the address of dy0, the fp32 gradient w.r.t. y0."""
+    B, P, st = bufs['B'], self.params, _capi.current_stream()
+    ws, wsb = self.ws
+    n = len(self.sizes)
+    d_last = self.sizes[-1]
+    if self.flow:
+      last = bufs[f'y{n - 1}'].data_ptr()
+      dy = gbufs[f'dy{n - 1}'].data_ptr()
+      _capi.call('b200rl_dense_head_bwd_bf16', B, self.head_dim, d_last, dout_ptr, self.head_dim, last, d_last,
+                 P.sp(f'{self.head}.w'), dy, d_last, last, ACT_ELU, P.g(f'{self.head}.w') if param_grads else None,
+                 P.g(f'{self.head}.b') if param_grads else None, ws, wsb, st)
+      for i in range(n - 1, 0, -1):
+        hdim, d = self.sizes[i], self.sizes[i - 1]
+        x = bufs[f'y{i - 1}'].data_ptr() if i > 1 else bufs['y0_bf16'].data_ptr()
+        if param_grads:
+          _capi.call('b200rl_linear_wgrad_bf16', B, hdim, d, dy, hdim, x, d, P.g(f'l{i}.w'), P.g(f'l{i}.b'), ws, wsb, st)
+        dx = gbufs[f'dy{i - 1}'].data_ptr()
+        # into y0 (tanh(LN(.)), handled by the fp32 LayerNorm backward): fp32, no mask
+        _capi.call('b200rl_linear_dgrad_bf16', B, hdim, d, dy, hdim, P.sp(f'l{i}.w'), dx, d, int(i > 1), x if i > 1 else None,
+                   1, ACT_ELU, ws, wsb, st)
+        dy = dx
+      return dy
+    last = bufs[f'y{n - 1}'] if n > 1 else bufs['y0']
+    if param_grads:
+      _linear_wgrad(B, self.head_dim, d_last, dout_ptr, self.head_dim, last.data_ptr(), d_last,
+                    P.g(f'{self.head}.w'), P.g(f'{self.head}.b'), self)
+    dy = gbufs[f'dy{n - 1}'].data_ptr()
+    _linear_dgrad(B, self.head_dim, d_last, dout_ptr, self.head_dim, P.p(f'{self.head}.w'), dy, d_last,
+                  last.data_ptr(), ACT_ELU if n > 1 else ACT_NONE, self)
+    for i in range(n - 1, 0, -1):
+      hdim, d = self.sizes[i], self.sizes[i - 1]
+      x = bufs[f'y{i - 1}']
+      if param_grads:
+        _linear_wgrad(B, hdim, d, dy, hdim, x.data_ptr(), d, P.g(f'l{i}.w'), P.g(f'l{i}.b'), self)
+      dx = gbufs[f'dy{i - 1}'].data_ptr()
+      # y_{i-1} is ELU output for i-1 >= 1; for i-1 == 0 it is tanh(LN(.)), handled by the LN backward
+      _linear_dgrad(B, hdim, d, dy, hdim, P.p(f'l{i}.w'), dx, d, x.data_ptr() if i - 1 >= 1 else None,
+                    ACT_ELU, self)
+      dy = dx
+    return dy
 
   def _forward_flat_bf16(self, x_ptr: int, bufs):
     B, P, st = bufs['B'], self.params, _capi.current_stream()
@@ -891,36 +1050,12 @@ class LayerNormMLP(Network):
                ACT_NONE, _capi.PRECISION_TC, ws, wsb, st)
     _capi.call('b200rl_layernorm_tanh_fwd_bf16', B, h0, bufs['z0'].data_ptr(), P.p('ln.scale'), P.p('ln.offset'), 1e-5,
                bufs['y0'].data_ptr(), bufs['y0_bf16'].data_ptr(), bufs['xhat'].data_ptr(), bufs['rstd'].data_ptr(), st)
-    x, d = bufs['y0_bf16'].data_ptr(), h0
-    for i in range(1, len(self.sizes)):
-      y = bufs[f'y{i}']
-      _capi.call('b200rl_linear_fwd_bf16', B, self.sizes[i], d, x, d, P.sp(f'l{i}.w'), P.p(f'l{i}.b'), y.data_ptr(), self.sizes[i],
-                 1, ACT_ELU, ws, wsb, st)
-      x, d = y.data_ptr(), self.sizes[i]
-    _capi.call('b200rl_linear_fwd_bf16', B, self.head_dim, d, x, d, P.sp(f'{self.head}.w'), P.p(f'{self.head}.b'),
-               bufs['out'].data_ptr(), self.head_dim, 0, ACT_NONE, ws, wsb, st)
-    return bufs['out']
+    return self._hidden_forward(bufs)
 
   def _backward_flat_bf16(self, x_ptr: int, bufs, gbufs, dout_ptr: int, param_grads: bool, input_grad: bool):
     B, P, st = bufs['B'], self.params, _capi.current_stream()
     ws, wsb = self.ws
-    n = len(self.sizes)
-    d_last = self.sizes[-1]
-    last = bufs[f'y{n - 1}'].data_ptr()
-    dy = gbufs[f'dy{n - 1}'].data_ptr()
-    _capi.call('b200rl_dense_head_bwd_bf16', B, self.head_dim, d_last, dout_ptr, self.head_dim, last, d_last,
-               P.sp(f'{self.head}.w'), dy, d_last, last, ACT_ELU, P.g(f'{self.head}.w') if param_grads else None,
-               P.g(f'{self.head}.b') if param_grads else None, ws, wsb, st)
-    for i in range(n - 1, 0, -1):
-      hdim, d = self.sizes[i], self.sizes[i - 1]
-      x = bufs[f'y{i - 1}'].data_ptr() if i > 1 else bufs['y0_bf16'].data_ptr()
-      if param_grads:
-        _capi.call('b200rl_linear_wgrad_bf16', B, hdim, d, dy, hdim, x, d, P.g(f'l{i}.w'), P.g(f'l{i}.b'), ws, wsb, st)
-      dx = gbufs[f'dy{i - 1}'].data_ptr()
-      # into y0 (tanh(LN(.)), handled by the fp32 LayerNorm backward): fp32, no mask
-      _capi.call('b200rl_linear_dgrad_bf16', B, hdim, d, dy, hdim, P.sp(f'l{i}.w'), dx, d, int(i > 1), x if i > 1 else None, 1,
-                 ACT_ELU, ws, wsb, st)
-      dy = dx
+    dy = self._hidden_backward(bufs, gbufs, dout_ptr, param_grads)
     h0 = self.sizes[0]
     _capi.call('b200rl_layernorm_tanh_bwd', B, h0, dy, bufs['y0'].data_ptr(), bufs['xhat'].data_ptr(),
                bufs['rstd'].data_ptr(), P.p('ln.scale'), gbufs['dz0'].data_ptr(),
@@ -941,14 +1076,7 @@ class LayerNormMLP(Network):
     _linear(B, h0, self.in_dim, x_ptr, self.in_dim, P.p('l0.w'), P.p('l0.b'), bufs['z0'].data_ptr(), h0, ACT_NONE, self)
     _capi.call('b200rl_layernorm_tanh_fwd', B, h0, bufs['z0'].data_ptr(), P.p('ln.scale'), P.p('ln.offset'), 1e-5,
                bufs['y0'].data_ptr(), bufs['xhat'].data_ptr(), bufs['rstd'].data_ptr(), st)
-    x, d = bufs['y0'].data_ptr(), h0
-    for i in range(1, len(self.sizes)):
-      y = bufs[f'y{i}']
-      _linear(B, self.sizes[i], d, x, d, P.p(f'l{i}.w'), P.p(f'l{i}.b'), y.data_ptr(), self.sizes[i], ACT_ELU, self)
-      x, d = y.data_ptr(), self.sizes[i]
-    _linear(B, self.head_dim, d, x, d, P.p(f'{self.head}.w'), P.p(f'{self.head}.b'), bufs['out'].data_ptr(),
-            self.head_dim, ACT_NONE, self)
-    return bufs['out']
+    return self._hidden_forward(bufs)
 
   def backward_flat(self, x_ptr: int, bufs, gbufs, dout_ptr: int, param_grads: bool = True, input_grad: bool = False):
     """dout: gradient w.r.t. the head output.  Writes params.grad (if param_grads) and gbufs['dx']
@@ -956,25 +1084,7 @@ class LayerNormMLP(Network):
     if self.flow:
       return self._backward_flat_bf16(x_ptr, bufs, gbufs, dout_ptr, param_grads, input_grad)
     B, P, st = bufs['B'], self.params, _capi.current_stream()
-    n = len(self.sizes)
-    d_last = self.sizes[-1]
-    last = bufs[f'y{n - 1}'] if n > 1 else bufs['y0']
-    if param_grads:
-      _linear_wgrad(B, self.head_dim, d_last, dout_ptr, self.head_dim, last.data_ptr(), d_last,
-                    P.g(f'{self.head}.w'), P.g(f'{self.head}.b'), self)
-    dy = gbufs[f'dy{n - 1}'].data_ptr()
-    _linear_dgrad(B, self.head_dim, d_last, dout_ptr, self.head_dim, P.p(f'{self.head}.w'), dy, d_last,
-                  last.data_ptr(), ACT_ELU if n > 1 else ACT_NONE, self)
-    for i in range(n - 1, 0, -1):
-      hdim, d = self.sizes[i], self.sizes[i - 1]
-      x = bufs[f'y{i - 1}']
-      if param_grads:
-        _linear_wgrad(B, hdim, d, dy, hdim, x.data_ptr(), d, P.g(f'l{i}.w'), P.g(f'l{i}.b'), self)
-      dx = gbufs[f'dy{i - 1}'].data_ptr()
-      # y_{i-1} is ELU output for i-1 >= 1; for i-1 == 0 it is tanh(LN(.)), handled by the LN backward
-      _linear_dgrad(B, hdim, d, dy, hdim, P.p(f'l{i}.w'), dx, d, x.data_ptr() if i - 1 >= 1 else None,
-                    ACT_ELU, self)
-      dy = dx
+    dy = self._hidden_backward(bufs, gbufs, dout_ptr, param_grads)
     h0 = self.sizes[0]
     _capi.call('b200rl_layernorm_tanh_bwd', B, h0, dy, bufs['y0'].data_ptr(), bufs['xhat'].data_ptr(),
                bufs['rstd'].data_ptr(), P.p('ln.scale'), gbufs['dz0'].data_ptr(),
@@ -984,6 +1094,75 @@ class LayerNormMLP(Network):
       _linear_wgrad(B, h0, self.in_dim, dz0, h0, x_ptr, self.in_dim, P.g('l0.w'), P.g('l0.b'), self)
     if input_grad:
       _linear_dgrad(B, h0, self.in_dim, dz0, h0, P.p('l0.w'), gbufs['dx'].data_ptr(), self.in_dim, None, ACT_NONE, self)
+
+  # ---- over observation-network features (d4pg/learning.py:189-195): the first layer's feature block is a GEMM on the
+  # features as the observation network wrote them (bf16 at precision 2), its action block (critics, after
+  # split_action_input) and bias, LayerNorm and tanh one b200rl_feature_layer_fwd launch.
+  def split_action_input(self):
+    """Critic over observation-network features: stores the first layer as two blocks, w_f [h0][obs_dim] ('l0.w') and
+    w_a [h0][act_dim] ('l0a.w'), instead of one matrix over the concatenated [obs, act] row, which at obs_dim = 7744 is
+    neither 16-byte aligned (TMA) nor bf16.  Values and the Sonnet export (one `l0/w` [obs_dim + act_dim, h0], features
+    first as CriticMultiplexer concatenates) are unchanged.  Call before buffers are made and graphs captured."""
+    if self.act_in:
+      return
+    values = self.variables()
+    old, P = self.params, ParamStore(self.device)
+    for name, (_, shape) in old.entries.items():
+      if name == 'l0.w':
+        P.declare('l0.w', (shape[0], self.obs_dim))
+        P.declare('l0a.w', (shape[0], self.act_dim))
+      else:
+        P.declare(name, shape)
+    P.allocate()
+    self.params, self.in_dim, self.act_in = P, self.obs_dim, self.act_dim
+    self._export = dict(self._export, **{'l0/w': ('l0.w', ('cat', 'l0a.w'))})
+    self.load_variables(values)
+    if old.shadow is not None:
+      P.ensure_shadow()
+
+  def forward_features(self, feat_ptr: int, act_ptr, bufs):
+    """feat [B, in_dim] (bf16 at precision 2, else fp32) and, after split_action_input(), act [B, act_dim] fp32 ->
+    bufs['out']."""
+    B, P, st = bufs['B'], self.params, _capi.current_stream()
+    ws, wsb = self.ws
+    h0, F = self.sizes[0], self.in_dim
+    zf = bufs['z0'].data_ptr()
+    if self.flow:
+      _capi.call('b200rl_linear_fwd_bf16', B, h0, F, feat_ptr, F, P.sp('l0.w'), None, zf, h0, 0, ACT_NONE, ws, wsb, st)
+    else:
+      _linear(B, h0, F, feat_ptr, F, P.p('l0.w'), None, zf, h0, ACT_NONE, self)
+    _capi.call('b200rl_feature_layer_fwd', B, h0, self.act_in, zf, act_ptr if self.act_in else None,
+               P.p('l0a.w') if self.act_in else None, P.p('l0.b'), P.p('ln.scale'), P.p('ln.offset'), 1e-5,
+               bufs['y0'].data_ptr(), bufs['y0_bf16'].data_ptr() if self.flow else None, bufs['xhat'].data_ptr(),
+               bufs['rstd'].data_ptr(), st)
+    return self._hidden_forward(bufs)
+
+  def backward_features(self, feat_ptr: int, act_ptr, bufs, gbufs, dout_ptr: int, param_grads: bool = True,
+                        action_grad: bool = False, feat_grad=None):
+    """Backward of forward_features from dout (gradient w.r.t. bufs['out']).  param_grads: params.grad; action_grad:
+    gbufs['da'] = d/d act (only the act_dim input columns); feat_grad = (dx_ptr, relu_y_ptr): the features' data
+    gradient, multiplied by relu'(relu_y) (the observation network's last ReLU), written to dx_ptr in the features' type."""
+    B, P, st = bufs['B'], self.params, _capi.current_stream()
+    ws, wsb = self.ws
+    h0, F, A = self.sizes[0], self.in_dim, self.act_in
+    dy = self._hidden_backward(bufs, gbufs, dout_ptr, param_grads)
+    pg = param_grads
+    dz0, dz0_bf = gbufs['dz0'].data_ptr(), gbufs['dz0_bf16'].data_ptr() if self.flow else None
+    _capi.call('b200rl_feature_layer_bwd', B, h0, A, dy, bufs['y0'].data_ptr(), bufs['xhat'].data_ptr(),
+               bufs['rstd'].data_ptr(), P.p('ln.scale'), act_ptr if A else None, P.p('l0a.w') if A else None, dz0, dz0_bf,
+               P.g('ln.scale') if pg else None, P.g('ln.offset') if pg else None, P.g('l0.b') if pg else None,
+               P.g('l0a.w') if pg and A else None, gbufs['da'].data_ptr() if action_grad else None, ws, wsb, st)
+    if pg:
+      if self.flow:
+        _capi.call('b200rl_linear_wgrad_bf16', B, h0, F, dz0_bf, h0, feat_ptr, F, P.g('l0.w'), None, ws, wsb, st)
+      else:
+        _linear_wgrad(B, h0, F, dz0, h0, feat_ptr, F, P.g('l0.w'), None, self)
+    if feat_grad is not None:
+      dx, relu_y = feat_grad
+      if self.flow:
+        _capi.call('b200rl_linear_dgrad_bf16', B, h0, F, dz0_bf, h0, P.sp('l0.w'), dx, F, 1, relu_y, 1, ACT_RELU, ws, wsb, st)
+      else:
+        _linear_dgrad(B, h0, F, dz0, h0, P.p('l0.w'), dx, F, relu_y, ACT_RELU, self)
 
 
 class D4PGCritic(LayerNormMLP):
@@ -1039,13 +1218,26 @@ class D4PGPolicy(LayerNormMLP):
     bufs['dpre'] = torch.empty_like(bufs['a'])
     return bufs
 
-  def action(self, obs, bufs):
-    pre = self.forward_flat(obs.data_ptr(), bufs)
+  def _to_spec(self, pre, bufs):
     _capi.call('b200rl_tanh_to_spec_fwd', bufs['B'], self.act_dim, pre.data_ptr(), self.scale.data_ptr(),
                self.offset.data_ptr(), bufs['a'].data_ptr(), _capi.current_stream())
     return bufs['a']
 
-  def backward_action(self, obs, bufs, gbufs, da):
+  def _to_spec_bwd(self, bufs, da):
     _capi.call('b200rl_tanh_to_spec_bwd', bufs['B'], self.act_dim, da.data_ptr(), bufs['out'].data_ptr(),
                self.scale.data_ptr(), bufs['dpre'].data_ptr(), _capi.current_stream())
+
+  def action(self, obs, bufs):
+    return self._to_spec(self.forward_flat(obs.data_ptr(), bufs), bufs)
+
+  def backward_action(self, obs, bufs, gbufs, da):
+    self._to_spec_bwd(bufs, da)
     self.backward_flat(obs.data_ptr(), bufs, gbufs, bufs['dpre'].data_ptr(), param_grads=True, input_grad=False)
+
+  def action_features(self, feat_ptr: int, bufs):
+    """The action from observation-network features (see LayerNormMLP.forward_features)."""
+    return self._to_spec(self.forward_features(feat_ptr, None, bufs), bufs)
+
+  def backward_action_features(self, feat_ptr: int, bufs, gbufs, da):
+    self._to_spec_bwd(bufs, da)
+    self.backward_features(feat_ptr, None, bufs, gbufs, bufs['dpre'].data_ptr(), param_grads=True)

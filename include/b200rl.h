@@ -382,6 +382,24 @@ int b200rl_layernorm_tanh_fwd(int32_t B, int32_t N, const float* x, const float*
 int b200rl_layernorm_tanh_bwd(int32_t B, int32_t N, const float* dy, const float* y, const float* xhat,
                               const float* rstd, const float* scale, float* dx, float* dscale,
                               float* doffset, void* stream);
+/* The first LayerNormMLP layer over observation-network features (d4pg/learning.py:189-195 then
+ * multiplexers.py:58-80 + continuous.py:37-58), its weight stored as two blocks w_f [N][F] and w_a [N][A]:
+ *   fwd: z0 = zf + a @ w_a^T + bias, then LayerNorm (eps) + tanh with b200rl_layernorm_tanh_fwd's arithmetic.
+ *        zf [B, N] = features @ w_f^T comes from a GEMM with an fp32 output.  Writes y, xhat, rstd and, when y_bf16 is
+ *        not NULL, RN-bf16(y).  A = 0 (a policy: no action input) leaves a and w_a unread.
+ *   bwd: dz [B, N] = the LayerNorm + tanh backward of dy (b200rl_layernorm_tanh_bwd's arithmetic), also as RN-bf16(dz)
+ *        when dz_bf16 is not NULL (the operand of the bf16 weight-gradient GEMM); da [B, A] = dz @ w_a when da is not
+ *        NULL; and, when requested together (all NULL: none), d scale, d offset, db = sum over the batch of dz and
+ *        dw_a [N][A] = dz^T a.  The batch sums run in a fixed order through `ws` (N * (3 + A) * 4 bytes per 8 rows) with
+ *        a per-stream last-CTA ticket: bit-identical across launches, streams and CUDA-graph replay.
+ * 1 <= N <= 1024, 0 <= A <= 64; anything else is B200RL_EINVAL without a launch. */
+int b200rl_feature_layer_fwd(int32_t B, int32_t N, int32_t A, const float* zf, const float* a, const float* w_a,
+                             const float* bias, const float* scale, const float* offset, float eps, float* y,
+                             void* y_bf16, float* xhat, float* rstd, void* stream);
+int b200rl_feature_layer_bwd(int32_t B, int32_t N, int32_t A, const float* dy, const float* y, const float* xhat,
+                             const float* rstd, const float* scale, const float* a, const float* w_a, float* dz,
+                             void* dz_bf16, float* dscale, float* doffset, float* db, float* dw_a, float* da,
+                             void* ws, int64_t ws_bytes, void* stream);
 /* TanhToSpec (rescaling.py:63-74): a = 0.5*(tanh(x)+1)*scale + offset; bwd: dx = da*0.5*scale*(1-tanh^2) */
 int b200rl_tanh_to_spec_fwd(int32_t B, int32_t A, const float* x, const float* scale,
                             const float* offset, float* a, void* stream);

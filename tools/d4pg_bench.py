@@ -10,7 +10,12 @@ d4pg` keeps measuring precision 1.
 
 `--replay prioritized` adds the opt-in prioritized learner (a Prioritized(0.6) table, importance_sampling_exponent 0.4,
 priorities written back every step) beside the uniform one; the two arms read separate tables with identical contents
-and alternate with the precisions.  Its results go to d4pg_bench_<precision>_prioritized.json."""
+and alternate with the precisions.  Its results go to d4pg_bench_<precision>_prioritized.json.
+
+`--observation atari` times D4PG from pixels instead: uint8 84 x 84 x 4 frames through an AtariTorso observation network,
+6-d actions, critic (512, 512, 256) with 51 atoms, policy (256, 256, 256), batch 256, n = 5, at any of fp32, tf32, bf16,
+fp32x3.  Each line adds the step's FLOP count (computed from the shapes by `pixel_step_flop`) and the achieved TFLOP/s.
+Results go to d4pg_bench_pixels_<precision>.json."""
 import argparse
 import json
 import os
@@ -24,7 +29,8 @@ import torch
 
 from acme_b200 import _capi, adders, d4pg, dm_env, loggers, networks, replay, specs
 
-PRECISIONS = {'fp32': _capi.PRECISION_FP32, 'tf32': _capi.PRECISION_TC, 'bf16': _capi.PRECISION_BF16FLOW}
+PRECISIONS = {'fp32': _capi.PRECISION_FP32, 'tf32': _capi.PRECISION_TC, 'bf16': _capi.PRECISION_BF16FLOW,
+              'fp32x3': _capi.PRECISION_FP32X3}
 
 
 def gpu_info():
@@ -62,6 +68,93 @@ def fill_table(OBS, ACT, n, items, sampler=None):
   return table, server
 
 
+def pixel_step_flop(B, torso, A, critic_sizes, K, policy_sizes):
+  """Multiply-adds x 2 of one pixel learner update: online torso forward + three weight gradients + conv3 / conv2 data
+  gradients, target torso forward; the critic's feature block in three forwards + weight and data gradient, the policy's
+  in two forwards + weight gradient; the remaining critic layers in 3 forwards + 2 (train) + 1 (dq/da) backward GEMMs,
+  the policy's in 2 forwards + 2 backward GEMMs."""
+  conv = [oh * oh * co * k * k * ci for (k, s, ci, co, h, oh, pad) in torso.convs]
+  F = torso.flat_dim
+  rest = lambda sizes, out: sum(a * b for a, b in zip(sizes, list(sizes[1:]) + [out]))
+  mac = (2 * sum(conv) + conv[2] + conv[1] + sum(conv) + 5 * F * critic_sizes[0] + 3 * F * policy_sizes[0] +
+         6 * (rest(critic_sizes, K) + A * critic_sizes[0]) + 4 * rest(policy_sizes, A))
+  return 2 * B * mac
+
+
+def fill_pixel_table(A, n, items):
+  rng = np.random.default_rng(0)
+  spec = specs.EnvironmentSpec(specs.Array((84, 84, 4), np.uint8), specs.BoundedArray((A,), np.float32, -1., 1.),
+                               specs.Array((), np.float32), specs.BoundedArray((), np.float32, 0., 1.))
+  table = replay.Table(replay.DEFAULT_PRIORITY_TABLE, replay.selectors.Uniform(), replay.selectors.Fifo(), max_size=items,
+                       rate_limiter=replay.rate_limiters.MinSize(1), signature=adders.NStepTransitionAdder.signature(spec),
+                       max_window=n, discount=0.99, stage_slots=256)
+  server = replay.Server([table])
+  adder = adders.NStepTransitionAdder(replay.Client(server), n_step=n, discount=0.99)
+  frames = rng.integers(0, 256, (64, 84, 84, 4), dtype=np.uint8)
+  steps = 0
+  while steps < items:
+    adder.add_first(dm_env.restart(frames[steps % 64]))
+    for t in range(100):
+      o = frames[(steps + t * 7) % 64]
+      a = rng.uniform(-1, 1, A).astype(np.float32)
+      adder.add(a, dm_env.termination(np.float32(rng.random()), o) if t == 99 else
+                dm_env.transition(np.float32(rng.random()), o, np.float32(1.)))
+    steps += 100
+    table.flush()
+  return table, server
+
+
+def main_pixels(args, precisions):
+  B, A, n, K = 256, 6, 5, 51
+  table, server = fill_pixel_table(A, n, 20_000)
+  lib = _capi.load()
+  learners, launches, flop = {}, {}, None
+  for p in precisions:
+    torso = networks.AtariTorso(precision=PRECISIONS[p], seed=0)
+    policy = networks.D4PGPolicy(torso.flat_dim, A, seed=1, precision=PRECISIONS[p])
+    critic = networks.D4PGCritic(torso.flat_dim, A, seed=2, precision=PRECISIONS[p])
+    flop = pixel_step_flop(B, torso, A, critic.sizes, K, policy.sizes)
+    ds = replay.ReplayDataset(table, B, seed=11, stratified=False)
+    L = d4pg.D4PGLearner(policy, critic, policy.clone(), critic.clone(), 0.99, target_update_period=100, dataset=ds,
+                         logger=loggers.NoOpLogger(), observation_network=torso, target_observation_network=torso.clone())
+    L.step(fetch_loss=False)
+    torch.cuda.synchronize()
+    n0 = lib.b200rl_launch_count()
+    L.step(fetch_loss=False)
+    torch.cuda.synchronize()
+    launches[p] = int(lib.b200rl_launch_count() - n0)
+    for _ in range(args.warmup):
+      L.step(fetch_loss=False)
+    torch.cuda.synchronize()
+    learners[p] = L
+  ms = {p: [] for p in precisions}
+  e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+  for _ in range(args.reps):
+    for p in precisions:
+      L = learners[p]
+      torch.cuda.synchronize()
+      e0.record()
+      for _ in range(args.steps):
+        L.step(fetch_loss=False)
+      e1.record()
+      torch.cuda.synchronize()
+      ms[p].append(e0.elapsed_time(e1) / args.steps)
+  gpu, power_limit = gpu_info()
+  for p in precisions:
+    med = float(np.median(ms[p]))
+    out = {'workload': 'D4PG from pixels: uint8 84x84x4, AtariTorso, 6-d actions, critic (512, 512, 256) C51, policy '
+                       '(256, 256, 256), batch 256, n=5', 'precision': p, 'precision_mode': PRECISIONS[p],
+           'steps_per_rep': args.steps, 'ms_per_step_reps': ms[p], 'ms_per_step': med, 'updates_per_s': 1e3 / med,
+           'launches_per_eager_step': launches[p], 'gflop_per_step': flop / 1e9, 'achieved_tflop_s': flop / (med * 1e-3) / 1e12,
+           'gpu': gpu, 'power_limit': power_limit}
+    print(json.dumps(out))
+    if args.out:
+      os.makedirs(args.out, exist_ok=True)
+      with open(os.path.join(args.out, f'd4pg_bench_pixels_{p}.json'), 'w') as f:
+        json.dump(out, f, indent=1)
+  server.stop()
+
+
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--precision', default='tf32', help='comma-separated subset of fp32, tf32, bf16')
@@ -70,11 +163,15 @@ def main():
   ap.add_argument('--warmup', type=int, default=20)
   ap.add_argument('--reps', type=int, default=3)
   ap.add_argument('--out', default=None, help='directory for d4pg_bench_<precision>.json')
+  ap.add_argument('--observation', default='state', choices=['state', 'atari'],
+                  help='state: flat 67-d observations; atari: uint8 frames through an AtariTorso observation network')
   args = ap.parse_args()
   precisions = [p.strip() for p in args.precision.split(',') if p.strip()]
   for p in precisions:
-    if p not in PRECISIONS:
-      ap.error(f'unknown precision {p!r} (fp32, tf32, bf16)')
+    if p not in PRECISIONS or (p == 'fp32x3' and args.observation == 'state'):
+      ap.error(f'unknown precision {p!r} (fp32, tf32, bf16; fp32x3 with --observation atari)')
+  if args.observation == 'atari':
+    return main_pixels(args, precisions)
   arms = [r.strip() for r in args.replay.split(',') if r.strip()]
   for r in arms:
     if r not in ('uniform', 'prioritized'):
