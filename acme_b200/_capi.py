@@ -143,6 +143,7 @@ PROTOTYPES = {
     'b200rl_workspace_bytes': (c_i64, [c_i64]),
     'b200rl_conv2d_rows_bytes': (c_i64, [C.POINTER(ConvGeom)]),
     'b200rl_conv2d_rows_from_u8': (c_int, [c_vp, C.POINTER(ConvGeom), c_vp, c_i64, c_vp]),
+    'b200rl_frames_pad_u8': (c_int, [c_vp, c_i64, c_i32, c_i32, c_vp, c_vp]),
     'b200rl_x3_ws_bytes': (c_i64, [c_int, c_i32, c_i32, c_i32, C.POINTER(ConvGeom), c_int]),
     'b200rl_linear_fwd_x3': (c_int, [c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i32, c_int, c_vp, c_i64, c_vp]),
     'b200rl_linear_dgrad_x3': (c_int, [c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_vp, c_i32, c_vp, c_int, c_vp, c_i64, c_vp]),

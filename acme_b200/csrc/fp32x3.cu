@@ -28,6 +28,8 @@ namespace b200rl {
 typedef __nv_bfloat16 bf16;
 int check_geom(const b200rl_conv_geom* g);                        // layers_api.cu
 int check_conv_ptr(const void* p, int u8, const char* what);
+int check_geom_frames(const b200rl_conv_geom* g);
+int rows_cp(int C);
 int h_linear_fwd(int M, int N, int K, const bf16* x, int ldx, const bf16* w, const float* bias, void* y, int ldy, int act,
                  int out_bf16, void* ws, int64_t wsb, cudaStream_t s);   // gemm_bf16.cu
 int h_linear_dgrad(int M, int N, int K, const bf16* dy, int lddy, const bf16* w, void* dx, int lddx, const void* mask, int ldmask,
@@ -140,6 +142,12 @@ enum { PATH_FFMA = 0, PATH_CONCAT = 1, PATH_STACK = 2 };
 static inline int rup(int a, int m) { return (a + m - 1) / m * m; }
 static inline int64_t al256(int64_t b) { return (b + 255) & ~(int64_t)255; }
 static bool rows_geom(const b200rl_conv_geom& g) { return h_rows_bytes(g) > 0; }
+// first layer on frames of C channels: the filter has rows_cp(C) channels (padding columns zero, gemm_bf16.cu)
+static b200rl_conv_geom filter_geom(const b200rl_conv_geom& g) {
+  b200rl_conv_geom f = g;
+  f.C = rows_cp(g.C);
+  return f;
+}
 
 static int path_of(int op, int M, int N, int K, const b200rl_conv_geom* g, int x_u8) {
   switch (op) {
@@ -280,8 +288,13 @@ using namespace b200rl;
 extern "C" int64_t b200rl_x3_ws_bytes(int op, int32_t M, int32_t N, int32_t K, const b200rl_conv_geom* g, int x_u8) {
   if (op < B200RL_X3_LINEAR_FWD || op > B200RL_X3_CONV_DGRAD) return -1;
   if (op >= B200RL_X3_CONV_FWD) {
-    if (!g || check_geom(g) || x_u8 < 0 || x_u8 > 2 || (x_u8 && op == B200RL_X3_CONV_DGRAD)) return -1;
-    if (x_u8 == 2 && !rows_geom(*g)) return -1;
+    if (!g || x_u8 < 0 || x_u8 > 2 || (x_u8 ? check_geom_frames(g) : check_geom(g)) || (x_u8 && op == B200RL_X3_CONV_DGRAD)) return -1;
+    if (x_u8 && (x_u8 == 2 || rows_cp(g->C) != g->C) && !rows_geom(*g)) return -1;
+    if (x_u8) {
+      b200rl_conv_geom gp = filter_geom(*g);
+      const Plan p = plan_of(op, M, N, K, &gp, x_u8);
+      return p.path == PATH_FFMA && rows_cp(g->C) != g->C ? -1 : p.total();
+    }
   } else if (M < 1 || N < 1 || K < 1) {
     return -1;
   }
@@ -340,18 +353,21 @@ extern "C" int b200rl_linear_wgrad_x3(int32_t M, int32_t N, int32_t K, const flo
 }
 
 static int conv_args(const b200rl_conv_geom* g, const void* x, int x_u8) {
-  if (int rc = check_geom(g)) return rc;
   B200RL_REQUIRE(x_u8 >= 0 && x_u8 <= 2, "x_u8 must be 0 (fp32 NHWC), 1 (uint8 frames) or 2 (the bf16 row image)");
-  B200RL_REQUIRE(x_u8 != 2 || rows_geom(*g), "a row image needs the first-layer geometry (C = 4, kw * C = 32, Cout 32 / 64)");
+  if (int rc = x_u8 ? check_geom_frames(g) : check_geom(g)) return rc;
+  B200RL_REQUIRE(!x_u8 || (x_u8 == 1 && rows_cp(g->C) == g->C) || rows_geom(*g),
+                 "frames of C = %d channels need the row-image geometry (kw * Cp = 32, 64 or 128 with Cp = 4, 8 or 16; Cout 32 / 64)", g->C);
   return check_conv_ptr(x, x_u8 == 1, "conv input x");
 }
 
-extern "C" int b200rl_conv2d_fwd_x3(const void* x, int x_u8, const float* w, const float* bias, float* y, const b200rl_conv_geom* g,
+extern "C" int b200rl_conv2d_fwd_x3(const void* x, int x_u8, const float* w, const float* bias, float* y, const b200rl_conv_geom* g_in,
                                     int act, void* ws, int64_t wsb, void* stream) {
   B200RL_REQUIRE(x && w && y, "null argument");
-  if (int rc = conv_args(g, x, x_u8)) return rc;
+  if (int rc = conv_args(g_in, x, x_u8)) return rc;
+  const b200rl_conv_geom gf = x_u8 ? filter_geom(*g_in) : *g_in, *g = &gf;   // the filter's geometry
   const Plan p = plan_of(B200RL_X3_CONV_FWD, 0, 0, 0, g, x_u8);
   if (int rc = check_ws(p, ws, wsb)) return rc;
+  B200RL_REQUIRE(p.path != PATH_FFMA || g->C == g_in->C, "frames of C = %d channels: batch too large for the row-image path", g_in->C);
   if (p.path == PATH_FFMA) return b200rl_conv2d_fwd(x, x_u8, w, bias, y, g, act, 0, ws, p.tail, stream);
   cudaStream_t s = as_stream(stream);
   const int taps = g->kh * g->kw, Kw = taps * g->C;
@@ -366,7 +382,7 @@ extern "C" int b200rl_conv2d_fwd_x3(const void* x, int x_u8, const float* w, con
     if (int rc = launch_split(row_job(w, Kw, g->Cout, Kw, g->Cout, 3, PAT_HML, wb), nullptr, s)) return rc;
     const bf16* rows = (const bf16*)x;
     if (x_u8 == 1) {
-      X3_GEMM(h_rows_from_u8((const uint8_t*)x, *g, img, p.img, s));
+      X3_GEMM(h_rows_from_u8((const uint8_t*)x, *g_in, img, p.img, s));
       rows = img;
     }
     for (int k = 0; k < 3; ++k)
@@ -385,12 +401,14 @@ extern "C" int b200rl_conv2d_fwd_x3(const void* x, int x_u8, const float* w, con
   return B200RL_OK;
 }
 
-extern "C" int b200rl_conv2d_wgrad_x3(const void* x, int x_u8, const float* dy, float* dw, float* db, const b200rl_conv_geom* g,
+extern "C" int b200rl_conv2d_wgrad_x3(const void* x, int x_u8, const float* dy, float* dw, float* db, const b200rl_conv_geom* g_in,
                                       void* ws, int64_t wsb, void* stream) {
   B200RL_REQUIRE(x && dy && dw, "null argument");
-  if (int rc = conv_args(g, x, x_u8)) return rc;
+  if (int rc = conv_args(g_in, x, x_u8)) return rc;
+  const b200rl_conv_geom gf = x_u8 ? filter_geom(*g_in) : *g_in, *g = &gf;   // the filter's geometry
   const Plan p = plan_of(B200RL_X3_CONV_WGRAD, 0, 0, 0, g, x_u8);
   if (int rc = check_ws(p, ws, wsb)) return rc;
+  B200RL_REQUIRE(p.path != PATH_FFMA || g->C == g_in->C, "frames of C = %d channels: batch too large for the row-image path", g_in->C);
   if (p.path == PATH_FFMA) return b200rl_conv2d_wgrad(x, x_u8, dy, dw, db, g, 0, ws, p.tail, stream);
   cudaStream_t s = as_stream(stream);
   const int64_t Mo = (int64_t)g->B * g->OH * g->OW;
@@ -405,7 +423,7 @@ extern "C" int b200rl_conv2d_wgrad_x3(const void* x, int x_u8, const float* dy, 
     if (int rc = launch_split(row_job(dy, per_img, g->B, per_img, g->B, 3, PAT_HML, da), nullptr, s)) return rc;
     const void* src = x;
     if (x_u8 == 1) {
-      X3_GEMM(h_rows_from_u8((const uint8_t*)x, *g, img, ib, s));
+      X3_GEMM(h_rows_from_u8((const uint8_t*)x, *g_in, img, ib, s));
       src = img;
     }
     for (int k = src == img ? 1 : 0; k < 3; ++k)

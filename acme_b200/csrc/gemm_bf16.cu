@@ -606,23 +606,31 @@ int h_conv_wgrad(const bf16* x, const bf16* dy, float* dw, float* db, const b200
   return B200RL_OK;
 }
 
-// ---- first layer on uint8 frames (C = 4, kw * C = 32).  The frames are rewritten once per batch as a zero-padded bf16
+// ---- first layer on uint8 frames.  The frames are rewritten once per batch as a zero-padded bf16
 // ROW IMAGE holding the INTEGER pixel values 0..255 (exact in bf16); the 1/255 of `atari_wrapper.py:303-304` is applied to
-// the fp32 accumulator in the epilogue, so the pixel operand carries no rounding at all.  A filter row (kw * C = 32
-// values = 64 bytes) is contiguous in the padded NHWC row: the convolution is a kh x 1 filter over overlapping
-// 32-channel "wide pixels" (tensor-map stride stride * C elements < extent), loaded by TMA's im2col mode.
-struct RowsView { int Hp, row_elems, wide_stride; int64_t bytes; };
+// the fp32 accumulator in the epilogue, so the pixel operand carries no rounding at all.  A filter row (kw * Cp values)
+// is contiguous in the padded NHWC row: the convolution is a kh x 1 filter over overlapping kw * Cp-channel "wide
+// pixels" (tensor-map stride stride * Cp elements < extent), loaded by TMA's im2col mode in 32- or 64-channel blocks.
+// Frames of C channels (1 <= C <= 16) get Cp = rows_cp(C) in {4, 8, 16} channels per pixel, channels C .. Cp-1 zero,
+// so that a filter row is 32, 64 or 128 values (one 32-channel block, or one / two 64-channel blocks) at kw = 8; the
+// filter is [Cout][kh][kw][Cp].  Atari frames (C = 4) take the original 32-channel kernels unchanged.
+struct RowsView { int Cp, Hp, row_elems, wide_stride, wide; int64_t bytes; };
+int rows_cp(int C) { return C <= 4 ? 4 : (C <= 8 ? 8 : 16); }
 static bool rows_eligible(const b200rl_conv_geom& g) {
-  return g.C == 4 && g.kw * g.C == 32 && (g.Cout == 32 || g.Cout == 64) && (g.stride * g.C * 2) % 16 == 0;
+  if (g.C < 1 || g.C > 16) return false;
+  const int cp = rows_cp(g.C), wide = g.kw * cp;
+  return (wide == 32 || wide == 64 || wide == 128) && (g.Cout == 32 || g.Cout == 64) && (g.stride * cp * 2) % 16 == 0;
 }
 static RowsView rows_view(const b200rl_conv_geom& g) {
   RowsView v;
+  v.Cp = rows_cp(g.C);
   const int pad_bottom = std::max((g.OH - 1) * g.stride + g.kh - g.H - g.pad_top, 0);
   const int pad_right = std::max((g.OW - 1) * g.stride + g.kw - g.W - g.pad_left, 0);
   v.Hp = g.H + g.pad_top + pad_bottom;
-  v.row_elems = (g.W + g.pad_left + pad_right) * g.C;
+  v.row_elems = (g.W + g.pad_left + pad_right) * v.Cp;
   v.row_elems = (v.row_elems + 7) & ~7;          // 16-byte rows
-  v.wide_stride = g.stride * g.C;
+  v.wide_stride = g.stride * v.Cp;
+  v.wide = g.kw * v.Cp;
   v.bytes = (int64_t)g.B * v.Hp * v.row_elems * 2;
   return v;
 }
@@ -662,38 +670,80 @@ u8_rows_to_bf16_kernel(const uint8_t* __restrict__ x, bf16* __restrict__ out, in
     reinterpret_cast<uint4*>(out)[(size_t)row * (per_row >> 1) + q] = make_uint4(w[0], w[1], w[2], w[3]);
   }
 }
-int h_rows_from_u8(const uint8_t* x, const b200rl_conv_geom& g, bf16* rows, int64_t bytes, cudaStream_t s) {
-  if (!rows_eligible(g) || !rows || (((uintptr_t)rows) & 127) != 0) return 1;
+// any C (1..16) into Cp-channel pixels: one thread = 8 consecutive elements of a padded row = one 16-byte store
+__global__ void __launch_bounds__(256)
+u8_rows_to_bf16_c_kernel(const uint8_t* __restrict__ x, uint4* __restrict__ out, int H, int W, int C, int Cp, int Hp,
+                         int row_v16, int pad_left, int pad_top, int64_t total) {
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t row = e / row_v16;
+    const int q = (int)(e - row * row_v16);
+    const int b = (int)(row / Hp), ys = (int)(row - (int64_t)b * Hp) - pad_top;
+    float v[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int el = 8 * q + j, px = el / Cp, c = el - px * Cp, xs = px - pad_left;
+      v[j] = (ys >= 0 && ys < H && xs >= 0 && xs < W && c < C) ? (float)__ldg(x + (((size_t)b * H + ys) * W + xs) * C + c) : 0.f;
+    }
+    uint32_t w[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const __nv_bfloat162 t = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
+      w[j] = *reinterpret_cast<const uint32_t*>(&t);
+    }
+    out[e] = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+}
+// the row image of B frames of g.C channels (no size / alignment checks: callers check them)
+int h_rows_write(const uint8_t* x, const b200rl_conv_geom& g, bf16* rows, cudaStream_t s) {
+  if (!rows_eligible(g)) return 1;
   const RowsView v = rows_view(g);
-  if (v.bytes > bytes) return 1;
-  const int total = g.B * v.Hp, rpc = 8;
-  u8_rows_to_bf16_kernel<<<ceil_div(total, rpc), 256, 0, s>>>(x, rows, g.H, g.W, v.Hp, v.row_elems / g.C, g.pad_left, g.pad_top,
-                                                              total, rpc);
+  if (g.C == 4) {
+    const int total = g.B * v.Hp, rpc = 8;
+    u8_rows_to_bf16_kernel<<<ceil_div(total, rpc), 256, 0, s>>>(x, rows, g.H, g.W, v.Hp, v.row_elems / g.C, g.pad_left, g.pad_top,
+                                                                total, rpc);
+  } else {
+    const int64_t total = (int64_t)g.B * v.Hp * (v.row_elems / 8);
+    const int blocks = (int)std::min<int64_t>(ceil_div<int64_t>(total, 256), 148 * 16);
+    u8_rows_to_bf16_c_kernel<<<blocks, 256, 0, s>>>(x, (uint4*)rows, g.H, g.W, g.C, v.Cp, v.Hp, v.row_elems / 8, g.pad_left,
+                                                   g.pad_top, total);
+  }
   B200RL_LAUNCH_OK();
   return B200RL_OK;
 }
-static bool make_rows_map(CUtensorMap* m, const bf16* rows, const b200rl_conv_geom& g, const RowsView& v, int pixels) {
+int h_rows_from_u8(const uint8_t* x, const b200rl_conv_geom& g, bf16* rows, int64_t bytes, cudaStream_t s) {
+  if (!rows_eligible(g) || !rows || (((uintptr_t)rows) & 127) != 0) return 1;
+  if (rows_view(g).bytes > bytes) return 1;
+  return h_rows_write(x, g, rows, s);
+}
+static bool make_rows_map(CUtensorMap* m, const bf16* rows, const b200rl_conv_geom& g, const RowsView& v, int channels,
+                          int pixels) {
   EncodeIm2colFn enc = get_encode_im2col();
   if (!enc) return false;
-  cuuint64_t dims[4] = {32, (cuuint64_t)g.OW, (cuuint64_t)v.Hp, (cuuint64_t)g.B};
+  cuuint64_t dims[4] = {(cuuint64_t)v.wide, (cuuint64_t)g.OW, (cuuint64_t)v.Hp, (cuuint64_t)g.B};
   cuuint64_t strides[3] = {(cuuint64_t)v.wide_stride * 2, (cuuint64_t)v.row_elems * 2, (cuuint64_t)v.Hp * v.row_elems * 2};
   int lower[2] = {0, 0};
   int upper[2] = {0, -(g.kh - 1)};
   cuuint32_t es[4] = {1, 1, (cuuint32_t)g.stride, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, (void*)rows, dims, strides, lower, upper, 32, (cuuint32_t)pixels, es,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, (void*)rows, dims, strides, lower, upper, (cuuint32_t)channels,
+             (cuuint32_t)pixels, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw_mode(channels * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 static int conv_fwd_rows(const bf16* rows, const bf16* w, const float* bias, void* y, const b200rl_conv_geom& g, int act,
                          int out_bf16, float scale, void* ws, int64_t wsb, cudaStream_t s) {
-  const int M = g.B * g.OH * g.OW, K = g.kh * g.kw * g.C;
-  if (!rows_eligible(g) || !ok16(w, K)) return 1;
+  if (!rows_eligible(g)) return 1;
+  const RowsView v = rows_view(g);
+  const int M = g.B * g.OH * g.OW, K = g.kh * v.wide, KE = v.wide == 32 ? 32 : 64;
+  if (!ok16(w, K)) return 1;
   CUtensorMap ma, mb;
-  if (!make_rows_map(&ma, rows, g, rows_view(g), HBM_ROWS) || !make_map_h(&mb, w, g.Cout, K, K, 32, g.Cout)) return 1;
+  if (!make_rows_map(&ma, rows, g, v, KE, HBM_ROWS) || !make_map_h(&mb, w, g.Cout, K, K, KE, g.Cout)) return 1;
   Epilogue e = make_epi(y, g.Cout, bias, act, nullptr, 0, 0, 0, out_bf16, 0, scale);
-  ConvA conv{1, 32, 1, g.OW, g.OH, 1, g.stride, 0, 0, g.kh};
-  if (g.Cout == 32) return launch_h<32, 0, 0, 32>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
-  return launch_h<32, 0, 0, 64>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
+  ConvA conv{1, v.wide, 1, g.OW, g.OH, 1, g.stride, 0, 0, g.kh};
+  if (KE == 32) {
+    if (g.Cout == 32) return launch_h<32, 0, 0, 32>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
+    return launch_h<32, 0, 0, 64>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
+  }
+  if (g.Cout == 32) return launch_h<64, 0, 0, 32>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
+  return launch_h<64, 0, 0, 64>(ma, mb, e, M, g.Cout, K, ws, wsb, s, conv);
 }
 int h_conv_fwd_rows(const bf16* rows, const bf16* w, const float* bias, void* y, const b200rl_conv_geom& g, int act, int out_bf16,
                     void* ws, int64_t wsb, cudaStream_t s) {
@@ -705,15 +755,19 @@ int h_conv_fwd_rows_raw(const bf16* rows, const bf16* w, float* y, const b200rl_
 }
 int h_conv_wgrad_rows(const bf16* rows, const bf16* dy, float* dw, float* db, const b200rl_conv_geom& g, void* ws, int64_t wsb,
                       cudaStream_t s) {
-  const int M = g.B * g.OH * g.OW, K = g.kh * g.kw * g.C;
   if (!rows_eligible(g) || !ok16(dy, g.Cout)) return 1;
+  const RowsView v = rows_view(g);
+  const int M = g.B * g.OH * g.OW, K = g.kh * v.wide, WB = v.wide == 32 ? 32 : 64;
   CUtensorMap ma, mb;
   const int WBb = g.Cout == 32 ? 32 : 64;
-  if (!make_rows_map(&ma, rows, g, rows_view(g), 64) || !make_map_h(&mb, dy, M, g.Cout, g.Cout, WBb, 64)) return 1;
+  if (!make_rows_map(&ma, rows, g, v, WB, 64) || !make_map_h(&mb, dy, M, g.Cout, g.Cout, WBb, 64)) return 1;
   Epilogue e = make_epi(dw, K, nullptr, 0, nullptr, 0, 0, 1, 0, 0, 1.0f / 255.0f);
-  ConvA conv{1, 32, 1, g.OW, g.OH, 1, g.stride, 0, 0, g.kh};
-  int rc = WBb == 32 ? launch_h<64, 2, 2, 32>(ma, mb, e, K, g.Cout, M, ws, wsb, s, conv)
-                     : launch_h<64, 2, 1, 64>(ma, mb, e, K, g.Cout, M, ws, wsb, s, conv);
+  ConvA conv{1, v.wide, 1, g.OW, g.OH, 1, g.stride, 0, 0, g.kh};
+  int rc;
+  if (WB == 32) rc = WBb == 32 ? launch_h<64, 2, 2, 32>(ma, mb, e, K, g.Cout, M, ws, wsb, s, conv)
+                               : launch_h<64, 2, 1, 64>(ma, mb, e, K, g.Cout, M, ws, wsb, s, conv);
+  else rc = WBb == 32 ? launch_h<64, 1, 2, 32>(ma, mb, e, K, g.Cout, M, ws, wsb, s, conv)
+                      : launch_h<64, 1, 1, 64>(ma, mb, e, K, g.Cout, M, ws, wsb, s, conv);
   if (rc) return rc;
   if (db) return launch_colsum_bf16(M, g.Cout, dy, g.Cout, db, ws, wsb, s);
   return B200RL_OK;

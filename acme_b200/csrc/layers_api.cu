@@ -75,6 +75,7 @@ int h_conv_fwd_rows(const __nv_bfloat16* rows, const __nv_bfloat16* w, const flo
                     int act, int out_bf16, void* ws, int64_t wsb, cudaStream_t s);
 int h_conv_wgrad_rows(const __nv_bfloat16* rows, const __nv_bfloat16* dy, float* dw, float* db, const b200rl_conv_geom& g,
                       void* ws, int64_t wsb, cudaStream_t s);
+int rows_cp(int C);
 int h_f32_to_bf16(int64_t n, const float* src, __nv_bfloat16* dst, cudaStream_t s);
 int launch_colsum_bf16(int M, int N, const __nv_bfloat16* x, int ld, float* out, void* ws, int64_t ws_bytes, cudaStream_t stream);
 }  // namespace b200rl
@@ -98,6 +99,14 @@ int check_geom(const b200rl_conv_geom* g) {
   B200RL_REQUIRE(g->C % 4 == 0 && g->Cout % 4 == 0, "channel counts must be multiples of 4");
   B200RL_REQUIRE((int64_t)g->B * g->H * g->W < (1ll << 31) && (int64_t)g->B * g->OH * g->OW < (1ll << 31), "too many pixels");
   return B200RL_OK;
+}
+// the first layer's input on the row-image paths (uint8 frames or their bf16 row image): any C in [1, 16]
+int check_geom_frames(const b200rl_conv_geom* g) {
+  B200RL_REQUIRE(g, "null geometry");
+  B200RL_REQUIRE(g->C >= 1 && g->C <= 16, "frames must have 1 to 16 channels (C = %d)", g->C);
+  b200rl_conv_geom g4 = *g;
+  g4.C = 4;
+  return check_geom(&g4);
 }
 // The convolution loaders of every precision read an fp32 activation / gradient / filter as float4 (im2col of x; dy and
 // w of the data gradient) and a uint8 frame as one 4-byte pixel (C % 4 == 0), with no alignment test on the device.
@@ -164,6 +173,33 @@ extern "C" int b200rl_conv2d_rows_from_u8(const void* x_u8, const b200rl_conv_ge
   int rc = tma_rows_from_u8((const uint8_t*)x_u8, *g, rows, rows_bytes, as_stream(stream));
   B200RL_REQUIRE(rc != 1, "geometry not eligible for a row image, buffer too small or not 128-byte aligned");
   return rc;
+}
+
+// one thread per 4-byte word of the padded pixels: word q of pixel p holds channels 4q .. 4q+3
+__global__ void __launch_bounds__(256)
+frames_pad_u8_kernel(const uint8_t* __restrict__ x, uint32_t* __restrict__ out, int64_t words, int C, int Cp) {
+  const int wpp = Cp >> 2;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < words; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t p = i / wpp;
+    const int c0 = (int)(i - p * wpp) * 4;
+    const uint8_t* src = x + p * C;
+    uint32_t v = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (c0 + j < C) v |= (uint32_t)__ldg(src + c0 + j) << (8 * j);
+    out[i] = v;
+  }
+}
+extern "C" int b200rl_frames_pad_u8(const void* x_u8, int64_t npix, int32_t C, int32_t Cp, void* out, void* stream) {
+  B200RL_REQUIRE(x_u8 && out && npix >= 0, "bad argument");
+  B200RL_REQUIRE(C >= 1 && C <= Cp && Cp <= 16 && Cp % 4 == 0, "need 1 <= C <= Cp <= 16 and Cp %% 4 == 0 (C = %d, Cp = %d)", C, Cp);
+  if (int rc = check_conv_ptr(out, 1, "padded frames")) return rc;
+  const int64_t words = npix * (Cp / 4);
+  if (words == 0) return B200RL_OK;
+  const int blocks = (int)std::min<int64_t>(ceil_div<int64_t>(words, 256), 148 * 16);
+  frames_pad_u8_kernel<<<blocks, 256, 0, as_stream(stream)>>>((const uint8_t*)x_u8, (uint32_t*)out, words, C, Cp);
+  B200RL_LAUNCH_OK();
+  return B200RL_OK;
 }
 
 extern "C" int b200rl_conv2d_dgrad(const float* dy, const float* w, float* dx, const b200rl_conv_geom* g,
@@ -236,19 +272,19 @@ extern "C" int b200rl_bf16_from_f32(int64_t n, const float* src, void* dst_bf16,
   H_CALL(h_f32_to_bf16(n, src, (bf16_t*)dst_bf16, as_stream(stream)), "bf16_from_f32 (n % 8 == 0, 16-byte aligned)");
 }
 extern "C" int64_t b200rl_conv2d_rows_bf16_bytes(const b200rl_conv_geom* g) {
-  if (!g || check_geom(g)) return 0;
+  if (!g || check_geom_frames(g)) return 0;
   return h_rows_bytes(*g);
 }
 extern "C" int b200rl_conv2d_rows_bf16_from_u8(const void* x_u8, const b200rl_conv_geom* g, void* rows, int64_t rows_bytes,
                                                void* stream) {
   B200RL_REQUIRE(x_u8 && rows, "null argument");
-  if (int rc = check_geom(g)) return rc;
+  if (int rc = check_geom_frames(g)) return rc;
   H_CALL(h_rows_from_u8((const uint8_t*)x_u8, *g, (bf16_t*)rows, rows_bytes, as_stream(stream)), "bf16 row image");
 }
 extern "C" int b200rl_conv2d_fwd_bf16(const void* x, int x_rows, const void* w, const float* bias, void* y, int y_bf16,
                                       const b200rl_conv_geom* g, int act, void* ws, int64_t wsb, void* stream) {
   B200RL_REQUIRE(x && w && y, "null argument");
-  if (int rc = check_geom(g)) return rc;
+  if (int rc = x_rows ? check_geom_frames(g) : check_geom(g)) return rc;
   if (x_rows)
     H_CALL(h_conv_fwd_rows((const bf16_t*)x, (const bf16_t*)w, bias, y, *g, act, y_bf16, ws, wsb, as_stream(stream)), "conv2d_fwd_bf16(rows)");
   H_CALL(h_conv_fwd((const bf16_t*)x, (const bf16_t*)w, bias, y, *g, act, y_bf16, ws, wsb, as_stream(stream)), "conv2d_fwd_bf16");
@@ -256,7 +292,7 @@ extern "C" int b200rl_conv2d_fwd_bf16(const void* x, int x_rows, const void* w, 
 extern "C" int b200rl_conv2d_wgrad_bf16(const void* x, int x_rows, const void* dy, float* dw, float* db, const b200rl_conv_geom* g,
                                         void* ws, int64_t wsb, void* stream) {
   B200RL_REQUIRE(x && dy && dw && ws, "null argument");
-  if (int rc = check_geom(g)) return rc;
+  if (int rc = x_rows ? check_geom_frames(g) : check_geom(g)) return rc;
   if (x_rows)
     H_CALL(h_conv_wgrad_rows((const bf16_t*)x, (const bf16_t*)dy, dw, db, *g, ws, wsb, as_stream(stream)), "conv2d_wgrad_bf16(rows)");
   H_CALL(h_conv_wgrad((const bf16_t*)x, (const bf16_t*)dy, dw, db, *g, ws, wsb, as_stream(stream)), "conv2d_wgrad_bf16");

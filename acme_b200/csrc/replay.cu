@@ -20,6 +20,7 @@
 
 namespace b200rl {
 int h_rows_layout(const b200rl_conv_geom& g, int* Hp, int* row_elems);   // gemm_bf16.cu
+int h_rows_write(const uint8_t* x, const b200rl_conv_geom& g, __nv_bfloat16* rows, cudaStream_t s);
 
 static thread_local std::string g_last_error;
 static unsigned long long g_launches = 0;
@@ -1234,10 +1235,16 @@ extern "C" int b200rl_replay_sample_philox(b200rl_replay* h, int32_t B, uint64_t
                      h->global_mass_dev, idx_dev, keys_dev, prob_dev, as_stream(stream), nullptr);
 }
 
+static int gather_locked(b200rl_replay* h, int32_t B, const int64_t* idx_dev, void* o_tm1, void* a_tm1, float* R, float* D,
+                         void* o_t, void* stream);
 extern "C" int b200rl_replay_gather(b200rl_replay* h, int32_t B, const int64_t* idx_dev, void* o_tm1,
                                     void* a_tm1, float* R, float* D, void* o_t, void* stream) {
   B200RL_REQUIRE(h && idx_dev && o_tm1 && a_tm1 && R && D && o_t, "null argument");
   B200RL_LOCK(h);
+  return gather_locked(h, B, idx_dev, o_tm1, a_tm1, R, D, o_t, stream);
+}
+static int gather_locked(b200rl_replay* h, int32_t B, const int64_t* idx_dev, void* o_tm1, void* a_tm1, float* R, float* D,
+                         void* o_t, void* stream) {
   B200RL_REQUIRE(h->cfg.obs_bytes > 0, "this replay was created without payload storage");
   B200RL_REQUIRE(B >= 1, "batch must be >= 1");
   int rc = ensure_device(h);
@@ -1270,12 +1277,21 @@ extern "C" int b200rl_replay_gather_rows(b200rl_replay* h, int32_t B, const int6
   B200RL_REQUIRE(h && idx_dev && o_tm1 && a_tm1 && R && D && o_t && rows_tm1 && rows_t && g, "null argument");
   B200RL_LOCK(h);
   B200RL_REQUIRE(B >= 1, "batch must be >= 1");
-  B200RL_REQUIRE(g->C == 4 && g->W % 4 == 0 && h->cfg.obs_bytes == g->H * g->W * g->C,
-                 "gather_rows: the table's observations are not [H][W][4] uint8 frames of this geometry");
-  B200RL_REQUIRE(g->pad_left % 2 == 0, "gather_rows: pad_left must be even (16-byte aligned pixel pairs)");
+  B200RL_REQUIRE(g->C >= 1 && g->C <= 16 && h->cfg.obs_bytes == g->H * g->W * g->C,
+                 "gather_rows: the table's observations are not [H][W][C] uint8 frames of this geometry (1 <= C <= 16)");
   int Hp = 0, row_elems = 0;
   B200RL_REQUIRE(h_rows_layout(*g, &Hp, &row_elems) == 0, "gather_rows: geometry not eligible for a row image");
   B200RL_REQUIRE(((((uintptr_t)o_tm1 | (uintptr_t)o_t | (uintptr_t)rows_tm1 | (uintptr_t)rows_t)) & 15) == 0, "buffers must be 16-byte aligned");
+  if (g->C != 4) {
+    // other channel counts (RGB frames, stacks of RGB frames): the batch gather, then the row image of each half written
+    // from the gathered frames (padding channels zero, as b200rl_conv2d_rows_bf16_from_u8 writes them)
+    if (int rc = gather_locked(h, B, idx_dev, o_tm1, a_tm1, R, D, o_t, stream)) return rc;
+    b200rl_conv_geom gb = *g;
+    gb.B = B;
+    if (int rc = h_rows_write((const uint8_t*)o_tm1, gb, (__nv_bfloat16*)rows_tm1, as_stream(stream))) return rc;
+    return h_rows_write((const uint8_t*)o_t, gb, (__nv_bfloat16*)rows_t, as_stream(stream));
+  }
+  B200RL_REQUIRE(g->W % 4 == 0 && g->pad_left % 2 == 0, "gather_rows: W %% 4 == 0 and an even pad_left (16-byte aligned pixel pairs)");
   int rc = ensure_device(h);
   if (rc) return rc;
   const int zsplit = std::max(1, std::min(4, (h->cfg.obs_bytes >> 4) / 256));

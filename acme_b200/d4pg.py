@@ -137,8 +137,16 @@ class D4PGLearner(core.Learner, core.Saveable):
         raise ValueError(f'the {name} reads {n.obs_dim} inputs but the observation network gives {o.flat_dim} features')
     if to.flat_dim != o.flat_dim or to.params.size != o.params.size:
       raise ValueError('the target observation network must have the observation network\'s architecture')
-    if o.flow and np.dtype(dataset.table.signature[0].dtype) != np.uint8:
+    sig = dataset.table.signature[0]
+    if o.flow and np.dtype(sig.dtype) != np.uint8:
       raise ValueError('precision 2 (the bf16 dataflow) reads uint8 frames: the observation spec must be uint8')
+    if int(np.prod(sig.shape)) != o.in_hw * o.in_hw * o.in_c:
+      raise ValueError(f'observations of shape {tuple(sig.shape)} are not {o.in_hw} x {o.in_hw} x {o.in_c} frames, the '
+                       'observation network\'s input')
+    if o.in_c != o.in_cp and np.dtype(sig.dtype) != np.uint8:
+      raise ValueError(f'frames of {o.in_c} channels (conv1 padded to {o.in_cp}) must be uint8')
+    if o.flow and not o.rows_frame_bytes():
+      raise ValueError(f'precision 2 (the bf16 dataflow) needs frames with a row image; got {o.in_c} channels')
 
   def _joint(self, torso, critic):
     """One flat parameter / gradient (/ bf16 shadow) buffer holding the torso's then the critic's parameters; both
@@ -283,6 +291,9 @@ class D4PGLearner(core.Learner, core.Saveable):
     ds.gather_only(self._gather_rows)
     o0, a0, o1 = self._views()
     rows0, rows1 = self._rows if self._gather_rows is not None else (None, None)
+    if O.pads_frames and self._obs_u8:
+      # frames padded to 4-channel pixels (precisions 0 and 1): one padded operand per batch, read by forward and backward
+      rows0, rows1 = O.prepare_frames(o0, 'tm1'), TO.prepare_frames(o1, 't')
     main = torch.cuda.current_stream()
     fork = self._concurrent
     if fork:

@@ -207,6 +207,8 @@ class DQNLearner(core.Learner, core.Saveable):
     self._act_dtype = np.dtype(t.signature[1].dtype)
     # bf16 dataflow on uint8 frames: K3 writes the first conv layer's row image itself (no conversion pass)
     self._gather_rows = None
+    if getattr(network, 'flow', False) and hasattr(network, 'rows_frame_bytes') and not network.rows_frame_bytes():
+      raise ValueError(f'precision 2 (the bf16 dataflow) needs frames with a row image; got {network.in_c} channels')
     if (self._fused and getattr(network, 'flow', False) and self._obs_dtype == np.uint8 and
         getattr(dataset, 'supports_gather_rows', True)):
       buf = network.rows_buffer(2 * B, 'all')

@@ -228,6 +228,8 @@ class Network:
       a = self.params.get(name, grad)
       if kind == 'conv':      # OHWI -> HWIO
         a = a.transpose(1, 2, 3, 0)
+      elif isinstance(kind, tuple) and kind[0] == 'conv':   # OHWI with padding input channels -> HWIO of the first kind[1]
+        a = a.transpose(1, 2, 3, 0)[:, :, :kind[1], :]
       elif kind == 'linear':  # [out, in] -> [in, out]
         a = a.T
       elif isinstance(kind, tuple) and kind[0] == 'rows':   # rows [lo:hi] of a stacked [out, in]
@@ -243,6 +245,12 @@ class Network:
       v = np.asarray(variables[sonnet_name], np.float32)
       if kind == 'conv':
         staged[name] = v.transpose(3, 0, 1, 2)
+      elif isinstance(kind, tuple) and kind[0] == 'conv':
+        if v.shape[2] != kind[1]:
+          raise ValueError(f'{sonnet_name}: expected {kind[1]} input channels, got shape {v.shape}')
+        full = np.zeros(self.params.entries[name][1], np.float32)
+        full[..., :kind[1]] = v.transpose(3, 0, 1, 2)
+        staged[name] = full
       elif kind == 'linear':
         staged[name] = v.T
       elif isinstance(kind, tuple) and kind[0] == 'rows':
@@ -313,9 +321,21 @@ class _ConvTorso(Network):
   images and the layer calls of their forward and backward passes, shared by AtariTorso and DQNAtariNetwork."""
 
   def _declare_convs(self, input_hw: int, input_channels: int):
-    self.in_hw, self.in_c = input_hw, input_channels
-    self.convs = []  # (k, stride, cin, cout, in_hw, out_hw, pad)
-    h, c = input_hw, input_channels
+    """input_channels C in [1, 16] (4: the grayscale Atari stack; 3: an RGB frame; 3 F: a flattened stack of F RGB frames).
+    conv1's filter is stored with Cp >= C input channels, the last Cp - C of them zero.  Precisions 2 and 3: Cp = 4, 8
+    or 16, the channel group of the bf16 row image, which is written from the C-channel frames with zero padding
+    channels.  Precisions 0 and 1: Cp = C rounded up to 4, the frames padded to Cp channels on the device
+    (`b200rl_frames_pad_u8`).  Every padding product is exactly zero.  Their weight gradient is exactly zero too, so those columns stay zero under clip, Adam, the bf16 shadow,
+    precision 3's split and the target copy; `variables()` exports and loads only the C real channels."""
+    if isinstance(input_channels, bool) or int(input_channels) != input_channels or not 1 <= input_channels <= 16:
+      raise ValueError(f'input_channels must be an integer in [1, 16], got {input_channels!r}')
+    self.in_hw, self.in_c = input_hw, int(input_channels)
+    # the filter's channel count: the bf16 row image's channel group 4, 8 or 16 at precisions 2 and 3 (built from the
+    # C-channel frames directly), C rounded up to 4 at precisions 0 and 1 (the frames padded by b200rl_frames_pad_u8)
+    c = self.in_c
+    self.in_cp = (4 if c <= 4 else 8 if c <= 8 else 16) if self._bf16_rows else -(-c // 4) * 4
+    self.convs = []  # (k, stride, cin, cout, in_hw, out_hw, pad); conv1's cin is the padded in_cp
+    h, c = input_hw, self.in_cp
     for k, s, co in ((8, 4, 32), (4, 2, 64), (3, 1, 64)):
       oh, pad = tf_same_pad(h, k, s)
       self.convs.append((k, s, c, co, h, oh, pad))
@@ -328,10 +348,47 @@ class _ConvTorso(Network):
   def _init_convs(self, rng):
     """Sonnet defaults: TruncatedNormal(stddev=1/sqrt(fan_in)) weights, zero biases."""
     for i, (k, s, ci, co, _, _, _) in enumerate(self.convs, 1):
-      self.params.set(f'conv{i}.w', _truncated_normal(rng, (co, k, k, ci), 1 / math.sqrt(k * k * ci)))
+      c = self.in_c if i == 1 else ci            # conv1: the real fan-in 8 * 8 * C; padding columns stay zero
+      w = np.zeros((co, k, k, ci), np.float32)
+      w[..., :c] = _truncated_normal(rng, (co, k, k, c), 1 / math.sqrt(k * k * c))
+      self.params.set(f'conv{i}.w', w)
+
+  def _conv_export(self, i: int):
+    """`_export` kind of conv i's filter: HWIO, conv1's restricted to the frame's real channels."""
+    return ('conv', self.in_c) if i == 1 and self.in_c != self.in_cp else 'conv'
+
+  @property
+  def pads_frames(self) -> bool:
+    """Precisions 0 and 1 on frames whose channel count is not a multiple of 4: uint8 frames are padded to in_cp channels
+    before conv1."""
+    return self.in_c != self.in_cp and not self._bf16_rows
+
+  def _padded_frames(self, obs, slot: str):
+    """uint8 [B, H, W, C] -> the cached [B, H, W, in_cp] copy with zero padding channels (`b200rl_frames_pad_u8`)."""
+    import torch
+    if obs.dtype != torch.uint8:
+      raise ValueError(f'frames with {self.in_c} channels (not a multiple of 4) must be uint8')
+    B = obs.shape[0]
+    if obs.numel() != B * self.in_hw * self.in_hw * self.in_c:
+      raise ValueError(f'expected {B} frames of {self.in_hw} x {self.in_hw} x {self.in_c} bytes, got shape {tuple(obs.shape)}')
+    cache = self.__dict__.setdefault('_rows', {})
+    key = ('pad', slot, B)
+    if key not in cache:
+      cache[key] = torch.empty((B, self.in_hw, self.in_hw, self.in_cp), dtype=torch.uint8, device=torch.device('cuda', self.device))
+    out = cache[key]
+    _capi.call('b200rl_frames_pad_u8', obs.data_ptr(), B * self.in_hw * self.in_hw, self.in_c, self.in_cp, out.data_ptr(),
+               _capi.current_stream())
+    return out
+
+  @property
+  def _bf16_rows(self) -> bool:
+    """conv1 reads the bf16 row image (precisions 2 and 3), whose entry points take the frames' own channel count."""
+    return self.flow or self.x3
 
   def geom(self, i: int, B: int) -> ConvGeom:
     k, s, ci, co, h, oh, pad = self.convs[i]
+    if i == 0 and self._bf16_rows:
+      ci = self.in_c
     return ConvGeom(B=B, H=h, W=h, C=ci, kh=k, kw=k, stride=s, pad_top=pad, pad_left=pad, OH=oh, OW=oh, Cout=co)
 
   def _conv_x3_calls(self, B: int):
@@ -339,7 +396,7 @@ class _ConvTorso(Network):
     calls = []
     for i in range(3):
       g = self.geom(i, B)
-      x_u8s = (1, 2) if i == 0 else (0,)     # conv1 on uint8 frames or on their row image
+      x_u8s = ((1, 2) if self.rows_frame_bytes() else (1,)) if i == 0 else (0,)   # conv1 on uint8 frames or their row image
       calls += [(op, 0, 0, 0, g, u) for u in x_u8s for op in (X.X3_CONV_FWD, X.X3_CONV_WGRAD)]
       if i > 0:
         calls.append((X.X3_CONV_DGRAD, 0, 0, 0, g, 0))
@@ -367,9 +424,13 @@ class _ConvTorso(Network):
         self._mark(f'fwd{B}.conv{i + 1}')
         x, x_rows = y.data_ptr(), 0
       return x
+    if obs.dtype != torch.uint8 and self.in_c != self.in_cp:
+      raise ValueError(f'frames of {self.in_c} channels (conv1 padded to {self.in_cp}) must be uint8')
+    if rows is None and self.pads_frames:
+      rows = self.prepare_frames(obs, 'fwd')
     x, x_u8 = obs.data_ptr(), int(obs.dtype == torch.uint8)
-    if rows is not None:              # the frames' row image from prepare_frames()
-      x, x_u8 = rows.data_ptr(), 2
+    if rows is not None:              # from prepare_frames(): the frames' row image, or the padded frames (4-D)
+      x, x_u8 = rows.data_ptr(), 1 if rows.dim() == 4 else 2
     for i in range(3):
       y = bufs[f'y{i + 1}']
       _conv_fwd(x, x_u8, P.p(f'conv{i + 1}.w'), P.p(f'conv{i + 1}.b'), y.data_ptr(), self.geom(i, B), ACT_RELU, self)
@@ -399,17 +460,22 @@ class _ConvTorso(Network):
     (two networks on o_t; forward + weight gradient on o_tm1).  Precision 1: zero-padded fp32 rows x/255
     (`b200rl_conv2d_rows_from_u8`); precisions 2 and 3: zero-padded bf16 rows of the integer pixel values
     (`b200rl_conv2d_rows_bf16_from_u8`, exact in bf16).  None when not applicable (fp32 mode, float frames, geometry not eligible):
-    callers then pass the frames themselves."""
-    import ctypes
+    callers then pass the frames themselves.  Frames whose channel count is not a multiple of 4 are first padded
+    (`_padded_frames`); without a row image the padded frames themselves ([B, H, W, in_cp] uint8) are returned."""
     import torch
-    if self.precision == _capi.PRECISION_FP32 or obs.dtype != torch.uint8:
+    if self.pads_frames:
+      obs = self._padded_frames(obs, slot)
+    if obs.dtype != torch.uint8:
       return None
+    if self.precision == _capi.PRECISION_FP32:
+      return obs if self.pads_frames else None
     B = obs.shape[0]
     buf = self.rows_buffer(B, slot)
     if buf is None:
       if self.flow:
-        raise ValueError('the bf16 dataflow needs the Atari first-layer geometry (C = 4, kw * C = 32)')
-      return None
+        raise ValueError(f'the bf16 dataflow needs the Atari first-layer geometry (kw * C = 32); frames of {self.in_c} '
+                         'channels have no row image: use precision 0, 1 or 3')
+      return obs if self.pads_frames else None
     name = 'b200rl_conv2d_rows_bf16_from_u8' if self.flow or self.x3 else 'b200rl_conv2d_rows_from_u8'
     _capi.call(name, obs.data_ptr(), self.geom(0, B), buf.data_ptr(), buf.numel(), _capi.current_stream())
     return buf
@@ -438,10 +504,12 @@ class _ConvTorso(Network):
       _capi.call('b200rl_conv2d_wgrad_bf16', x, x_rows, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b') if bias else None, g,
                  ws, wsb, _capi.current_stream())
       return
+    if i == 0 and rows is None and self.pads_frames:
+      rows = self.prepare_frames(obs, 'bwd')
     if i > 0:
       x, x_u8 = bufs[f'y{i}'].data_ptr(), 0
     elif rows is not None:
-      x, x_u8 = rows.data_ptr(), 2
+      x, x_u8 = rows.data_ptr(), 1 if rows.dim() == 4 else 2
     else:
       x, x_u8 = obs.data_ptr(), int(obs.dtype == torch.uint8)
     _conv_wgrad(x, x_u8, dy, P.g(f'conv{i + 1}.w'), P.g(f'conv{i + 1}.b'), g, self)
@@ -475,7 +543,7 @@ class DQNAtariNetwork(_ConvTorso):
     P.declare('a2.w', (self.A, 512))
     P.declare('a2.b', (self.A,))
     self._export = {
-        'conv1/w': ('conv1.w', 'conv'), 'conv1/b': ('conv1.b', None),
+        'conv1/w': ('conv1.w', self._conv_export(1)), 'conv1/b': ('conv1.b', None),
         'conv2/w': ('conv2.w', 'conv'), 'conv2/b': ('conv2.b', None),
         'conv3/w': ('conv3.w', 'conv'), 'conv3/b': ('conv3.b', None),
         'value/l0/w': ('fc1.w', ('rows', 0, 512)), 'value/l0/b': ('fc1.b', ('rows', 0, 512)),
@@ -765,7 +833,7 @@ class AtariTorso(_ConvTorso):
     self._declare_convs(input_hw, input_channels)
     self._export = {}
     for i in range(1, 4):
-      self._export[f'conv{i}/w'] = (f'conv{i}.w', 'conv')
+      self._export[f'conv{i}/w'] = (f'conv{i}.w', self._conv_export(i))
       self._export[f'conv{i}/b'] = (f'conv{i}.b', None)
     self._finalize()
     self._init_convs(np.random.default_rng(seed))

@@ -124,7 +124,10 @@ class Table:
                device: int = 0, shard_count: int = 1, shard_rank: int = 0, stage_slots: int = 0, frame_stack: int = 0):
     """frame_stack = F > 1 (SURVEY §8f-1): the observation is a uint8 stack of F frames on its LAST axis, as
     `FrameStacker` / `AtariWrapper` produce it (`acme/wrappers/frame_stacking.py:64-88`, `atari_wrapper.py:277-308`: the
-    newest frame last, blank frames before the episode's first observation).  The HBM ring then stores ONE frame per
+    newest frame last, blank frames before the episode's first observation).  The last axis may also hold C * F bytes:
+    the stack of F frames of C channels ([..., C, F]) flattened, as `AtariWrapper(grayscaling=False)` gives it; its byte
+    c * F + f is channel c of frame f (f = F - 1 the newest), the bytes of [..., C, F] in the same order, so both
+    layouts are one ring layout.  The HBM ring then stores ONE frame per
     step and K3 rebuilds the stacks when it gathers: obs_bytes / F bytes per step (7,056 instead of 28,224 for Atari)
     and F times less host-to-device traffic per insert.  The caller's observations must really be such stacks: the
     older F-1 frames of every observation are taken from the previous observations of the same episode."""
@@ -184,9 +187,10 @@ class Table:
     self.signature = sig
     if self.frame_stack:
       leaves = tree.flatten(sig[0])
-      if len(leaves) != 1 or np.dtype(leaves[0].dtype) != np.uint8 or tuple(leaves[0].shape)[-1:] != (self.frame_stack,):
-        raise ValueError(f'frame_stack={self.frame_stack} needs a single uint8 observation whose last axis is the frame stack; '
-                         f'got {sig[0]}')
+      shape = tuple(leaves[0].shape) if len(leaves) == 1 else ()
+      if len(leaves) != 1 or np.dtype(leaves[0].dtype) != np.uint8 or not shape or shape[-1] % self.frame_stack != 0:
+        raise ValueError(f'frame_stack={self.frame_stack} needs a single uint8 observation whose last axis is the frame stack '
+                         f'([..., F]) or C channels of F frames flattened ([..., C * F]); got {sig[0]}')
 
   def _ensure(self):
     if self._handle is not None:

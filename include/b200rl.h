@@ -139,10 +139,12 @@ int b200rl_replay_mass_ptr(b200rl_replay* h, float** mass_dev);
  * every shard's *mass_dev); K1 then reports weight / sum_r M_r instead of weight / (R * M_r).  NULL switches it off. */
 int b200rl_replay_set_global_mass(b200rl_replay* h, const float* global_mass_dev);
 
-/* K3 with the first layer's input fused in (bf16 dataflow): as b200rl_replay_gather, and the frames ([H][W][4] uint8) are
- * also written into the zero-padded bf16 row images that b200rl_conv2d_fwd_bf16(x_rows = 1) reads (layout:
- * b200rl_conv2d_rows_bf16_bytes(g with B = 1) bytes per frame; the images must be zero-initialised once -- the padding is
- * never written).  Replaces gather + b200rl_conv2d_rows_bf16_from_u8. */
+/* K3 with the first layer's input fused in (bf16 dataflow): as b200rl_replay_gather, and the frames ([H][W][C] uint8,
+ * 1 <= C <= 16; on a frame-deduplicated table the rebuilt stacks, C = channels per frame x 4) are also written into the
+ * zero-padded bf16 row images that b200rl_conv2d_fwd_bf16(x_rows = 1) reads (layout: b200rl_conv2d_rows_bf16_bytes(g
+ * with B = 1) bytes per frame), byte for byte as b200rl_conv2d_rows_bf16_from_u8 writes them.  C = 4 writes the frames'
+ * interior inside the gather kernel (the images must be zero-initialised once -- the padding is never written); other
+ * channel counts write each whole image after the gather, padding included.  Replaces gather + rows_bf16_from_u8. */
 struct b200rl_conv_geom;   /* defined with the network layers below */
 int b200rl_replay_gather_rows(b200rl_replay* h, int32_t B, const int64_t* idx_dev, void* o_tm1, void* a_tm1, float* R,
                               float* D, void* o_t, void* rows_tm1, void* rows_t, const struct b200rl_conv_geom* g,
@@ -334,6 +336,13 @@ typedef struct b200rl_conv_geom {
 int64_t b200rl_conv2d_rows_bytes(const b200rl_conv_geom* g);
 int b200rl_conv2d_rows_from_u8(const void* x_u8, const b200rl_conv_geom* g, float* rows, int64_t rows_bytes,
                                void* stream);
+/* Frames whose channel count is not a multiple of 4 (RGB: C = 3; C = 1 .. 16).  The first-layer calls read uint8
+ * pixels 4 channels at a time, so such frames are first copied into pixels of Cp channels (C <= Cp <= 16, Cp % 4 == 0),
+ * channels C .. Cp-1 zero: out[p][c] = c < C ? x[p][c] : 0 for the npix pixels.  The filter of the layer that reads
+ * them is stored with Cp input channels whose last Cp - C are zero, so every product of a padding channel is exactly
+ * zero and the convolution equals the one over the C real channels (and the weight gradient of those filter
+ * columns is exactly zero).  out: npix * Cp bytes, 4-byte aligned; x needs no alignment. */
+int b200rl_frames_pad_u8(const void* x_u8, int64_t npix, int32_t C, int32_t Cp, void* out, void* stream);
 /* y = act(conv(x, w) + b).  x_u8 = 1: x is uint8 and is read as float(x)/255 (atari_wrapper.py:303); x_u8 = 2: x is
  * the row image of the frames (precision 1 only). */
 int b200rl_conv2d_fwd(const void* x, int x_u8, const float* w, const float* bias, float* y,
@@ -437,8 +446,12 @@ int b200rl_duelling_head_wgrad(int32_t B, int32_t A, int32_t H, const float* dva
  * always bf16 here.  Shapes outside the kernels' coverage are an error (no fallback): channel counts 32 or multiples
  * of 64, Cout in {32, 64, 128}, dense K and N multiples of 64, 16-byte aligned rows.  Stated tolerance: DESIGN.md. */
 int b200rl_bf16_from_f32(int64_t n, const float* src, void* dst_bf16, void* stream);   /* n % 8 == 0: weight shadows */
-/* First layer on uint8 frames (C = 4, kw * C = 32, networks/atari.py:44): zero-padded bf16 row image holding the
- * INTEGER pixel values (exact in bf16); the 1/255 of atari_wrapper.py:303-304 is applied to the fp32 accumulator. */
+/* First layer on uint8 frames (networks/atari.py:44): zero-padded bf16 row image holding the INTEGER pixel values
+ * (exact in bf16); the 1/255 of atari_wrapper.py:303-304 is applied to the fp32 accumulator.  g->C is the frames' own
+ * channel count, 1 <= C <= 16; each pixel of the image has Cp = 4, 8 or 16 channels (the least >= C), channels C .. Cp-1
+ * zero, and kw * Cp must be 32, 64 or 128.  The filter of the row-image calls (here, and x_u8 != 0 of the `*_x3` calls)
+ * is [Cout][kh][kw][Cp]; its columns C .. Cp-1 should be zero (they multiply zeros) and come out of the weight gradient
+ * as exactly zero.  C = 4 is the Atari stack (Cp = 4). */
 int64_t b200rl_conv2d_rows_bf16_bytes(const b200rl_conv_geom* g);
 int b200rl_conv2d_rows_bf16_from_u8(const void* x_u8, const b200rl_conv_geom* g, void* rows_bf16, int64_t rows_bytes,
                                     void* stream);

@@ -15,6 +15,8 @@ and alternate with the precisions.  Its results go to d4pg_bench_<precision>_pri
 `--observation atari` times D4PG from pixels instead: uint8 84 x 84 x 4 frames through an AtariTorso observation network,
 6-d actions, critic (512, 512, 256) with 51 atoms, policy (256, 256, 256), batch 256, n = 5, at any of fp32, tf32, bf16,
 fp32x3.  Each line adds the step's FLOP count (computed from the shapes by `pixel_step_flop`) and the achieved TFLOP/s.
+`--channels 4,3,12` times frames of those channel counts side by side; C = 4 writes
+d4pg_bench_pixels_<precision>.json as before, other counts d4pg_bench_pixels_c<C>_<precision>.json.
 Results go to d4pg_bench_pixels_<precision>.json."""
 import argparse
 import json
@@ -81,16 +83,16 @@ def pixel_step_flop(B, torso, A, critic_sizes, K, policy_sizes):
   return 2 * B * mac
 
 
-def fill_pixel_table(A, n, items):
+def fill_pixel_table(A, n, items, C=4):
   rng = np.random.default_rng(0)
-  spec = specs.EnvironmentSpec(specs.Array((84, 84, 4), np.uint8), specs.BoundedArray((A,), np.float32, -1., 1.),
+  spec = specs.EnvironmentSpec(specs.Array((84, 84, C), np.uint8), specs.BoundedArray((A,), np.float32, -1., 1.),
                                specs.Array((), np.float32), specs.BoundedArray((), np.float32, 0., 1.))
   table = replay.Table(replay.DEFAULT_PRIORITY_TABLE, replay.selectors.Uniform(), replay.selectors.Fifo(), max_size=items,
                        rate_limiter=replay.rate_limiters.MinSize(1), signature=adders.NStepTransitionAdder.signature(spec),
                        max_window=n, discount=0.99, stage_slots=256)
   server = replay.Server([table])
   adder = adders.NStepTransitionAdder(replay.Client(server), n_step=n, discount=0.99)
-  frames = rng.integers(0, 256, (64, 84, 84, 4), dtype=np.uint8)
+  frames = rng.integers(0, 256, (64, 84, 84, C), dtype=np.uint8)
   steps = 0
   while steps < items:
     adder.add_first(dm_env.restart(frames[steps % 64]))
@@ -104,16 +106,20 @@ def fill_pixel_table(A, n, items):
   return table, server
 
 
-def main_pixels(args, precisions):
+def main_pixels(args, precisions, channels):
+  """One learner per (channel count, precision), timed alternately; C = 4 keeps the names it always had."""
   B, A, n, K = 256, 6, 5, 51
-  table, server = fill_pixel_table(A, n, 20_000)
+  tables = {C: fill_pixel_table(A, n, 20_000, C) for C in channels}
   lib = _capi.load()
-  learners, launches, flop = {}, {}, None
-  for p in precisions:
-    torso = networks.AtariTorso(precision=PRECISIONS[p], seed=0)
+  learners, launches, flop = {}, {}, {}
+  arms = [(C, p) for C in channels for p in precisions]
+  for arm in arms:
+    C, p = arm
+    table = tables[C][0]
+    torso = networks.AtariTorso(precision=PRECISIONS[p], seed=0, input_channels=C)
     policy = networks.D4PGPolicy(torso.flat_dim, A, seed=1, precision=PRECISIONS[p])
     critic = networks.D4PGCritic(torso.flat_dim, A, seed=2, precision=PRECISIONS[p])
-    flop = pixel_step_flop(B, torso, A, critic.sizes, K, policy.sizes)
+    flop[arm] = pixel_step_flop(B, torso, A, critic.sizes, K, policy.sizes)
     ds = replay.ReplayDataset(table, B, seed=11, stratified=False)
     L = d4pg.D4PGLearner(policy, critic, policy.clone(), critic.clone(), 0.99, target_update_period=100, dataset=ds,
                          logger=loggers.NoOpLogger(), observation_network=torso, target_observation_network=torso.clone())
@@ -122,37 +128,41 @@ def main_pixels(args, precisions):
     n0 = lib.b200rl_launch_count()
     L.step(fetch_loss=False)
     torch.cuda.synchronize()
-    launches[p] = int(lib.b200rl_launch_count() - n0)
+    launches[arm] = int(lib.b200rl_launch_count() - n0)
     for _ in range(args.warmup):
       L.step(fetch_loss=False)
     torch.cuda.synchronize()
-    learners[p] = L
-  ms = {p: [] for p in precisions}
+    learners[arm] = L
+  ms = {arm: [] for arm in arms}
   e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
   for _ in range(args.reps):
-    for p in precisions:
-      L = learners[p]
+    for arm in arms:
+      L = learners[arm]
       torch.cuda.synchronize()
       e0.record()
       for _ in range(args.steps):
         L.step(fetch_loss=False)
       e1.record()
       torch.cuda.synchronize()
-      ms[p].append(e0.elapsed_time(e1) / args.steps)
+      ms[arm].append(e0.elapsed_time(e1) / args.steps)
   gpu, power_limit = gpu_info()
-  for p in precisions:
-    med = float(np.median(ms[p]))
-    out = {'workload': 'D4PG from pixels: uint8 84x84x4, AtariTorso, 6-d actions, critic (512, 512, 256) C51, policy '
-                       '(256, 256, 256), batch 256, n=5', 'precision': p, 'precision_mode': PRECISIONS[p],
-           'steps_per_rep': args.steps, 'ms_per_step_reps': ms[p], 'ms_per_step': med, 'updates_per_s': 1e3 / med,
-           'launches_per_eager_step': launches[p], 'gflop_per_step': flop / 1e9, 'achieved_tflop_s': flop / (med * 1e-3) / 1e12,
-           'gpu': gpu, 'power_limit': power_limit}
+  for arm in arms:
+    C, p = arm
+    med = float(np.median(ms[arm]))
+    # gflop_per_step counts the MMA work done: conv1 over the filter's padded channel count (networks._ConvTorso)
+    out = {'workload': f'D4PG from pixels: uint8 84x84x{C}, AtariTorso, 6-d actions, critic (512, 512, 256) C51, policy '
+                       '(256, 256, 256), batch 256, n=5', 'channels': C, 'precision': p, 'precision_mode': PRECISIONS[p],
+           'steps_per_rep': args.steps, 'ms_per_step_reps': ms[arm], 'ms_per_step': med, 'updates_per_s': 1e3 / med,
+           'launches_per_eager_step': launches[arm], 'gflop_per_step': flop[arm] / 1e9,
+           'achieved_tflop_s': flop[arm] / (med * 1e-3) / 1e12, 'gpu': gpu, 'power_limit': power_limit}
     print(json.dumps(out))
     if args.out:
       os.makedirs(args.out, exist_ok=True)
-      with open(os.path.join(args.out, f'd4pg_bench_pixels_{p}.json'), 'w') as f:
+      name = f'd4pg_bench_pixels_{p}.json' if C == 4 else f'd4pg_bench_pixels_c{C}_{p}.json'
+      with open(os.path.join(args.out, name), 'w') as f:
         json.dump(out, f, indent=1)
-  server.stop()
+  for _, server in tables.values():
+    server.stop()
 
 
 def main():
@@ -165,13 +175,18 @@ def main():
   ap.add_argument('--out', default=None, help='directory for d4pg_bench_<precision>.json')
   ap.add_argument('--observation', default='state', choices=['state', 'atari'],
                   help='state: flat 67-d observations; atari: uint8 frames through an AtariTorso observation network')
+  ap.add_argument('--channels', default='4',
+                  help='--observation atari: comma-separated frame channel counts in [1, 16] (4: grayscale stack, 3: RGB)')
   args = ap.parse_args()
+  channels = [int(c) for c in args.channels.split(',') if c.strip()]
+  if any(not 1 <= c <= 16 for c in channels) or (channels != [4] and args.observation != 'atari'):
+    ap.error('--channels takes counts in [1, 16] with --observation atari')
   precisions = [p.strip() for p in args.precision.split(',') if p.strip()]
   for p in precisions:
     if p not in PRECISIONS or (p == 'fp32x3' and args.observation == 'state'):
       ap.error(f'unknown precision {p!r} (fp32, tf32, bf16; fp32x3 with --observation atari)')
   if args.observation == 'atari':
-    return main_pixels(args, precisions)
+    return main_pixels(args, precisions, channels)
   arms = [r.strip() for r in args.replay.split(',') if r.strip()]
   for r in arms:
     if r not in ('uniform', 'prioritized'):
